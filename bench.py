@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the joint-step hot path (fused front-end x3 + CTC + 41-step AttLoc loop, fwd + bwd).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[2]/[3] per-GPU shape -- B=32 utterances, T=800 STFT
 frames x 257 bins -> 40 mel, encoder length Th=200, U=40 labels (41 decoder steps), vocab 4233,
@@ -559,6 +559,32 @@ def kernel_rooflines(hp, db, cfg, peak, dev):
     return res
 
 
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+
+
+def dump_items(out):
+    """(name, tensor) of what a step returns to its caller (``HotPath.step``: features, losses, attention, gradients).
+    Keys starting with '_' are buffers a data-parallel job adds after the replay (the all-reduced gradients)."""
+    for k, v in out.items():
+        if not k.startswith("_"):
+            yield k, (torch.stack(list(v)) if isinstance(v, (list, tuple)) else v)   # per-step loop: d_dec_z is a list
+
+
+def check_dump_size(out):
+    total = sum(4 * v.numel() for _, v in dump_items(out))
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+
+
+def dump_outputs(out, path):
+    """Every tensor of ``dump_items(out)`` as ``path/<name>.npy`` in float32, so that two builds can be compared output
+    for output on the same seeded inputs.  At the bench shape that is the whole output, about 56 MB."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for k, v in dump_items(out):
+        np.save(os.path.join(path, k + ".npy"), v.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -571,7 +597,14 @@ def main():
     ap.add_argument("--no-recog", action="store_true", help="skip the beam-search (configs[4]) record")
     ap.add_argument("--per-step-loop", action="store_true",
                     help="one AttLoc launch per decoder step instead of the persistent loop kernels (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs and gradients of the last timed step of --impl ours as DIR/<name>.npy "
+                         "(rank 0); choose a DIR outside the source tree")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     from robust_e2e_gan_b200.parallel import init_distributed
@@ -652,6 +685,8 @@ def main():
     # only what is host-resident in the reference flow crosses PCIe per step (mix, clean, lengths, labels); the
     # stand-ins for tensors that upstream networks produce on the device stay resident (declared in the e2e record)
     runner = StepRunner(hp, hb, slots=3, upstream="device")
+    if args.dump_outputs:
+        check_dump_size(runner.slots[0]["out"])     # every rank, before any collective: all of them stop together
     mode = "cuda_graph" + ("" if args.no_overlap else " (front-end | CTC | decoder-loop branches on 3 streams)")
     if reduce_in_graph:
         mode += "; gradient all-reduce captured in the graph (ctc_lo.weight from its grad hook, the rest as one flat message)"
@@ -677,7 +712,7 @@ def main():
             flush.fill_(0.0)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(rs)
-        runner.replay_resident(0)
+        out = runner.replay_resident(0)
         e1.record(rs)
         evs.append((e0, e1))
     barrier()
@@ -688,6 +723,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_per_step = float(t.item()) / args.steps
     value = cfg["B"] * world / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through StepRunner: every step copies its pinned host batch in and reads the loss back.
     #      Two steps of look-ahead over three input slots: while step i computes, batch i+1 is already resident and
