@@ -104,22 +104,24 @@ def best_path(lp_btv):
 
 # ----------------------------------------------------------------------------- prefix score
 class CTCPrefixScoreOracle(object):
-    """Restatement of e2e_ctc.py:78-155 in float32 numpy (logzero = -1e10)."""
+    """Restatement of e2e_ctc.py:78-155 in numpy (logzero = -1e10).  ``dtype``: float32 is the reference's own
+    arithmetic; float64 gives the high-precision truth the device kernel is judged against."""
 
-    def __init__(self, x, blank, eos):
+    def __init__(self, x, blank, eos, dtype=np.float32):
         self.logzero = -10000000000.0
         self.blank = blank
         self.eos = eos
+        self.dtype = dtype
         self.input_length = len(x)
-        self.x = np.asarray(x, dtype=np.float32)
+        self.x = np.asarray(x, dtype=dtype)
 
     def initial_state(self):
         """:95-107 -- r[t,1] = cumulative blank log-prob, r[t,0] = logzero."""
         T = self.input_length
-        r = np.full((T, 2), self.logzero, dtype=np.float32)
-        acc = np.float32(0.0)
+        r = np.full((T, 2), self.logzero, dtype=self.dtype)
+        acc = self.dtype(0.0)
         for t in range(T):
-            acc = np.float32(acc + self.x[t, self.blank]) if t > 0 else self.x[0, self.blank]
+            acc = self.dtype(acc + self.x[t, self.blank]) if t > 0 else self.x[0, self.blank]
             r[t, 1] = acc
         return r
 
@@ -130,12 +132,12 @@ class CTCPrefixScoreOracle(object):
         cs = np.asarray(cs)
         n = len(cs)
         output_length = len(y) - 1
-        r = np.full((T, 2, n), self.logzero, dtype=np.float32)
+        r = np.full((T, 2, n), self.logzero, dtype=self.dtype)
         xs = self.x[:, cs]
         if output_length == 0:
             r[0, 0] = xs[0]
             r[0, 1] = self.logzero
-        r_sum = np.logaddexp(r_prev[:, 0], r_prev[:, 1]).astype(np.float32)
+        r_sum = np.logaddexp(r_prev[:, 0], r_prev[:, 1]).astype(self.dtype)
         last = y[-1]
         log_phi = np.repeat(r_sum[:, None], n, axis=1)
         if output_length > 0:
@@ -151,4 +153,4 @@ class CTCPrefixScoreOracle(object):
         eos_pos = np.where(cs == self.eos)[0]
         if len(eos_pos) > 0:
             log_psi[eos_pos] = r_sum[-1]
-        return log_psi.astype(np.float32), np.moveaxis(r, 2, 0), start
+        return log_psi.astype(self.dtype), np.moveaxis(r, 2, 0), start

@@ -157,7 +157,7 @@ class _FusedSearch(object):
     end_detect; model/e2e_decoder.py:296-333) on the oldest chunk that has arrived.  Positions launched beyond the one
     where the search ends are discarded (past maxlen the merge kernel is a no-op)."""
 
-    def __init__(self, dec, hb, lpz, recog_args, Cb, maxlen, minlen, stream, slot, chunk=8):
+    def __init__(self, dec, hb, lpz, recog_args, Cb, maxlen, minlen, stream, slot, tables, chunk=8):
         self.dec, self.args, self.maxlen, self.minlen, self.chunk = dec, recog_args, maxlen, minlen, chunk
         self.stream, self.dev = stream, hb.device
         self.beam = hb.size(0)
@@ -171,7 +171,7 @@ class _FusedSearch(object):
         self.pin, self.events = pin
         self.hist_np = self.pin.numpy()
         with torch.cuda.stream(stream):
-            self.position = dec._fused_position(hb, lpz, Cb, self.beam, recog_args.ctc_weight, maxlen, self.pin,
+            self.position = dec._fused_position(hb, lpz, Cb, self.beam, recog_args.ctc_weight, maxlen, self.pin, tables,
                                                 bool(getattr(recog_args, "fused_tail", True)))
         self.use_graph = bool(getattr(recog_args, "cuda_graph", True)) and maxlen >= 6
         self.graph = None
@@ -195,6 +195,7 @@ class _FusedSearch(object):
         dec, dev = self.dec, self.dev
         if getattr(dec, "_cap_stream", None) is None or dec._cap_stream.device != dev:
             dec._cap_stream = torch.cuda.Stream(dev)
+            dec._graph_pool = None        # (the generic position's pool belongs to the previous device)
         dec._cap_stream.wait_stream(self.stream)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.stream(dec._cap_stream):
@@ -399,37 +400,32 @@ class Decoder(torch.nn.Module):
     # ------------------------------------------------------------------------------------------ beam search
     @torch.no_grad()
     def _beam_tables(self):
-        """Per-model constants of the fused beam-search position, rebuilt when a parameter changes: the embedding half of
-        the LSTMCell input product for EVERY token (V, 4Z) = embed.weight @ W_ih[:, :E]^T + b_ih + b_hh (looked up by token
-        in the step kernel), the recurrent matrices side by side (4Z, D+Z), and the output layer."""
+        """Per-model constants of the fused beam-search position: the embedding half of the LSTMCell input product for
+        EVERY token (V, 4Z) = embed.weight @ W_ih[:, :E]^T + b_ih + b_hh (looked up by token in the step kernel), the
+        recurrent matrices side by side (4Z, D+Z), and the output layer.  Built once per recognize_beam /
+        recognize_beam_batch call, never cached across calls: a write through ``.data`` (checkpoint averaging, a
+        training step between decodes) changes a parameter without bumping its version counter, so no cache key can see
+        it, and stale tables would make the fused search silently decode with the old weights."""
         cell = self.decoder[0]
-        ps = (self.embed.weight, cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, self.output.weight,
-              self.output.bias)
-        key = tuple((p.data_ptr(), p._version) for p in ps)
-        tb = getattr(self, "_beam_tab", None)
-        if tb is None or tb[0] != key:
-            with torch.no_grad():
-                E = self.embed.weight.size(1)
-                eg = linear(_lib.f32c(self.embed.weight.detach()), cell.weight_ih.detach()[:, :E].contiguous(),
-                            (cell.bias_ih + cell.bias_hh).detach()).contiguous()
-                wcat = torch.cat((cell.weight_ih.detach()[:, E:], cell.weight_hh.detach()), 1).float().contiguous()
-                tb = (key, eg, wcat, _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach()))
-            self._beam_tab = tb
-        return tb[1:]
+        E = self.embed.weight.size(1)
+        eg = linear(_lib.f32c(self.embed.weight.detach()), cell.weight_ih.detach()[:, :E].contiguous(),
+                    (cell.bias_ih + cell.bias_hh).detach()).contiguous()
+        wcat = torch.cat((cell.weight_ih.detach()[:, E:], cell.weight_hh.detach()), 1).float().contiguous()
+        return eg, wcat, _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach())
 
-    def _fused_position(self, hb, lpz, Cb, beam, ctc_weight, maxlen, hist, fused_tail=True):
+    def _fused_position(self, hb, lpz, Cb, beam, ctc_weight, maxlen, hist, tables, fused_tail=True):
         """One output position for all W rows as launches of the library over static buffers (csrc/beam.cu):
         AttLoc step, LSTMCell step (embedding half by token lookup), output layer, log-softmax + top-Cb, CTC prefix
         scores, then joint score + merge + gather of the chosen rows' states for the next position (one launch,
         ``re2e_beam_advance``; ``fused_tail=False`` runs them as three).  ``hist`` (>= maxlen, 4, beam): page-locked host
-        tensor the winners of every position are written to.  Returns the position closure.
-        The first position needs no special case: the states start as every row's initial state."""
+        tensor the winners of every position are written to.  ``tables``: ``_beam_tables()`` of this call.  Returns the
+        position closure.  The first position needs no special case: the states start as every row's initial state."""
         import ctypes
         lib = _lib.lib()
         dev = hb.device
         W, Th, D = hb.shape
         Z, V = self.dunits, self.output.out_features
-        eg, wcat, w_out, b_out = self._beam_tables()
+        eg, wcat, w_out, b_out = tables
         st = self.att.precompute(hb)
         _, _, _, A, _, C, K = st.dims
         W_dec, W_att, W_conv, gvec, gvec_b = st.weights
@@ -538,7 +534,8 @@ class Decoder(torch.nn.Module):
 
     def _recognize_fused(self, hb, lpz, recog_args, Cb, maxlen, minlen):
         """Beam search with the whole position on the device, one utterance on the current stream (``_FusedSearch``)."""
-        search = _FusedSearch(self, hb, lpz, recog_args, Cb, maxlen, minlen, torch.cuda.current_stream(hb.device), 0)
+        search = _FusedSearch(self, hb, lpz, recog_args, Cb, maxlen, minlen, torch.cuda.current_stream(hb.device), 0,
+                              self._beam_tables())
         while not search.done:
             search.pump()
             search.poll(block=True)
@@ -580,6 +577,7 @@ class Decoder(torch.nn.Module):
         if streams is None or len(streams) < concurrency or streams[0].device != dev:
             streams = self._search_streams = [torch.cuda.Stream(dev) for _ in range(concurrency)]
         active = {}                       # slot -> (utterance index, search)
+        tables = None                     # made on the caller's stream, which every search stream waits for below
         nxt = 0
         while nxt < n or active:
             for slot in range(concurrency):
@@ -590,13 +588,15 @@ class Decoder(torch.nn.Module):
                     if plan is None:      # shapes the fused position does not take: the per-utterance path
                         results[i] = self.recognize_beam(hs[i], lp, recog_args, char_list)
                         continue
+                    if tables is None:
+                        tables = self._beam_tables()
                     for t in plan[:2]:    # made on the caller's stream, consumed on the search's
                         if t is not None:
                             t.record_stream(streams[slot])
                     streams[slot].wait_stream(cur)
                     self.att.reset()
                     active[slot] = (i, _FusedSearch(self, plan[0], plan[1], recog_args, plan[2], plan[3], plan[4],
-                                                    streams[slot], slot))
+                                                    streams[slot], slot, tables))
             progressed = False
             for slot, (i, srch) in list(active.items()):
                 srch.pump()
@@ -736,6 +736,8 @@ class Decoder(torch.nn.Module):
                     cur = torch.cuda.current_stream(dev)
                     if getattr(self, "_cap_stream", None) is None or self._cap_stream.device != dev:
                         self._cap_stream = torch.cuda.Stream(dev)
+                        self._graph_pool = None
+                    if getattr(self, "_graph_pool", None) is None:     # (a fused search creates the stream only)
                         self._graph_pool = torch.cuda.graph_pool_handle()
                     self._cap_stream.wait_stream(cur)
                     graph = torch.cuda.CUDAGraph()

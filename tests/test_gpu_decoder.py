@@ -54,11 +54,38 @@ def test_beam_search_matches_reference_golden(name):
     assert ctc.best_path(hd.unsqueeze(0))[0].cpu().tolist() == [int(t) for t in GOLD[name + ".best_path"]]
 
 
-@pytest.mark.parametrize("seed,beam,ctc_weight", [(7, 1, 0.0), (8, 6, 0.3), (9, 4, 1.0)])
-def test_beam_search_matches_oracle(seed, beam, ctc_weight):
-    """greedy (beam 1), hybrid and CTC-only scoring on fresh seeds: GPU tokens == oracle tokens."""
-    helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES["beam_eos"], seed=seed, beam=beam, ctc_weight=ctc_weight,
-                                      nbest=min(beam, 3), Th=22)
+def _never_eos(Th):
+    # <eos> far below every other token: not even among the CTC candidates, so every search ends through the append at
+    # the last position.  maxlen = Th puts that end at every offset within the 8-position graph chunk (5: no graph).
+    return pytest.param("beam_eos", dict(seed=50 + Th, beam=5, ctc_weight=0.5, nbest=3, Th=Th, eos_bias=-30.0),
+                        id="never_eos-maxlen%d" % Th)
+
+
+ORACLE_CASES = [
+    # greedy (beam 1), hybrid and CTC-only scoring on fresh seeds
+    pytest.param("beam_eos", dict(seed=7, beam=1, ctc_weight=0.0, nbest=1, Th=22), id="7-1-0.0"),
+    pytest.param("beam_eos", dict(seed=8, beam=6, ctc_weight=0.3, nbest=3, Th=22), id="8-6-0.3"),
+    pytest.param("beam_eos", dict(seed=9, beam=4, ctc_weight=1.0, nbest=3, Th=22), id="9-4-1.0"),
+] + [_never_eos(Th) for Th in (5, 6, 7, 8, 9, 16, 17, 23)] + [
+    # <eos> is the best candidate at position 0: hypotheses end in the first (single-position) flight and end_detect
+    # fires inside the first chunk
+    pytest.param("beam_eos", dict(seed=60, beam=5, ctc_weight=0.0, nbest=3, Th=22, eos_bias=40.0), id="eos_first-att"),
+    pytest.param("beam_eos", dict(seed=61, beam=5, ctc_weight=0.3, nbest=3, Th=22, eos_bias=100.0), id="eos_first-ctc"),
+    # the fused position's limits (Cb = int(1.5 beam) <= 32, W <= 32) and the dispatch to the generic position beyond
+    pytest.param("beam_default_dims", dict(seed=70, beam=21, nbest=3), id="beam21-Cb31"),
+    pytest.param("beam_default_dims", dict(seed=71, beam=22, nbest=3), id="beam22-Cb33-generic"),
+    pytest.param("beam_default_dims", dict(seed=72, beam=32, ctc_weight=0.0, nbest=3), id="beam32-att_only"),
+    pytest.param("beam_default_dims", dict(seed=73, ctc_weight=1.0, nbest=3), id="ctc_only-generic"),
+    # length penalty, minimum and maximum length on a long search (no end_detect with maxlenratio > 0)
+    pytest.param("beam_eos", dict(seed=80, beam=5, ctc_weight=0.5, nbest=3, Th=80, eos_bias=0.5, penalty=0.5,
+                                  minlenratio=0.3, maxlenratio=0.5), id="nbest3-minlen-maxlen-penalty"),
+]
+
+
+@pytest.mark.parametrize("base,over", ORACLE_CASES)
+def test_beam_search_matches_oracle(base, over):
+    """GPU tokens == oracle tokens, scores to 1e-4, for search settings beyond the golden cases."""
+    helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES[base], **over)
     try:
         c, sd, h, _ = helpers.beam_case("_tmp")
     finally:
@@ -69,48 +96,85 @@ def test_beam_search_matches_oracle(seed, beam, ctc_weight):
     assert [x["yseq"] for x in nbest] == [x["yseq"] for x in ref]
     for a, b in zip(nbest, ref):
         assert abs(a["score"] - b["score"]) <= 1e-4 * abs(b["score"])
+    # the cases do what their names say
+    if c["eos_bias"] <= -30.0:
+        assert all(len(x["yseq"]) == c["Th"] + 2 and c["eos"] not in x["yseq"][1:-1] for x in ref)
+    if c["eos_bias"] >= 40.0:
+        assert ref[0]["yseq"] == [c["sos"], c["eos"]]
 
 
-def test_decoder_training_loop_matches_oracle():
-    """Decoder.forward (teacher forcing): loss, accuracy and gradients w.r.t. the encoder output, the attention
-    parameters and the decoder's own layers."""
-    c, sd, _, _ = helpers.beam_case("beam_small")
+def training_case(name):
+    """(decoder on the GPU in train mode, its CPU state dict, hpad, hlen, ys, sos, eos) of a training-loop input:
+    ``beam_small`` dims, or ``bench`` = the workload of bench.py's decoder_forward_bench (must stay equal to it:
+    B = 32, Th = 200, U = 40, V = 4233, default AttLoc / decoder dimensions, the same seeds)."""
+    if name == "bench":
+        from robust_e2e_gan_b200 import synth
+        from robust_e2e_gan_b200.hotpath import DEFAULT_CFG
+        B, Th, D, A, Z, C, V, U = (DEFAULT_CFG[k] for k in ("B", "Th", "D", "A", "Z", "C", "V", "U"))
+        torch.manual_seed(7)
+        att = AttLoc(D, Z, A, C, DEFAULT_CFG["filts"], "softmax")
+        dec = Decoder(D, V, 1, Z, V - 1, V - 1, att)
+        sd = {k: v.detach().clone() for k, v in dec.state_dict().items()}
+        hpad, hlen = synth.encoder_batch(B=B, Th=Th, D=D, seed=77)
+        ys = synth.targets(B=B, V=V, hlens=hlen, seed=77, fixed_U=U)
+        return dec.to(DEV).train(), sd, hpad, hlen, ys, V - 1, V - 1
+    c, sd, _, _ = helpers.beam_case(name)
     B, Th = 3, 19
     g = torch.Generator().manual_seed(5)
     hpad = torch.tanh(torch.randn(B, Th, c["D"], generator=g))
     hlen = [19, 15, 11]
     ys = [torch.randint(1, c["V"] - 1, (n,), generator=g) for n in (6, 4, 5)]
-    # oracle (CPU autograd)
-    sd_o = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
-    h_o = hpad.clone().requires_grad_(True)
-    loss_o, acc_o = obeam.decoder_forward(sd_o, h_o, hlen, ys, c["sos"], c["eos"])
-    loss_o.backward()
-    # product
     dec, _ = build(c, sd)
-    dec.train()
+    return dec.train(), sd, hpad, hlen, ys, c["sos"], c["eos"]
+
+
+TRAINING_INPUTS = ("beam_small", "bench")
+
+
+def test_decoder_training_loop_matches_oracle():
+    """Decoder.forward (teacher forcing): loss, accuracy and gradients w.r.t. the encoder output, the attention
+    parameters and the decoder's own layers, against the fp32 oracle with the fp64 oracle as tie-breaker, for every
+    input of TRAINING_INPUTS."""
+    for case in TRAINING_INPUTS:
+        _check_training_loop(case)
+
+
+def _check_training_loop(case):
+    dec, sd, hpad, hlen, ys, sos, eos = training_case(case)
+    # oracle (CPU autograd), fp32 and fp64
+    ref = {}
+    for dt in (torch.float32, torch.float64):
+        sd_o = {k: v.detach().clone().to(dt).requires_grad_(True) for k, v in sd.items()}
+        h_o = hpad.detach().clone().to(dt).requires_grad_(True)
+        loss_o, acc_o = obeam.decoder_forward(sd_o, h_o, hlen, ys, sos, eos)
+        loss_o.backward()
+        ref[dt] = (loss_o.detach(), acc_o, h_o.grad, {k: v.grad for k, v in sd_o.items()})
+    (loss_o, acc_o, gh_o, g_o), (loss_t, _, gh_t, g_t) = ref[torch.float32], ref[torch.float64]
+    # product
     h_d = hpad.to(DEV).requires_grad_(True)
     loss, acc = dec(h_d, hlen, [y.to(DEV) for y in ys], 0.0)
     loss.backward()
-    helpers.assert_close(loss, loss_o, what="loss")
-    assert acc == pytest.approx(acc_o)
-    helpers.assert_close(h_d.grad, h_o.grad, what="d hpad")
+    helpers.assert_close(loss, loss_o, truth=loss_t, what="%s: loss" % case)
+    assert acc == pytest.approx(acc_o), case
+    helpers.assert_close(h_d.grad, gh_o, truth=gh_t, what="%s: d hpad" % case)
     for k, p in dec.named_parameters():
         if k == "att.gvec.bias":          # analytically zero gradient (softmax shift invariance)
             continue
-        helpers.assert_close(p.grad, sd_o[k].grad, what="d " + k)
+        helpers.assert_close(p.grad, g_o[k], truth=g_t[k], what="%s: d %s" % (case, k))
 
 
 def test_decoder_forward_with_device_lengths_is_capturable_and_identical():
     """Lengths given as a CUDA tensor keep Decoder.forward free of host round trips (CUDA-graph capturable); results
-    equal the list-of-ints call, and a captured forward + backward replays to the same loss and gradients."""
-    c, sd, _, _ = helpers.beam_case("beam_small")
-    B, Th = 3, 19
-    g = torch.Generator().manual_seed(5)
-    hpad = torch.tanh(torch.randn(B, Th, c["D"], generator=g)).to(DEV)
-    hlen = [19, 15, 11]
-    ys = [torch.randint(1, c["V"] - 1, (n,), generator=g).to(DEV) for n in (6, 4, 5)]
-    dec, _ = build(c, sd)
-    dec.train()
+    equal the list-of-ints call, and a captured forward + backward replays to the same loss and gradients, for every
+    input of TRAINING_INPUTS."""
+    for case in TRAINING_INPUTS:
+        _check_capturable(case)
+
+
+def _check_capturable(case):
+    dec, _, hpad, hlen, ys, _, _ = training_case(case)
+    hpad = hpad.to(DEV)
+    ys = [y.to(DEV) for y in ys]
     # everything -- the eager reference run included -- on ONE side stream: a parameter's gradient accumulator stays tied
     # to the stream of its first backward, and a capture may not synchronise with the legacy default stream
     st = torch.cuda.Stream()
@@ -141,13 +205,13 @@ def test_decoder_forward_with_device_lengths_is_capturable_and_identical():
         loss2.backward()
     graph.replay()
     torch.cuda.synchronize()
-    assert torch.is_tensor(acc2) and float(acc2) == pytest.approx(acc1)
-    helpers.assert_close(loss2, loss1, what="loss (graph replay)")
-    helpers.assert_close(h2.grad, h1g, what="d hpad (graph replay)")
+    assert torch.is_tensor(acc2) and float(acc2) == pytest.approx(acc1), case
+    helpers.assert_close(loss2, loss1, what="%s: loss (graph replay)" % case)
+    helpers.assert_close(h2.grad, h1g, what="%s: d hpad (graph replay)" % case)
     for k, p in dec.named_parameters():
         if k == "att.gvec.bias":
             continue
-        helpers.assert_close(p.grad, g1[k], what="d %s (graph replay)" % k)
+        helpers.assert_close(p.grad, g1[k], what="%s: d %s (graph replay)" % (case, k))
 
 
 @pytest.mark.parametrize("B,Z,D,L", [(32, 300, 320, 5), (3, 48, 64, 4), (10, 300, 320, 3), (40, 52, 36, 3), (33, 640, 640, 2), (5, 12, 4, 2), (4, 48, 1284, 2)])
@@ -300,8 +364,9 @@ def test_fused_beam_position_matches_generic_path(ctc_weight, beam, Th):
     hd = h.to(DEV)
     lpz = ctc.log_softmax(hd.unsqueeze(0))[0] if ctc_weight > 0.0 else None
     res = {}
-    for fused, graph, tail in ((False, False, True), (False, True, True), (True, False, True), (True, True, True),
-                               (True, False, False), (True, True, False)):
+    # (fused first: a generic search with its graph must also work on a decoder that has run fused searches)
+    for fused, graph, tail in ((True, True, True), (True, False, True), (True, True, False), (True, False, False),
+                               (False, True, True), (False, False, True)):
         ra = recog_args(c)
         ra.fused_position, ra.cuda_graph, ra.fused_tail = fused, graph, tail
         n0 = _lib_count()
@@ -318,23 +383,67 @@ def test_fused_beam_position_matches_generic_path(ctc_weight, beam, Th):
 
 def test_recognize_beam_batch_equals_per_utterance():
     """recognize_beam_batch (interleaved searches on their own streams and graphs) returns, for every utterance, exactly
-    what recognize_beam returns for it alone: lengths differ, some searches end early through <eos> / end_detect."""
-    helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES["beam_eos"], seed=41, beam=5, ctc_weight=0.3, nbest=2, Th=30)
+    what recognize_beam returns for it alone: lengths differ, some searches end early through <eos> / end_detect
+    (eos_bias 2.5) or all run to maxlen (-30).  The last utterance (Th = 300) follows shorter ones on the same slot and
+    needs a longer history buffer than the first 256 positions."""
+    for eos_bias in (2.5, -30.0):
+        helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES["beam_eos"], seed=41, beam=5, ctc_weight=0.3, nbest=2, Th=30,
+                                          eos_bias=eos_bias)
+        try:
+            c, sd, h, _ = helpers.beam_case("_tmp")
+        finally:
+            del helpers.BEAM_CASES["_tmp"]
+        dec, ctc = build(c, sd)
+        g = torch.Generator().manual_seed(99)
+        hs = [torch.tanh(torch.randn(int(t), c["D"], generator=g)).to(DEV) for t in (30, 12, 47, 8, 25, 33, 6, 300)]
+        with torch.no_grad():
+            lpzs = [ctc.log_softmax(x.unsqueeze(0))[0] for x in hs]
+            one = [dec.recognize_beam(x, l, recog_args(c), None) for x, l in zip(hs, lpzs)]
+            for conc in (1, 3):
+                dec.__dict__.pop("_hist_pins", None)        # every slot's history buffer starts at its first utterance
+                got = dec.recognize_beam_batch(hs, lpzs, recog_args(c), None, concurrency=conc)
+                assert got == one, "eos_bias %g, concurrency %d" % (eos_bias, conc)
+            att_only = [dec.recognize_beam(x, None, recog_args(c), None) for x in hs[:3]]
+            assert dec.recognize_beam_batch(hs[:3], None, recog_args(c), None, concurrency=2) == att_only
+        if eos_bias < 0:
+            assert len(one[-1][0]["yseq"]) == 302, "the long search should run to maxlen"
+
+
+def test_fused_search_sees_weights_written_through_data():
+    """Parameters overwritten through ``.data`` (which does not bump their version counter): the next fused search
+    decodes with the new weights, exactly as the oracle with the new state dict and the generic position (run after a
+    fused search on the same decoder, with its CUDA graph) do."""
+    helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES["beam_eos"], seed=45, Th=30)
     try:
         c, sd, h, _ = helpers.beam_case("_tmp")
+        helpers.BEAM_CASES["_tmp"]["seed"] = 46
+        _, sd2, _, _ = helpers.beam_case("_tmp")
     finally:
         del helpers.BEAM_CASES["_tmp"]
     dec, ctc = build(c, sd)
-    g = torch.Generator().manual_seed(99)
-    hs = [torch.tanh(torch.randn(int(t), c["D"], generator=g)).to(DEV) for t in (30, 12, 47, 8, 25, 33, 6)]
+    hd = h.to(DEV)
     with torch.no_grad():
-        lpzs = [ctc.log_softmax(x.unsqueeze(0))[0] for x in hs]
-        one = [dec.recognize_beam(x, l, recog_args(c), None) for x, l in zip(hs, lpzs)]
-        for conc in (1, 3):
-            got = dec.recognize_beam_batch(hs, lpzs, recog_args(c), None, concurrency=conc)
-            assert got == one, "concurrency %d" % conc
-        att_only = [dec.recognize_beam(x, None, recog_args(c), None) for x in hs[:3]]
-        assert dec.recognize_beam_batch(hs[:3], None, recog_args(c), None, concurrency=2) == att_only
+        lpz = ctc.log_softmax(hd.unsqueeze(0))[0]
+        before = dec.recognize_beam(hd, lpz, recog_args(c), None)
+        for name, p in (("decoder.0.weight_hh", dec.decoder[0].weight_hh), ("embed.weight", dec.embed.weight)):
+            v = p._version
+            p.data.copy_(sd2[name].to(DEV))
+            assert p._version == v
+        fused = dec.recognize_beam(hd, lpz, recog_args(c), None)
+        ref = obeam.recognize_beam(dict(sd, **{k: sd2[k] for k in ("decoder.0.weight_hh", "embed.weight")}), h, c)
+    assert [x["yseq"] for x in ref] != [x["yseq"] for x in before], "the new weights should change the result"
+
+    def same(got, name):
+        assert [x["yseq"] for x in got] == [x["yseq"] for x in ref], name
+        for a, b in zip(got, ref):
+            assert abs(a["score"] - b["score"]) <= 1e-4 * abs(b["score"]), name
+
+    same(fused, "fused")
+    ra = recog_args(c)
+    ra.fused_position = False
+    with torch.no_grad():
+        generic = dec.recognize_beam(hd, lpz, ra, None)
+    same(generic, "generic")
 
 
 def test_label_batches_and_length_mask_match_the_list_formulation():
