@@ -47,6 +47,8 @@ unsigned long long re2e_launch_count(void);
  *
  * mask_is_logit: 1 -> act = sigmoid (mask holds linear_out), 0 -> act = identity.
  * enh_out (optional): receives x (the reference's `enhance_out`, (B,T,F)).
+ * Shapes: re2e_fbank_fwd and re2e_fbank_bwd accept the same (F, M) and return RE2E_E_UNSUPPORTED for the rest before
+ * launching anything -- M <= 176 at F = 257 (the SIMT forward's shared-memory tile above 80 filters is the limit).
  * ------------------------------------------------------------------------------------------ */
 int re2e_fbank_fwd(const float *mask, int mask_is_logit, const float *mag, const float *fc,
                    const float *cmvn, const int32_t *lens, float *Y, float *G, float *enh_out,

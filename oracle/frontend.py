@@ -13,9 +13,10 @@ import numpy as np
 import torch
 
 
-def mask_tail(linear_out, mix_inputs, ilens):
-    """enhance_model.py:157-164 -- sigmoid, zero the frames t >= ilens[b], times mix."""
-    out = torch.sigmoid(linear_out)
+def mask_tail(linear_out, mix_inputs, ilens, mask_is_logit=True):
+    """enhance_model.py:157-164 -- sigmoid, zero the frames t >= ilens[b], times mix.  ``mask_is_logit=False``: the
+    mask is used as given, without the sigmoid (the kernels' identity activation)."""
+    out = torch.sigmoid(linear_out) if mask_is_logit else linear_out
     B, T = out.shape[0], out.shape[1]
     pad = torch.zeros(B, T, 1, dtype=torch.bool)
     for i, length in enumerate(ilens):
@@ -43,9 +44,9 @@ def fbank_forward(xs, fc, fbank_cmvn=None):
     return out
 
 
-def masked_fbank_forward(linear_out, mix_inputs, ilens, fc, fbank_cmvn=None):
+def masked_fbank_forward(linear_out, mix_inputs, ilens, fc, fbank_cmvn=None, mask_is_logit=True):
     """The fused stage named by north_star: mask tail followed by FbankModel.forward."""
-    return fbank_forward(mask_tail(linear_out, mix_inputs, ilens), fc, fbank_cmvn)
+    return fbank_forward(mask_tail(linear_out, mix_inputs, ilens, mask_is_logit), fc, fbank_cmvn)
 
 
 class CmvnAccumulator(object):

@@ -506,6 +506,24 @@ int fbank_tc_fwd(const float *mask, int mask_is_logit, const float *mag, const f
                  cudaStream_t st);
 int fbank_tc_bwd(const float *dY, const float *G, const float *mask, int mask_is_logit, const float *mag,
                  const float *fc, const int32_t *lens, float *d_in, int B, int T, int F, int M, cudaStream_t st);
+bool fbank_tc_fwd_fits(int F, int M);
+
+namespace {
+constexpr size_t kBwdSmemBudget = 200 * 1024;   // SIMT backward: filter bank + as many row tiles as fit
+
+// Shapes that BOTH directions run: a forward kernel (tcgen05, or the SIMT fallback) and the SIMT backward, which is
+// the d_in path whenever the tcgen05 backward does not apply (M > 64, M % 4 != 0, F > 260, unaligned dY).
+// re2e_fbank_fwd and re2e_fbank_bwd both reject everything else up front, so no shape takes a forward and then fails
+// in its backward.  At F = 257 this is M <= 176: the SIMT forward tile of M = 177 needs 237,120 B of shared memory.
+bool fbank_shape_ok(int F, int M) {
+  if (M > 256) return false;
+  const FbankGeom gf = M <= 48 ? make_geom<2>(F, M) : make_geom<4>(F, M);
+  const size_t fwd_smem = sizeof(float) * ((size_t)gf.Fp * gf.Mp + (size_t)gf.R * gf.Fp);
+  if (fwd_smem > 227 * 1024 && !fbank_tc_fwd_fits(F, M)) return false;
+  const FbankGeom gb = make_geom<2>(F, M);
+  return sizeof(float) * ((size_t)gb.Fp * gb.Mq + 4 * (size_t)(gb.Mq + gb.Fp)) <= kBwdSmemBudget;
+}
+}  // namespace
 }  // namespace re2e
 
 using namespace re2e;
@@ -514,7 +532,7 @@ extern "C" int re2e_fbank_fwd(const float *mask, int mask_is_logit, const float 
                               const float *cmvn, const int32_t *lens, float *Y, float *G,
                               float *enh_out, int B, int T, int F, int M, void *stream) {
   RE2E_CHECK_ARG(mag && fc && Y && B > 0 && T > 0 && F > 0 && M > 0);
-  if (M > 256) return RE2E_E_UNSUPPORTED;
+  if (!fbank_shape_ok(F, M)) return RE2E_E_UNSUPPORTED;
   const int N = B * T;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int vec_ok = aligned16(mag) && (!mask || aligned16(mask)) && (!enh_out || aligned16(enh_out));
@@ -547,7 +565,7 @@ extern "C" int re2e_fbank_bwd(const float *dY, const float *G, const float *mask
                               float *dfc, int B, int T, int F, int M, void *stream) {
   RE2E_CHECK_ARG(dY && G && mag && fc && B > 0 && T > 0 && F > 0 && M > 0);
   RE2E_CHECK_ARG(d_in || dfc);
-  if (M > 256) return RE2E_E_UNSUPPORTED;
+  if (!fbank_shape_ok(F, M)) return RE2E_E_UNSUPPORTED;
   const int N = B * T;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int rc;
@@ -562,8 +580,7 @@ extern "C" int re2e_fbank_bwd(const float *dY, const float *G, const float *mask
     // rows per tile: fill what is left of ~200 KB after the filter bank, multiple of 4
     size_t fixed = sizeof(float) * (size_t)g.Fp * g.Mq;
     size_t per_row = sizeof(float) * (size_t)(g.Mq + g.Fp);
-    size_t budget = 200 * 1024;
-    if (fixed + 4 * per_row > budget) return RE2E_E_UNSUPPORTED;
+    size_t budget = kBwdSmemBudget;
     int R = (int)((budget - fixed) / per_row);
     R -= R % 4;
     if (R > 128) R = 128;

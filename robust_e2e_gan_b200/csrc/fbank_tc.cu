@@ -819,6 +819,15 @@ extern "C" int re2e_fb_debug_read(long long *host_out) {   // 16 x 256 values of
 }
 #endif
 
+// Whether fbank_tc_fwd has a configuration for (F, M): two accumulator buffers of [hi.hi | hi.lo | lo.hi] columns fit
+// tensor memory and one stage fits shared memory.  Pointer alignment is checked at launch.
+bool fbank_tc_fwd_fits(int F, int M) {
+  const int NB = (M + 15) / 16 * 16, MB = (M + 7) / 8 * 8;
+  const int ntail = (F >= kKC && (F % kKC) >= 1 && (F % kKC) <= 4) ? F % kKC : 0;
+  const int nchunks = (F - ntail + kKC - 1) / kKC;
+  return 2 * (2 * MB + NB) <= 512 && fwd_smem_bytes(nchunks, MB, NB, 1) <= 226 * 1024;
+}
+
 // Returns RE2E_E_UNSUPPORTED when the shape does not fit the tensor-core path (caller falls back to the SIMT kernel).
 int fbank_tc_fwd(const float *mask, int mask_is_logit, const float *mag, const float *fc, const float *cmvn,
                  const int32_t *lens, float *Y, float *G, float *enh_out, int B, int T, int F, int M,
@@ -841,10 +850,9 @@ int fbank_tc_fwd(const float *mask, int mask_is_logit, const float *mag, const f
   p.ntail = (F >= kKC && (F % kKC) >= 1 && (F % kKC) <= 4) ? F % kKC : 0;
   p.nchunks = (F - p.ntail + kKC - 1) / kKC;
   p.ksteps_last = (F - p.ntail - (p.nchunks - 1) * kKC + 7) / 8;
-  if (2 * (2 * p.MB + p.NB) > 512) return RE2E_E_UNSUPPORTED;   // two accumulator buffers of [hi.hi | hi.lo | lo.hi] columns
+  if (!fbank_tc_fwd_fits(F, M)) return RE2E_E_UNSUPPORTED;
   int ns = kMaxStagesTc;
-  while (ns >= 1 && fwd_smem_bytes(p.nchunks, p.MB, p.NB, ns) > 226 * 1024) --ns;
-  if (ns < 1) return RE2E_E_UNSUPPORTED;
+  while (ns > 1 && fwd_smem_bytes(p.nchunks, p.MB, p.NB, ns) > 226 * 1024) --ns;
   p.nstages = ns;
   if (((M & 3) == 0) && !(aligned16(Y) && (!G || aligned16(G)))) return RE2E_E_UNSUPPORTED;
   const int sms = num_sms();

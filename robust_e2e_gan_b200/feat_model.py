@@ -7,6 +7,8 @@ fully fused stage named by the north star -- mask tail of EnhanceModel.forward
 (model/enhance_model.py:157-164) + power + mel + log + CMVN in one kernel -- so that the
 (B,T,257) ``enhance_out`` never round-trips through HBM.
 """
+import weakref
+
 import numpy as np
 import torch
 
@@ -74,7 +76,7 @@ def generic_mel_banks(nfilt=40, nfft=512, samplerate=16000, lowfreq=0, highfreq=
 
 # ------------------------------------------------------------------------------------ band tables
 BAND_W, BIN_W = 32, 4          # csrc/fbank_band.cu: bins per filter window, filters per bin window
-_BAND_CACHE = {}
+_BAND_CACHE = {}               # id(fc) -> (weak reference to fc, copy of fc the tables were built from, tables or None)
 
 
 def band_tables(fc):
@@ -105,21 +107,41 @@ def band_tables(fc):
 
 
 def _band_for(fc, B, T):
-    """Device band tables of ``fc`` when the banded kernels apply to this call, else None.  The structure is detected
-    once per (storage, version) of ``fc`` -- a device-to-host read, so never during a CUDA-graph capture (a capture
-    whose warm-up did not already see this ``fc`` uses the dense kernels)."""
+    """Device band tables of ``fc`` when the banded kernels apply to this call, else None.
+
+    Entries are keyed on the tensor object through a weak reference, so a freed bank's entry goes with it and a new bank
+    allocated at the same address never finds it.  Each entry keeps a copy of the values its tables were built from.
+    Outside a CUDA-graph capture every call compares ``fc`` with that copy on the device (one small compare and a sync)
+    and rebuilds on a mismatch: a write through ``fc.data`` does not bump ``fc._version``, so nothing cheaper sees it.
+    Building the tables is a device-to-host read, so a capture never builds or checks them: it uses the entry of this
+    ``fc`` that its eager warm-up left, or the dense kernels when there is none.  A captured graph replays the tables
+    it was captured with, so a bank is frozen for the life of a captured StepRunner."""
     F, M = fc.shape
     if not _lib.load().re2e_fbank_band_supported(B, T, F, M):
         return None
-    key = (fc.data_ptr(), fc._version, fc.device, F, M)
-    if key not in _BAND_CACHE:
-        if torch.cuda.is_current_stream_capturing():
-            return None
-        tabs = band_tables(fc.detach().float().cpu().numpy())
-        if len(_BAND_CACHE) > 16:
-            _BAND_CACHE.clear()
-        _BAND_CACHE[key] = None if tabs is None else tuple(torch.from_numpy(t).to(fc.device) for t in tabs)
-    return _BAND_CACHE[key]
+    ent = _BAND_CACHE.get(id(fc))
+    if ent is not None and (ent[0]() is not fc or (ent[1].device, ent[1].dtype) != (fc.device, fc.dtype)):
+        ent = None
+    if torch.cuda.is_current_stream_capturing():
+        return None if ent is None else ent[2]
+    if ent is not None and torch.equal(ent[1], fc.detach()):
+        return ent[2]
+    snap = fc.detach().clone()
+    tabs = band_tables(snap.float().cpu().numpy())
+    tabs = None if tabs is None else tuple(torch.from_numpy(t).to(fc.device) for t in tabs)
+    key = id(fc)
+
+    def forget(ref):
+        if _BAND_CACHE.get(key, (None,))[0] is ref:
+            del _BAND_CACHE[key]
+
+    _BAND_CACHE[key] = (weakref.ref(fc, forget), snap, tabs)
+    return tabs
+
+
+def _aligned16(*ts):
+    """The banded kernels move rows with 16 B bulk copies: every buffer they read or write must be 16 B aligned."""
+    return all(t is None or t.data_ptr() % 16 == 0 for t in ts)
 
 
 # --------------------------------------------------------------------------------------- autograd
@@ -142,7 +164,7 @@ class _FbankFunction(torch.autograd.Function):
         Y = torch.empty(B, T, M, device=dev, dtype=torch.float32)
         G = torch.empty(B, T, M, device=dev, dtype=torch.float32) if need_grad else None
         enh = torch.empty(B, T, F, device=dev, dtype=torch.float32) if (want_enh and mask is not None) else None
-        band = _band_for(fc, B, T) if enh is None else None
+        band = _band_for(fc, B, T) if enh is None and _aligned16(mag, mask) else None
         with _lib.on(dev):
             if band is not None:      # banded (mel) bank: the streaming kernels
                 _lib.check(L.re2e_fbank_band_fwd(_lib.ptr(mask), int(mask_is_logit), _lib.ptr(mag), None,
@@ -173,7 +195,7 @@ class _FbankFunction(torch.autograd.Function):
         want_in = ctx.needs_input_grad[0] if mask is not None else ctx.needs_input_grad[1]
         d_in = torch.empty(B, T, F, device=dev, dtype=torch.float32) if want_in else None
         dfc = torch.zeros(F, M, device=dev, dtype=torch.float32) if ctx.needs_input_grad[2] else None
-        band = ctx.band
+        band = ctx.band if _aligned16(dY) else None      # mask, mag: checked in forward; G, d_in: fresh
         with _lib.on(dev):
             if band is not None and d_in is not None:      # banded bank: d_in from the streaming kernel
                 _lib.check(L.re2e_fbank_band_bwd(_lib.ptr(dY), _lib.ptr(G), _lib.ptr(mask), ctx.mask_is_logit,
@@ -215,21 +237,27 @@ class _FbankJoint(torch.autograd.Function):
                                              _lib.ptr(Ym), _lib.ptr(Yc), B, T, F, M, _lib.stream_ptr()),
                        "re2e_fbank_band_fwd")
         if need_grad:
-            ctx.save_for_backward(mask, mix, ln, G, band[2], band[3])
+            ctx.save_for_backward(mask, mix, _lib.f32c(fc.detach(), dev), ln, G, band[2], band[3])
         ctx.mark_non_differentiable(Ym, Yc)
         return Y, Ym, Yc
 
     @staticmethod
     def backward(ctx, dY, _dYm, _dYc):
         L = _lib.lib()
-        mask, mix, ln, G, mlo, bw = ctx.saved_tensors
+        mask, mix, fcc, ln, G, mlo, bw = ctx.saved_tensors
         B, T, F = mix.shape
         M = G.shape[2]
+        dY = _lib.f32c(dY, mix.device)
         d_mask = torch.empty(B, T, F, device=mix.device, dtype=torch.float32)
         with _lib.on(mix.device):
-            _lib.check(L.re2e_fbank_band_bwd(_lib.ptr(_lib.f32c(dY, mix.device)), _lib.ptr(G), _lib.ptr(mask), 1,
-                                             _lib.ptr(mix), _lib.ptr(mlo), _lib.ptr(bw), _lib.ptr(ln), _lib.ptr(d_mask),
-                                             B, T, F, M, _lib.stream_ptr()), "re2e_fbank_band_bwd")
+            if _aligned16(dY):
+                _lib.check(L.re2e_fbank_band_bwd(_lib.ptr(dY), _lib.ptr(G), _lib.ptr(mask), 1, _lib.ptr(mix),
+                                                 _lib.ptr(mlo), _lib.ptr(bw), _lib.ptr(ln), _lib.ptr(d_mask),
+                                                 B, T, F, M, _lib.stream_ptr()), "re2e_fbank_band_bwd")
+            else:                 # the banded kernel needs 16 B aligned rows: the dense kernels take any dY
+                _lib.check(L.re2e_fbank_bwd(_lib.ptr(dY), _lib.ptr(G), _lib.ptr(mask), 1, _lib.ptr(mix), _lib.ptr(fcc),
+                                            _lib.ptr(ln), _lib.ptr(d_mask), None, B, T, F, M, _lib.stream_ptr()),
+                           "re2e_fbank_bwd")
         return d_mask, None, None, None, None, None, None
 
 
@@ -369,8 +397,10 @@ def _joint_features(self, linear_out, mix_inputs, clean_inputs, input_sizes, fba
     if not torch.is_tensor(input_sizes):
         input_sizes = torch.as_tensor(np.asarray(input_sizes))
     B, T = mix_inputs.shape[0], mix_inputs.shape[1]
-    band = None if self.fc.requires_grad else _band_for(self.fc, B, T)
-    if band is not None and not (mix_inputs.requires_grad or clean_inputs.requires_grad):
+    joint = not (self.fc.requires_grad or mix_inputs.requires_grad or clean_inputs.requires_grad)
+    # an aligned input stays aligned through f32c (the same buffer, or a fresh copy)
+    band = _band_for(self.fc, B, T) if joint and _aligned16(linear_out, mix_inputs, clean_inputs) else None
+    if band is not None:
         return _FbankJoint.apply(linear_out, mix_inputs, clean_inputs, self.fc, fbank_cmvn, input_sizes, band)
     enh = masked_fbank(linear_out, mix_inputs, input_sizes, self.fc, fbank_cmvn)
     return enh, self.forward(mix_inputs, fbank_cmvn), self.forward(clean_inputs, fbank_cmvn)
