@@ -205,6 +205,16 @@ int re2e_skinny_nn(const float *X, const float *W, float *out, int M, int N, int
  * (128-bit staging when K % 4 == 0 and X, W are 16 B aligned, scalar staging otherwise).  The backward uses it on transposed weight copies made once per loop. */
 int re2e_batch_nt(const float *X, const float *W, const float *bias /* (N) or NULL */, float *out, int M, int N, int K,
                   int accumulate, void *stream);
+/* Scheduled sampling (model/e2e_decoder.py:123-127): the next input token of every batch row, chosen on the device.
+ *   *flag != 0: tok[m] = argmax_n (X[m,:] . W[n,:] + bias[n])   (lowest n among equal values; -0 and +0 are equal)
+ *   *flag == 0: tok unchanged (the caller pre-fills the teacher tokens)
+ * X (M,K) top-layer decoder state, W (N,K) output layer, bias (N) or NULL; flag: device int32 (read by the kernel, so one
+ * captured graph serves any draw pattern); tok: device int32 (M).  The logits are never written.
+ * ws: re2e_sample_tokens_ws_bytes(M) bytes, zero before the first call; every call leaves it zero (graph-replayable with
+ * no memset).  One call at a time per ws. */
+int re2e_sample_tokens_ws_bytes(int M);
+int re2e_sample_tokens(const float *X, const float *W, const float *bias, const int32_t *flag, int32_t *tok,
+                       unsigned long long *ws, int M, int N, int K, void *stream);
 /* One LSTMCell position in one launch (after the embedding half): gates = egate + ctx @ Wcat[:, :D]^T + h_prev @
  * Wcat[:, D:]^T, then the cell's pointwise arithmetic -> act (B,4Z) gate activations (kept for the backward), c_out, h_out
  * (B,Z).  Wcat (4Z, D+Z) = [W_ih[:, E:] | W_hh].  Clusters of 4 CTAs split the reduction (deterministic order).

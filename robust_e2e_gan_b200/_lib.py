@@ -51,6 +51,8 @@ SIGNATURES = {
     "re2e_skinny_nt": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "re2e_skinny_nn": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "re2e_batch_nt": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "re2e_sample_tokens_ws_bytes": (_I, [_I]),
+    "re2e_sample_tokens": (_I, [_P] * 6 + [_I, _I, _I, _P]),
     "re2e_beam_gather": (_I, [_P, _P, _I, _I, _P, _P, _P, _P, _P]),
     "re2e_log_softmax_topk": (_I, [_P, _LL, _I, _I, _P, _P, _P, _P]),
     "re2e_beam_advance": (_I, [_P, _P, _P, _P, _P, _F, _F, _I, _I, _I, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),

@@ -6,7 +6,8 @@
 //     W_ih[:, Z:]^T and h . W_hh^T -- reduced across a 4-CTA cluster, with the pointwise cell as the epilogue;
 //   * backward per position: the pointwise kernel (gate gradients, d c_prev) + ONE product launch for d context | d h_prev
 //     (lstm_step_kernel<false>, 8-CTA clusters); the weight gradients of all positions are two dense GEMMs after the loop;
-//   * batch_nt_kernel: the generic batch-sized product (any dimensions; also the decoder's output layer in beam search).
+//   * batch_nt_kernel: the generic batch-sized product (any dimensions; also the decoder's output layer in beam search);
+//   * sample_tokens_kernel: the same product reduced to each row's arg-max (scheduled sampling in training).
 #include "attloc_common.cuh"
 #include "common.cuh"
 
@@ -66,60 +67,108 @@ __global__ void __launch_bounds__(256) lstm_pointwise_bwd_kernel(const float *__
 constexpr int kBK = 320;       // reduction chunk
 constexpr int kBM = 32;        // rows per pass
 
+// One pass of up to kBM rows: returns sum_k X[m0 + lane, k] * W[n, k] in lanes < rows (0 for a column n >= N).  Every
+// thread of the CTA must call it (block barriers inside).
+__device__ __forceinline__ float batch_nt_pass(const float *__restrict__ X, const float *__restrict__ W, float *x_s,
+                                               float *w_s, int m0, int rows, int n, int N, int K, int vec) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  const int G = 32 / rows;                                     // lanes per row
+  const int mrow = lane % rows, part = lane / rows;            // part >= G: idle lane
+  float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+  for (int k0 = 0; k0 < K; k0 += kBK) {
+    const int kc = min(kBK, K - k0), kq = (kc + 3) >> 2;
+    __syncthreads();                                           // previous chunk consumed
+    if (vec) {                                                 // K % 4 == 0, 16 B aligned operands
+      for (int r = warp; r < rows; r += nwarps)
+        for (int q = lane; q < kq; q += 32)
+          *reinterpret_cast<float4 *>(x_s + r * (kBK + 4) + 4 * q) =
+              __ldcg(reinterpret_cast<const float4 *>(X + (size_t)(m0 + r) * K + k0) + q);   // (X: the predecessor's result)
+      for (int q = lane; q < kq; q += 32)
+        *reinterpret_cast<float4 *>(w_s + warp * kBK + 4 * q) =
+            n < N ? __ldg(reinterpret_cast<const float4 *>(W + (size_t)n * K + k0) + q) : make_float4(0.f, 0.f, 0.f, 0.f);
+    } else {                                                   // scalar staging, the chunk zero-padded to a quad
+      for (int r = warp; r < rows; r += nwarps)
+        for (int k = lane; k < 4 * kq; k += 32)
+          x_s[r * (kBK + 4) + k] = k < kc ? __ldcg(X + (size_t)(m0 + r) * K + k0 + k) : 0.f;
+      for (int k = lane; k < 4 * kq; k += 32)
+        w_s[warp * kBK + k] = (n < N && k < kc) ? __ldg(W + (size_t)n * K + k0 + k) : 0.f;
+    }
+    __syncthreads();
+    if (part < G) {
+      const float4 *xr = reinterpret_cast<const float4 *>(x_s + mrow * (kBK + 4));
+      const float4 *wr = reinterpret_cast<const float4 *>(w_s + warp * kBK);
+#pragma unroll 4
+      for (int q = part; q < kq; q += G) {
+        const float4 x = xr[q], w = wr[q];
+        a0 = fmaf(x.x, w.x, a0); a1 = fmaf(x.y, w.y, a1); a2 = fmaf(x.z, w.z, a2); a3 = fmaf(x.w, w.w, a3);
+      }
+    }
+  }
+  float v = (a0 + a1) + (a2 + a3);
+  for (int g = 1; g < G; ++g) {
+    const float o = __shfl_down_sync(0xffffffffu, v, g * rows);
+    if (lane < rows) v += o;
+  }
+  return v;
+}
+
 __global__ void __launch_bounds__(512) batch_nt_kernel(const float *__restrict__ X, const float *__restrict__ W,
                                                       const float *__restrict__ bias, float *__restrict__ out, int M,
                                                       int N, int K, int accumulate, int vec) {
   extern __shared__ __align__(16) float batch_smem[];
   float *x_s = batch_smem, *w_s = batch_smem + kBM * (kBK + 4);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
-  const int n = blockIdx.x * nwarps + warp;
+  const int lane = threadIdx.x & 31, n = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   pdl_wait();
   pdl_launch_dependents();
   for (int m0 = 0; m0 < M; m0 += kBM) {
     const int rows = min(kBM, M - m0);
-    const int G = 32 / rows;                                   // lanes per row
-    const int mrow = lane % rows, part = lane / rows;          // part >= G: idle lane
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-    for (int k0 = 0; k0 < K; k0 += kBK) {
-      const int kc = min(kBK, K - k0), kq = (kc + 3) >> 2;
-      __syncthreads();                                         // previous chunk consumed
-      if (vec) {                                               // K % 4 == 0, 16 B aligned operands
-        for (int r = warp; r < rows; r += nwarps)
-          for (int q = lane; q < kq; q += 32)
-            *reinterpret_cast<float4 *>(x_s + r * (kBK + 4) + 4 * q) =
-                __ldcg(reinterpret_cast<const float4 *>(X + (size_t)(m0 + r) * K + k0) + q);   // (X: the predecessor's result)
-        for (int q = lane; q < kq; q += 32)
-          *reinterpret_cast<float4 *>(w_s + warp * kBK + 4 * q) =
-              n < N ? __ldg(reinterpret_cast<const float4 *>(W + (size_t)n * K + k0) + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-      } else {                                                 // scalar staging, the chunk zero-padded to a quad
-        for (int r = warp; r < rows; r += nwarps)
-          for (int k = lane; k < 4 * kq; k += 32)
-            x_s[r * (kBK + 4) + k] = k < kc ? __ldcg(X + (size_t)(m0 + r) * K + k0 + k) : 0.f;
-        for (int k = lane; k < 4 * kq; k += 32)
-          w_s[warp * kBK + k] = (n < N && k < kc) ? __ldg(W + (size_t)n * K + k0 + k) : 0.f;
-      }
-      __syncthreads();
-      if (part < G) {
-        const float4 *xr = reinterpret_cast<const float4 *>(x_s + mrow * (kBK + 4));
-        const float4 *wr = reinterpret_cast<const float4 *>(w_s + warp * kBK);
-#pragma unroll 4
-        for (int q = part; q < kq; q += G) {
-          const float4 x = xr[q], w = wr[q];
-          a0 = fmaf(x.x, w.x, a0); a1 = fmaf(x.y, w.y, a1); a2 = fmaf(x.z, w.z, a2); a3 = fmaf(x.w, w.w, a3);
-        }
-      }
-    }
-    float v = (a0 + a1) + (a2 + a3);
-    for (int g = 1; g < G; ++g) {
-      const float o = __shfl_down_sync(0xffffffffu, v, g * rows);
-      if (lane < rows) v += o;
-    }
+    float v = batch_nt_pass(X, W, x_s, w_s, m0, rows, n, N, K, vec);
     if (lane < rows && n < N) {
       float *o = out + (size_t)(m0 + lane) * N + n;
       v += bias ? __ldg(bias + n) : 0.f;
       *o = accumulate ? __ldcg(o) + v : v;
     }
   }
+}
+
+// Scheduled sampling (model/e2e_decoder.py:123-127): tok[m] = argmax_n (X[m,:] . W[n,:] + bias[n]) when *flag != 0, the
+// product of batch_nt_kernel without writing the logits.  A row's winner is the largest 64-bit key
+//   (order-preserving bits of v + 0.0f) << 32 | (0xFFFFFFFF - n)
+// -- larger value first, lower index on equal values, -0 == +0 -- so one atomicMax per (CTA, row) into ws[m] gives an exact
+// result whatever order the CTAs finish in.  The last CTA to finish (fence + counter ws[M]) turns the keys into tokens and
+// leaves ws zero again: the kernel needs no memset node in a CUDA graph.
+__device__ __forceinline__ unsigned long long argmax_key(float v, int n) {
+  uint32_t u = __float_as_uint(v + 0.0f);
+  u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((unsigned long long)u << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)n);
+}
+
+__global__ void __launch_bounds__(512) sample_tokens_kernel(const float *__restrict__ X, const float *__restrict__ W,
+                                                           const float *__restrict__ bias, const int32_t *__restrict__ flag,
+                                                           int32_t *__restrict__ tok, unsigned long long *ws, int M,
+                                                           int N, int K, int vec) {
+  extern __shared__ __align__(16) float batch_smem[];
+  __shared__ unsigned long long key_s[kBM];
+  __shared__ int last_s;
+  float *x_s = batch_smem, *w_s = batch_smem + kBM * (kBK + 4);
+  const int tid = threadIdx.x, lane = tid & 31, n = blockIdx.x * (blockDim.x >> 5) + (tid >> 5);
+  if (__ldcg(flag) == 0) return;                               // teacher token: tok[] stays as the caller filled it
+  for (int m0 = 0; m0 < M; m0 += kBM) {
+    const int rows = min(kBM, M - m0);
+    if (tid < kBM) key_s[tid] = 0ull;                          // (ordered before the atomics by the pass's barriers)
+    const float v = batch_nt_pass(X, W, x_s, w_s, m0, rows, n, N, K, vec);
+    if (lane < rows && n < N) atomicMax(&key_s[lane], argmax_key(v + (bias ? __ldg(bias + n) : 0.f), n));
+    __syncthreads();
+    if (tid < rows) atomicMax(ws + m0 + tid, key_s[tid]);
+  }
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last_s = atomicAdd(ws + M, 1ull) == (unsigned long long)(gridDim.x - 1);
+  __syncthreads();
+  if (!last_s) return;
+  __threadfence();
+  for (int m = tid; m < M; m += blockDim.x) tok[m] = (int32_t)(0xFFFFFFFFu - (uint32_t)atomicExch(ws + m, 0ull));
+  if (tid == 0) atomicExch(ws + M, 0ull);
 }
 
 // ---- one LSTMCell position per launch -----------------------------------------------------------------------------
@@ -357,6 +406,22 @@ extern "C" int re2e_batch_nt(const float *X, const float *W, const float *bias, 
                              static_cast<cudaStream_t>(stream), X, W, bias, out, M, N, K, accumulate, vec);
   count_launch();
   return e == cudaSuccess ? launch_status() : (int)e;
+}
+
+extern "C" int re2e_sample_tokens_ws_bytes(int M) { return M > 0 ? (int)sizeof(unsigned long long) * (M + 1) : 0; }
+
+extern "C" int re2e_sample_tokens(const float *X, const float *W, const float *bias, const int32_t *flag, int32_t *tok,
+                                  unsigned long long *ws, int M, int N, int K, void *stream) {
+  RE2E_CHECK_ARG(X && W && flag && tok && ws && M > 0 && N > 0 && K > 0);
+  const int vec = !(K & 3) && aligned16(X) && aligned16(W);
+  const int cols = N >= 2048 ? 16 : 8;
+  const size_t smem = sizeof(float) * (kBM * (kBK + 4) + cols * kBK);
+  int rc = ensure_smem(reinterpret_cast<const void *>(sample_tokens_kernel), smem);
+  if (rc != RE2E_OK) return rc;
+  sample_tokens_kernel<<<(N + cols - 1) / cols, cols * 32, smem, static_cast<cudaStream_t>(stream)>>>(X, W, bias, flag, tok,
+                                                                                                  ws, M, N, K, vec);
+  count_launch();
+  return launch_status();
 }
 
 extern "C" int re2e_lstm_step_supported(int B, int D, int Z) {

@@ -6,10 +6,16 @@ state_dict keys as the reference's ``Decoder`` for the configuration the scripts
 
 * ``forward(hpad, hlen, ys, scheduled_sampling_rate)`` -- the training loop of model/e2e_decoder.py:79-167:
   AttLoc step kernel per output position with the alignment fed back un-detached, teacher forcing or scheduled
-  sampling, cross-entropy rescaled by ``mean(len(ys_in)) - 1``.  With teacher forcing the output layer of all positions
-  is ONE product on the tcgen05 GEMM after the loop; the LSTMCell and the cross-entropy are library ops.  The decoder
-  state fed to step i depends on the context of step i-1 through the LSTMCell, so this loop calls the per-step AttLoc
-  kernels (``AttLoc.forward_loop``, the persistent loop kernels, needs the states of all steps up front).
+  sampling, cross-entropy rescaled by ``mean(len(ys_in)) - 1``.  The output layer of all positions is ONE product on the
+  tcgen05 GEMM after the loop, the first LSTMCell is one cluster kernel per position (lstm.py) and the cross-entropy
+  runs on the library's kernels.  The decoder state fed to step i depends on the context of step i-1 through the
+  LSTMCell, so this loop calls the per-step AttLoc kernels (``AttLoc.forward_loop``, the persistent loop kernels, needs
+  the states of all steps up front).  Scheduled sampling (rate > 0) keeps that shape: the reference's one
+  ``random.random()`` per position is drawn before the loop, the flags reach the device through a page-locked buffer,
+  and a flagged position's token -- the arg-max of the previous position's logits -- is chosen on the device by
+  ``re2e_sample_tokens`` (the logits are never written) into the token buffer the LSTM step looks its embedding half up
+  from.  No host round trip, so the forward + backward can be captured once and replayed with new draws
+  (``draw_sampling``).  ``fused_lstm = False`` or a CPU module runs the reference's own loop.
 * ``recognize_beam(h, lpz, recog_args, char_list, rnnlm=None, fstlm=None)`` -- hybrid CTC/attention beam search
   (model/e2e_decoder.py:170-369) re-designed for the GPU: ALL live hypotheses advance together (B = beam instead of
   beam x (B = 1) calls) and the whole output position runs on the device as SIX launches of the library over static
@@ -347,20 +353,42 @@ class Decoder(torch.nn.Module):
         att_w = None
         y_all = []
         self.att.reset()
-        eys = self.embed(pad_ys_in)
         y_i = None
+        fused = self.fused_lstm and dev.type == 'cuda'
+        sampling = scheduled_sampling_rate > 0.0
         # Teacher forcing (scheduled_sampling_rate == 0, the scripts' default): no step ever looks at its own output
         # distribution, so the output layer of ALL positions is one dense product after the loop (tcgen05 3xTF32 GEMM,
         # (B*olength) x odim x dunits) instead of olength skinny ones inside it -- same values as model/e2e_decoder.py:150.
-        batched_output = scheduled_sampling_rate <= 0.0
-        # ... and the embedding half of the first LSTMCell's input product is one dense product before the loop; per
-        # position only the context / state products (batch-sized) and one fused pointwise kernel remain (lstm.py)
-        lstm0 = LSTMLoop(self.decoder[0], eys) if (batched_output and self.fused_lstm and dev.type == 'cuda') else None
+        # With scheduled sampling the fused loop keeps that product after the loop too: a sampled position only needs
+        # the previous position's arg-max, which re2e_sample_tokens takes from the top-layer state on the device.
+        batched_output = fused or not sampling
+        if fused and sampling:
+            # the embedding half is looked up by token from a per-token table; tok (olength, B) starts as the teacher
+            # tokens and a flagged position i >= 1 overwrites row i with the previous position's arg-max
+            flags = self._sampling_flags(olength, scheduled_sampling_rate, dev)
+            tok = pad_ys_in.t().to(torch.int32).contiguous()
+            lstm0 = LSTMLoop.by_token(self.decoder[0], self.embed.weight, tok)
+            w_out, b_out = _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach())
+            ws = self._sampling_ws(batch, dev)
+            self._ss_tokens = tok
+        else:
+            eys = self.embed(pad_ys_in)
+            # ... and the embedding half of the first LSTMCell's input product is one dense product before the loop; per
+            # position only the context / state products (batch-sized) and one fused pointwise kernel remain (lstm.py)
+            lstm0 = LSTMLoop(self.decoder[0], eys) if (fused and not sampling) else None
         z_top = []
         for i in range(olength):
             att_c, att_w = self.att(hpad, hlen, z_list[0], att_w)
             if lstm0 is not None:
-                random.random()                                  # (the reference draws one number per position)
+                if not sampling:
+                    random.random()                              # (the reference draws one number per position)
+                elif i > 0:                                      # (the draws were taken up front, see _sampling_flags)
+                    zt = _lib.f32c(z_list[-1].detach())
+                    with _lib.on(dev):
+                        _lib.check(_lib.lib().re2e_sample_tokens(_lib.ptr(zt), _lib.ptr(w_out), _lib.ptr(b_out),
+                                                                 _lib.ptr(flags[i]), _lib.ptr(tok[i]), _lib.ptr(ws), batch,
+                                                                 w_out.size(0), w_out.size(1), _lib.stream_ptr()),
+                                   "re2e_sample_tokens")
                 z_list[0], c_list[0] = lstm0.step(i, att_c, z_list[0], c_list[0])
             else:
                 if random.random() < scheduled_sampling_rate and i > 0:
@@ -396,6 +424,44 @@ class Decoder(torch.nn.Module):
             loss_reg = -torch.sum((F.log_softmax(y_all, dim=1) * self.vlabeldist).view(-1), dim=0) / len(ys_in_lens)
             self.loss = (1. - self.lsm_weight) * self.loss + self.lsm_weight * loss_reg
         return self.loss, acc
+
+    def _sampling_flags(self, olength, rate, dev):
+        """Device int32 (olength,) flags of one scheduled-sampling forward: flag i = (draw_i < rate and i > 0), with the
+        olength draws of random.random() taken here, in the reference's order (one per position, position 0 included).
+        They travel through a page-locked buffer, so a captured graph re-reads it at every replay (draw_sampling)."""
+        pin = torch.empty(olength, dtype=torch.int32).pin_memory()
+        self._fill_flags(pin, rate)
+        if torch.cuda.is_current_stream_capturing():
+            # kept for the module's life: the graph re-reads `pin` at every replay, and freeing the previous buffer
+            # inside the capture would record its reuse event into the graph (torch's page-locked allocator then fails
+            # on its next allocation)
+            self.__dict__.setdefault("_ss_pins", []).extend(p for p in (getattr(self, "_ss_flags", None), pin)
+                                                            if p is not None)
+        self._ss_flags = pin
+        return pin.to(dev, non_blocking=True)
+
+    @staticmethod
+    def _fill_flags(pin, rate):
+        pin.numpy()[:] = [1 if (random.random() < rate and i > 0) else 0 for i in range(pin.numel())]
+
+    def _sampling_ws(self, batch, dev):
+        """Scratch of re2e_sample_tokens: zero when allocated, left zero by every call, so it is kept across forwards."""
+        ws = getattr(self, "_ss_ws", None)
+        n = (int(_lib.lib().re2e_sample_tokens_ws_bytes(batch)) + 7) // 8
+        if ws is None or ws.device != dev or ws.numel() < n:
+            ws = self._ss_ws = torch.zeros(n, dtype=torch.int64, device=dev)
+        return ws
+
+    def draw_sampling(self, scheduled_sampling_rate):
+        """New draws for the most recent scheduled-sampling forward (the one a captured CUDA graph replays): one
+        random.random() per position, exactly as an eager forward at this rate would take them.  Waits for the device
+        first, so a replay still in flight keeps the flags it started with.  A job that ramps the rate up captures the
+        forward + backward once (at a rate > 0) and calls ``draw_sampling(rate_k)`` before each replay."""
+        pin = getattr(self, "_ss_flags", None)
+        if pin is None:
+            raise RuntimeError("draw_sampling: no scheduled-sampling forward has run on this decoder")
+        torch.cuda.synchronize(self.embed.weight.device)
+        self._fill_flags(pin, scheduled_sampling_rate)
 
     # ------------------------------------------------------------------------------------------ beam search
     @torch.no_grad()
