@@ -272,6 +272,25 @@ int re2e_ctc_loss_bwd(const float *logits, long long stride_b, long long stride_
                       const void *ws, size_t ws_bytes, float *grad, int B, int Th, int V, int Umax,
                       void *stream);
 
+/* Forced alignment: the single most likely path of each transcript through its blank-interleaved lattice (Viterbi,
+ * max-plus forward recursion + backtrace on the device; no reference counterpart).  Inputs as re2e_ctc_loss_fwd, the
+ * same workspace (re2e_ctc_ws_bytes); logits may also be log-probabilities (a per-frame constant does not move the path).
+ * Two launches (the loss's log-sum-exp / lattice gather, then one warp per utterance); no host synchronisation.
+ *   states (B,Th) int32   lattice state s in [0, 2U] of every frame (even = blank, odd 2u+1 = label u)
+ *   tokens (B,Th) int32   blank or labels[u] for that state
+ *   spans (B,Umax,2)      first and last frame of each label
+ *   score (B) fp32        log-probability of the path under softmax(logits)
+ * Tie rule: on equal scores a state prefers staying (s), then s-1, then s-2; at the last frame S-1 (final blank) is
+ * preferred to S-2.  Frames t >= min(input_lens[b], Th), labels u >= label_lens[b] and every entry of an infeasible
+ * utterance (input_lens[b] < U + adjacent repeats) are -1; an infeasible utterance scores -inf.  U = 0 gives the all-blank
+ * path; input_lens[b] <= 0 gives score 0 if U = 0, else -inf.
+ * Umax <= 255 and Th up to ~1550..1680 (the backpointers, 128 B per frame, live in shared memory), else
+ * RE2E_E_UNSUPPORTED before anything is launched. */
+int re2e_ctc_align(const float *logits, long long stride_b, long long stride_t, const int32_t *labels,
+                   const int32_t *label_offs, const int32_t *label_lens, const int32_t *input_lens, int blank,
+                   int32_t *states, int32_t *tokens, int32_t *spans, float *score, void *ws, size_t ws_bytes, int B,
+                   int Th, int V, int Umax, void *stream);
+
 /* out = log_softmax(logits, dim=-1) over rows of length V (e2e_ctc.py:68-75 after ctc_lo);
  * best (optional, int32 per row) = argmax_v  ("CTC best-path alignment", lowest index on ties). */
 int re2e_log_softmax(const float *logits, float *out, int32_t *best, long long rows, int V,

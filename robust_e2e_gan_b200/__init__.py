@@ -13,7 +13,7 @@ CPU, Triton or PyTorch fallback -- calls raise if the library or the GPU is miss
 from .feat_model import FbankModel, FFTModel, fbank, masked_fbank, apply_mask  # noqa: F401
 from .e2e_attention import AttLoc  # noqa: F401
 from .e2e_ctc import (CTC, CTCPrefixScore, PreparedTargets, prepare_targets, ctc_loss,  # noqa: F401
-                      log_softmax_rows, ctc_prefix_score_batch)
+                      log_softmax_rows, ctc_prefix_score_batch, ctc_forced_align, CTCAlignment)
 from .e2e_decoder import Decoder  # noqa: F401
 from .parallel import GradBuckets, init_distributed, shard_range  # noqa: F401
 

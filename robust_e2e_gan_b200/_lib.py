@@ -72,6 +72,7 @@ SIGNATURES = {
     "re2e_ctc_ws_bytes": (_SZ, [_I, _I, _I, _I]),
     "re2e_ctc_loss_fwd": (_I, [_P, _LL, _LL, _P, _P, _P, _P, _I, _P, _P, _P, _SZ, _I, _I, _I, _I, _P]),
     "re2e_ctc_loss_bwd": (_I, [_P, _LL, _LL, _P, _P, _P, _P, _I, _P, _P, _P, _SZ, _P, _I, _I, _I, _I, _P]),
+    "re2e_ctc_align": (_I, [_P, _LL, _LL, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _SZ, _I, _I, _I, _I, _P]),
     "re2e_log_softmax": (_I, [_P, _P, _P, _LL, _I, _P]),
     "re2e_ctc_prefix_score": (_I, [_P] * 7 + [_I] * 6 + [_P]),
 }

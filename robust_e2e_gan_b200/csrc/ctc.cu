@@ -13,6 +13,8 @@
 //                      in fp64, so |alpha| stays O(100) and fp32 rounding does not grow with T
 //                      (plain fp32 log-domain CTC loses ~1e-4 at |alpha| ~ 1e3).
 //   ctc_grad_kernel  : one warp per frame; grad = gscale * (softmax - occupancy), written once.
+// Forced alignment (re2e_ctc_align) is ctc_lse_kernel followed by ctc_viterbi_warp_kernel: the forward recursion in the
+// max-plus semiring with 2-bit backpointers in shared memory and an on-device backtrace.
 // Algorithmic bytes: 4*V per valid frame (lse) + 2*4*V per frame (grad read + write).
 #include <math_constants.h>
 
@@ -451,6 +453,180 @@ ctc_ab_kernel(const float *__restrict__ lpc, const float *__restrict__ lpmax,
 }
 
 // ---------------------------------------------------------------------------------------------
+// Forced alignment: the Viterbi path through the blank-interleaved lattice of a GIVEN transcript, i.e. the forward half
+// of ctc_ab_warp_kernel in the max-plus semiring plus backpointers and a backtrace.  One CTA of one warp per utterance,
+// lane l owns states [l*SPL, (l+1)*SPL) in registers, lp rows prefetched through the same cp.async ring.
+//   v_t(s) = max(v(s), v(s-1), skip ? v(s-2) : -inf) + lp_t(s)        (no transcendental functions)
+// Tie rule (also the oracle's, oracle/ctc_align.py ctc_viterbi): on equal values stay in s, then come from s-1, then from s-2;
+// at the end take S-1 (final blank) over S-2.  As in alpha / beta, every frame is shifted by its lpmax and the column is
+// renormalised every kRenorm frames (offsets in fp64): each subtracts one constant from all states, which keeps |v| and
+// hence fp32 rounding small over long utterances and never reverses the order of two states.
+// Backpointers: 2 bits per state (0 stay, 1 from s-1, 2 from s-2), one uint32 per lane and frame in dynamic shared
+// memory (128 B per frame).  After the last frame lane 0 walks them back from the chosen end state and leaves the state
+// of frame t in the same array; the warp then writes states / tokens / spans in parallel over frames.
+template <int SPL>
+struct ViterbiSmem {
+  static constexpr int kRing = SPL <= 4 ? 32 : 16, kAhead = kRing - 8, kSlot = 32 * SPL + 1;
+  static constexpr size_t ring_bytes = sizeof(float) * kRing * kSlot;    // multiple of 4 B: bp words follow directly
+  static size_t bytes(int Th) { return ring_bytes + sizeof(uint32_t) * 32 * (size_t)Th; }
+};
+
+template <int SPL>
+__global__ void __launch_bounds__(32)
+ctc_viterbi_warp_kernel(const float *__restrict__ lpc, const float *__restrict__ lpmax,
+                        const int32_t *__restrict__ labels, const int32_t *__restrict__ label_offs,
+                        const int32_t *__restrict__ label_lens, const int32_t *__restrict__ input_lens, int blank,
+                        int32_t *__restrict__ states, int32_t *__restrict__ tokens, int32_t *__restrict__ spans,
+                        float *__restrict__ score, int Th, int Smax, int Umax) {
+  static_assert(SPL <= 16, "2-bit backpointers of one lane must fit one uint32");
+  using L = ViterbiSmem<SPL>;
+  constexpr int kRing = L::kRing, kAhead = L::kAhead, kSlot = L::kSlot;
+  extern __shared__ __align__(16) float vsm[];
+  float *ring = vsm;                                                    // [kRing][32*SPL states | frame max]
+  uint32_t *bp = reinterpret_cast<uint32_t *>(vsm + kRing * kSlot);     // [Th][32 lanes]
+  const int b = blockIdx.x, lane = threadIdx.x;
+  const int T = min(Th, max(0, __ldg(input_lens + b)));
+  const int U = __ldg(label_lens + b), S = 2 * U + 1;
+  const int32_t *lab = labels + __ldg(label_offs + b);
+  const float NEG = -CUDART_INF_F;
+  const unsigned FULL = 0xffffffffu;
+  const int s0 = lane * SPL;
+  uint32_t live = 0, skip = 0, start = 0;                               // one bit per state of this lane
+#pragma unroll
+  for (int k = 0; k < SPL; ++k) {
+    const int s = s0 + k;
+    if (s < S) {
+      live |= 1u << k;
+      if ((s & 1) && s >= 3 && __ldg(lab + (s >> 1)) != __ldg(lab + (s >> 1) - 1)) skip |= 1u << k;
+      if (s < 2) start |= 1u << k;
+    }
+  }
+  const float *lp_b = lpc + (size_t)b * Th * Smax;
+  const float *src_p = lp_b + s0;               // frame being ISSUED (advances with the loop)
+  const float *srcm_p = lpmax + (size_t)b * Th;
+  auto issue_frame = [&](int i) {
+    if (i < T) {
+      float *dst = ring + (i & (kRing - 1)) * kSlot;
+#pragma unroll
+      for (int k = 0; k < SPL; ++k)
+        if ((live >> k) & 1u) cp_async4(dst + s0 + k, src_p + k);
+      if (lane == 0) cp_async4(dst + 32 * SPL, srcm_p);
+    }
+    src_p += Smax;
+    srcm_p += 1;
+    cp_async_commit();
+  };
+  // states beyond the lattice are never copied and read as -inf for the whole run
+#pragma unroll
+  for (int k = 0; k < SPL; ++k)
+    if (!((live >> k) & 1u))
+      for (int r = 0; r < kRing; ++r) ring[r * kSlot + s0 + k] = NEG;
+  __syncwarp();
+  for (int i = 0; i < kAhead; ++i) issue_frame(i);
+  double off = 0.0;
+  float a[SPL];
+#pragma unroll
+  for (int k = 0; k < SPL; ++k) a[k] = NEG;
+  uint32_t *bp_p = bp + lane;
+#pragma unroll 2
+  for (int i = 0; i < T; ++i) {
+    issue_frame(i + kAhead);
+    cp_async_wait<kAhead>();
+    __syncwarp();                                   // lane 0's copy of the frame max is visible to the warp
+    const float *fr = ring + (i & (kRing - 1)) * kSlot;
+    const float lpm = fr[32 * SPL];
+    if (lane == 0) off += (double)lpm;
+    float n1 = __shfl_up_sync(FULL, a[SPL - 1], 1);
+    float n2 = SPL >= 2 ? __shfl_up_sync(FULL, a[SPL >= 2 ? SPL - 2 : 0], 1) : __shfl_up_sync(FULL, a[0], 2);
+    if (lane == 0) { n1 = NEG; n2 = NEG; }
+    if (SPL == 1 && lane == 1) n2 = NEG;
+    float v[SPL];
+    uint32_t word = 0;
+#pragma unroll
+    for (int k = 0; k < SPL; ++k) {
+      const float x1 = k >= 1 ? a[k >= 1 ? k - 1 : 0] : n1;
+      const float x2 = k >= 2 ? a[k >= 2 ? k - 2 : 0] : (k == 1 ? n1 : n2);
+      float m = a[k];
+      uint32_t d = 0;
+      if (x1 > m) { m = x1; d = 1; }                                  // strict: ties stay
+      if (((skip >> k) & 1u) && x2 > m) { m = x2; d = 2; }            // strict: ties come from s-1
+      word |= d << (2 * k);
+      const float lpv = fr[s0 + k] - lpm;                             // -inf for states outside the lattice
+      // frame 0: the column is -inf everywhere and the start states are seeded instead
+      v[k] = i == 0 ? (((start >> k) & 1u) ? lpv : NEG) : m + lpv;
+    }
+    *bp_p = word;
+    bp_p += 32;
+    if ((i & (kRenorm - 1)) == kRenorm - 1) {
+      float m = v[0];
+#pragma unroll
+      for (int k = 1; k < SPL; ++k) m = fmaxf(m, v[k]);
+      m = warp_max(m);
+      if (m != NEG) {
+#pragma unroll
+        for (int k = 0; k < SPL; ++k) v[k] -= m;
+        if (lane == 0) off += (double)m;
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < SPL; ++k) a[k] = v[k];
+    __syncwarp();   // every lane is done with this ring slot before it is refilled kRing - kAhead frames later
+  }
+  // final column -> shared memory (the ring is idle: every issued copy belonged to a frame < T and has landed)
+#pragma unroll
+  for (int k = 0; k < SPL; ++k) ring[s0 + k] = a[k];
+  __syncwarp();
+  int feasible = 0;
+  if (lane == 0) {
+    float sc;
+    if (T == 0) {
+      sc = U == 0 ? 0.0f : NEG;
+    } else {
+      const float x = ring[S - 1], y = S > 1 ? ring[S - 2] : NEG;
+      int s = y > x ? S - 2 : S - 1;                                    // ties: final blank
+      const float e = fmaxf(x, y);
+      if (e == NEG) {
+        sc = NEG;
+      } else {
+        sc = (float)(off + (double)e);
+        feasible = 1;
+        // serial walk; the state of frame t replaces word t % 32 of frame t once that frame has been read (a bank
+        // per lane for the parallel pass below)
+        for (int t = T - 1; t >= 0; --t) {
+          const uint32_t w = bp[t * 32 + s / SPL];
+          bp[t * 32 + (t & 31)] = (uint32_t)s;
+          if (t > 0) s -= (int)((w >> (2 * (s % SPL))) & 3u);
+        }
+      }
+    }
+    score[b] = sc;
+  }
+  feasible = __shfl_sync(FULL, feasible, 0);   // also orders lane 0's shared-memory writes before the reads below
+  __syncwarp();
+  int32_t *st_b = states + (size_t)b * Th, *tk_b = tokens + (size_t)b * Th;
+  int32_t *sp_b = spans + (size_t)b * Umax * 2;
+  const int Tv = feasible ? T : 0;
+  for (int t = lane; t < Th; t += 32) {
+    int s = -1, tok = -1;
+    if (t < Tv) {
+      s = (int)bp[t * 32 + (t & 31)];
+      tok = (s & 1) ? __ldg(lab + (s >> 1)) : blank;
+      if (s & 1) {      // every label state is visited by one run of frames: its ends are written exactly once
+        const int u = s >> 1;
+        if (t == 0 || (int)bp[(t - 1) * 32 + ((t - 1) & 31)] != s) sp_b[2 * u] = t;
+        if (t == Tv - 1 || (int)bp[(t + 1) * 32 + ((t + 1) & 31)] != s) sp_b[2 * u + 1] = t;
+      }
+    }
+    st_b[t] = s;
+    tk_b[t] = tok;
+  }
+  for (int u = (feasible ? U : 0) + lane; u < Umax; u += 32) {
+    sp_b[2 * u] = -1;
+    sp_b[2 * u + 1] = -1;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
 ctc_grad_kernel(const float *__restrict__ logits, long long stride_b, long long stride_t,
                 const int32_t *__restrict__ labels, const int32_t *__restrict__ label_offs,
@@ -771,6 +947,59 @@ extern "C" int re2e_ctc_loss_bwd(const float *logits, long long stride_b, long l
       w.lpc, w.alpha, w.beta, w.offA, w.offB, grad, B, Th, V, Smax, vec_ok);
   count_launch();
   return launch_status();
+}
+
+namespace re2e {
+namespace {
+template <int SPL>
+int launch_viterbi(const CtcWs &w, const int32_t *labels, const int32_t *label_offs, const int32_t *label_lens,
+                   const int32_t *input_lens, int blank, int32_t *states, int32_t *tokens, int32_t *spans, float *score,
+                   int B, int Th, int Smax, int Umax, cudaStream_t st) {
+  const size_t smem = ViterbiSmem<SPL>::bytes(Th);
+  ctc_viterbi_warp_kernel<SPL><<<B, 32, smem, st>>>(w.lpc, w.lpmax, labels, label_offs, label_lens, input_lens, blank,
+                                                    states, tokens, spans, score, Th, Smax, Umax);
+  count_launch();
+  return launch_status();
+}
+// the backpointers of the whole utterance live in shared memory: 128 B per frame next to the prefetch ring
+template <int SPL>
+int prepare_viterbi(int Th) {
+  const size_t smem = ViterbiSmem<SPL>::bytes(Th);
+  if (smem > 227 * 1024) return RE2E_E_UNSUPPORTED;
+  return ensure_smem(reinterpret_cast<const void *>(&ctc_viterbi_warp_kernel<SPL>), smem);
+}
+}  // namespace
+}  // namespace re2e
+
+extern "C" int re2e_ctc_align(const float *logits, long long stride_b, long long stride_t, const int32_t *labels,
+                              const int32_t *label_offs, const int32_t *label_lens, const int32_t *input_lens, int blank,
+                              int32_t *states, int32_t *tokens, int32_t *spans, float *score, void *ws, size_t ws_bytes,
+                              int B, int Th, int V, int Umax, void *stream) {
+  RE2E_CHECK_ARG(logits && labels && label_offs && label_lens && input_lens && states && tokens && score && ws);
+  RE2E_CHECK_ARG(B > 0 && Th > 0 && V > 0 && Umax >= 0 && blank >= 0 && blank < V && (spans || Umax == 0));
+  if (Umax > 255) return RE2E_E_UNSUPPORTED;       // the loss's limit: Smax <= 511, at most 16 states per lane
+  const int Smax = 2 * Umax + 1;
+  const int spl = (Smax + 31) / 32;
+  // every shape check comes before the first launch
+#define RE2E_VIT(F)                                                                                                  \
+  (spl <= 1 ? F<1> : spl == 2 ? F<2> : spl == 3 ? F<3> : spl == 4 ? F<4> : spl <= 6 ? F<6> : spl <= 8 ? F<8>         \
+   : spl <= 12 ? F<12> : F<16>)
+  int rc = RE2E_VIT(prepare_viterbi)(Th);
+  if (rc != RE2E_OK) return rc;
+  CtcWs w = carve(ws, B, Th, Smax);
+  if (ws_bytes < w.bytes) return RE2E_E_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long rows = (long long)B * Th;
+  const int grid = (int)((rows + kWarpsPerCta - 1) / kWarpsPerCta);
+  ctc_lse_kernel<<<grid, kWarpsPerCta * 32, 0, st>>>(logits, stride_b, stride_t, labels, label_offs, label_lens,
+                                                     input_lens, blank, w.lse, w.lpmax, w.lpc, B, Th, V, Smax);
+  count_launch();
+  rc = launch_status();
+  if (rc != RE2E_OK) return rc;
+  rc = RE2E_VIT(launch_viterbi)(w, labels, label_offs, label_lens, input_lens, blank, states, tokens, spans, score, B, Th,
+                                Smax, Umax, st);
+#undef RE2E_VIT
+  return rc;
 }
 
 extern "C" int re2e_log_softmax(const float *logits, float *out, int32_t *best, long long rows, int V,

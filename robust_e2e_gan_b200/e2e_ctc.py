@@ -5,8 +5,11 @@
 loss = sum_b nll_b / B with blank = 0, and ``log_softmax(hs_pad)``.  The softmax + alpha/beta +
 gradient that the reference delegates to the third-party ``warpctc_pytorch`` (e2e_ctc.py:11,30,63)
 run in csrc/ctc.cu on the (B,Th,V) logits in place (no (Th,B,V) transpose copy).  Gradients follow
-autograd semantics (scaled by grad_output).
+autograd semantics (scaled by grad_output).  ``ctc_forced_align`` / ``CTC.forced_align`` add what the reference
+lacks: the forced (Viterbi) alignment of a given transcript, computed on the device.
 """
+import collections
+
 import numpy as np
 import torch
 import torch.nn.functional as F
@@ -92,18 +95,63 @@ def _strided_ok(t):
             and t.stride(1) >= t.shape[2] and t.stride(0) >= t.stride(1) * t.shape[1])
 
 
+def _device_hlens(hlens, dev):
+    """int32 CUDA lengths from host ints or a CUDA int tensor (the latter without a copy or a synchronisation)."""
+    if torch.is_tensor(hlens) and hlens.is_cuda:
+        return hlens.to(torch.int32).contiguous()
+    return torch.from_numpy(np.fromiter((int(h) for h in hlens), dtype=np.int32)).to(dev, non_blocking=True)
+
+
 def ctc_loss(logits, hlens, targets, blank=0):
     """logits (B,Th,V) raw activations on CUDA; hlens host ints (or int32 CUDA tensor);
     targets: PreparedTargets or anything prepare_targets accepts.  Returns (loss (1,), nll (B,))."""
     dev = logits.device
     if not isinstance(targets, PreparedTargets):
         targets = prepare_targets(targets, dev)
-    if torch.is_tensor(hlens) and hlens.is_cuda:
-        hl = hlens.to(torch.int32).contiguous()
-    else:
-        hl = torch.from_numpy(np.fromiter((int(h) for h in hlens), dtype=np.int32)).to(dev, non_blocking=True)
+    hl = _device_hlens(hlens, dev)
     assert targets.nutt == logits.shape[0] and hl.numel() == logits.shape[0]
     return _CTCLossFunction.apply(logits, hl, targets, blank)
+
+
+CTCAlignment = collections.namedtuple("CTCAlignment", ["states", "tokens", "spans", "score"])
+CTCAlignment.__doc__ = """Forced CTC alignment of a batch (``ctc_forced_align``); -1 marks padding and infeasible
+    utterances.
+    states (B,Th) int32  lattice state per frame (2u: blank before label u, 2u+1: label u)
+    tokens (B,Th) int32  blank id or the label emitted by that state
+    spans (B,Umax,2) int32  first and last frame of each label
+    score (B) fp32  log-probability of the path under softmax(logits) (-inf when no path exists)"""
+
+
+def ctc_forced_align(logits, hlens, targets, blank=0):
+    """Viterbi path of each transcript through its CTC lattice, on the device (csrc/ctc.cu ctc_viterbi_warp_kernel).
+    logits (B,Th,V) fp32 CUDA raw activations or log-probabilities (rows may be pitched, like the ctc_lo GEMM output);
+    hlens host ints or an int CUDA tensor (clamped to Th); targets: PreparedTargets or anything prepare_targets
+    accepts.  On equal scores a state stays, then comes from s-1, then from s-2; the path ends in the final blank
+    when that ties with the last label.  Returns CTCAlignment; takes no part in autograd.  With PreparedTargets and
+    device hlens the call never synchronises with the host and can be captured into a CUDA graph."""
+    L = _lib.lib()
+    dev = logits.device
+    if not isinstance(targets, PreparedTargets):
+        targets = prepare_targets(targets, dev)
+    hl = _device_hlens(hlens, dev)
+    x = logits.detach()
+    x = x if _strided_ok(x) else _lib.f32c(x)
+    B, Th, V = x.shape
+    assert targets.nutt == B and hl.numel() == B
+    umax = targets.umax
+    nbytes = int(L.re2e_ctc_ws_bytes(B, Th, V, umax))
+    ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+    states = torch.empty(B, Th, device=dev, dtype=torch.int32)
+    tokens = torch.empty(B, Th, device=dev, dtype=torch.int32)
+    spans = torch.empty(B, umax, 2, device=dev, dtype=torch.int32)
+    score = torch.empty(B, device=dev, dtype=torch.float32)
+    with _lib.on(dev):
+        _lib.check(L.re2e_ctc_align(_lib.ptr(x), x.stride(0), x.stride(1), _lib.ptr(targets.labels),
+                                    _lib.ptr(targets.offs), _lib.ptr(targets.lens), _lib.ptr(hl), int(blank),
+                                    _lib.ptr(states), _lib.ptr(tokens), _lib.ptr(spans) if umax else None,
+                                    _lib.ptr(score), _lib.ptr(ws), nbytes, B, Th, V, umax, _lib.stream_ptr()),
+                   "re2e_ctc_align")
+    return CTCAlignment(states, tokens, spans, score)
 
 
 def log_softmax_rows(logits, want_best=False):
@@ -149,6 +197,15 @@ class CTC(torch.nn.Module):
         dev = self.ctc_lo.weight.device
         with torch.no_grad():
             return log_softmax_rows(_linear_tc(hs_pad.to(dev), self.ctc_lo.weight, self.ctc_lo.bias))
+
+    def forced_align(self, hs_pad, hlens, ys_pad):
+        """Forced alignment of ys_pad (padded tensor with ignore_id, list of 1-D tensors or PreparedTargets) to
+        ctc_lo(hs_pad) without dropout; see ctc_forced_align.  Returns CTCAlignment."""
+        dev = self.ctc_lo.weight.device
+        tgt = ys_pad if isinstance(ys_pad, PreparedTargets) else prepare_targets(ys_pad, dev, self.ignore_id)
+        with torch.no_grad():
+            ys_hat = _linear_tc(hs_pad.to(dev), self.ctc_lo.weight, self.ctc_lo.bias)
+            return ctc_forced_align(ys_hat, hlens, tgt, blank=0)
 
     def best_path(self, hs_pad):
         """argmax_v log_softmax(ctc_lo(h))[b,t,:] -- the 'CTC alignment' of the north star."""
