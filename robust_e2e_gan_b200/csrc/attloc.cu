@@ -21,8 +21,6 @@
 // backward are register-blocked sliding-window FMAs (5 outputs per thread, K split 4 ways).
 #include <math_constants.h>
 
-#include <cstdlib>
-
 #include "attloc_common.cuh"
 
 namespace re2e {
@@ -49,7 +47,6 @@ __device__ __forceinline__ long long att_gtime() {
 #define ATT_MARK_T(which, slot, t)
 #endif
 
-constexpr int kDplMax = 16;   // D <= 512
 constexpr int kMaxStages = 30;
 
 struct AttGeom {
@@ -1280,65 +1277,20 @@ inline bool pick_geom_bwd(int B, int Th, int D, int A, int Z, int C, int K, int 
   }
 }
 
-template <typename Kern, typename Params>
-int launch_cluster(Kern kern, const Params &prm, int B, int CL, int threads, size_t smem, cudaStream_t st) {
-  int rc0 = ensure_smem(reinterpret_cast<const void *>(kern), smem);
-  if (rc0 != RE2E_OK) return rc0;
-  cudaError_t e;
-  if (CL > 8) {
-    e = cudaFuncSetAttribute(reinterpret_cast<const void *>(kern), cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e != cudaSuccess) return (int)e;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(B * CL));
-  cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  // programmatic dependent launch: the grid may start its prologue while the previous kernel of the stream drains
-  // (see pdl_wait()); RE2E_NO_PDL=1 in the environment restores plain stream order (debugging / A-B timing)
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
-  e = cudaLaunchKernelEx(&cfg, kern, prm);
-  count_launch();
-  return e == cudaSuccess ? RE2E_OK : (int)e;
-}
-
-#define ATT_DISPATCH(NAME, APLV, CPV, ...)                                              \
-  switch (APLV) {                                                                       \
-    case 1: rc = (CPV) == 10 ? NAME<1, 10> __VA_ARGS__ : NAME<1, 16> __VA_ARGS__; break; \
-    case 2: rc = (CPV) == 10 ? NAME<2, 10> __VA_ARGS__ : NAME<2, 16> __VA_ARGS__; break; \
-    case 4: rc = (CPV) == 10 ? NAME<4, 10> __VA_ARGS__ : NAME<4, 16> __VA_ARGS__; break; \
-    case 5: rc = (CPV) == 10 ? NAME<5, 10> __VA_ARGS__ : NAME<5, 16> __VA_ARGS__; break; \
-    case 8: rc = (CPV) == 10 ? NAME<8, 10> __VA_ARGS__ : NAME<8, 16> __VA_ARGS__; break; \
-    default: rc = RE2E_E_UNSUPPORTED;                                                   \
-  }
-
+// the step kernels are launched with programmatic dependent launch: the grid may start its prologue while the
+// previous kernel of the stream drains (see pdl_wait())
 template <int APL, int CP>
 int run_fwd(const AttFwdParams &prm, int CL, size_t smem, cudaStream_t st) {
+  const dim3 grid((unsigned)(prm.B * CL));
   // encoder channels per lane: the common D == A case gets an exact instantiation, anything else the general one
-  if (prm.D == prm.A) return launch_cluster(attloc_fwd_kernel<APL, CP, APL>, prm, prm.B, CL, kFT, smem, st);
-  return launch_cluster(attloc_fwd_kernel<APL, CP, kDpl>, prm, prm.B, CL, kFT, smem, st);
+  if (prm.D == prm.A) return launch_cluster(attloc_fwd_kernel<APL, CP, APL>, grid, dim3(kFT), smem, st, CL, true, prm);
+  return launch_cluster(attloc_fwd_kernel<APL, CP, kDpl>, grid, dim3(kFT), smem, st, CL, true, prm);
 }
 template <int APL, int CP>
 int run_bwd(const AttBwdParams &prm, int CL, size_t smem, cudaStream_t st) {
-  if (prm.D == prm.A) return launch_cluster(attloc_bwd_kernel<APL, CP, 2 * APL>, prm, prm.B, CL, kBT, smem, st);
-  return launch_cluster(attloc_bwd_kernel<APL, CP, 2 * kDpl>, prm, prm.B, CL, kBT, smem, st);
-}
-
-inline int check_dims(int B, int Th, int D, int A, int C, int K) {
-  if (B <= 0 || Th <= 0 || D <= 0 || A <= 0 || C <= 0 || K <= 0) return RE2E_E_ARG;
-  if ((K & 1) == 0) return RE2E_E_ARG;
-  if (A % 64 != 0 || A > 512 || (D & 3) || D > 32 * kDplMax || C > 16) return RE2E_E_UNSUPPORTED;
-  const int apl = A / 64;
-  if (!(apl == 1 || apl == 2 || apl == 4 || apl == 5 || apl == 8)) return RE2E_E_UNSUPPORTED;
-  return RE2E_OK;
+  const dim3 grid((unsigned)(prm.B * CL));
+  if (prm.D == prm.A) return launch_cluster(attloc_bwd_kernel<APL, CP, 2 * APL>, grid, dim3(kBT), smem, st, CL, true, prm);
+  return launch_cluster(attloc_bwd_kernel<APL, CP, 2 * kDpl>, grid, dim3(kBT), smem, st, CL, true, prm);
 }
 
 int skinny(bool nn, const float *X, const float *W, float *out, int M, int N, int Kd, int accumulate,

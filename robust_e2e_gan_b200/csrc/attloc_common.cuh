@@ -1,4 +1,4 @@
-// Device helpers shared by the AttLoc kernels (attloc.cu: one step per launch; attloc_loop.cu: the whole decoder
+// Helpers shared by the AttLoc kernels (attloc.cu: one step per launch; attloc_loop.cu: the whole decoder
 // loop in one persistent cluster kernel).  sm_100a only.
 #pragma once
 #include "common.cuh"
@@ -69,5 +69,26 @@ __device__ __forceinline__ void cluster_arrive_relaxed() {
   asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
 }
 
+// ---- host side ------------------------------------------------------------------------------
+// shapes both kernel families take: A = 64 * APL attention channels, D <= 512 encoder channels, C <= 16, odd K
+inline int check_dims(int B, int Th, int D, int A, int C, int K) {
+  if (B <= 0 || Th <= 0 || D <= 0 || A <= 0 || C <= 0 || K <= 0) return RE2E_E_ARG;
+  if ((K & 1) == 0) return RE2E_E_ARG;
+  if (A % 64 != 0 || A > 512 || (D & 3) || D > 512 || C > 16) return RE2E_E_UNSUPPORTED;
+  const int apl = A / 64;
+  if (!(apl == 1 || apl == 2 || apl == 4 || apl == 5 || apl == 8)) return RE2E_E_UNSUPPORTED;
+  return RE2E_OK;
+}
+
+// rc = NAME<APL, CP> ARGS for the instantiated (A / 64, C padded to 10 or 16) pairs
+#define ATT_DISPATCH(NAME, APLV, CPV, ...)                                              \
+  switch (APLV) {                                                                       \
+    case 1: rc = (CPV) == 10 ? NAME<1, 10> __VA_ARGS__ : NAME<1, 16> __VA_ARGS__; break; \
+    case 2: rc = (CPV) == 10 ? NAME<2, 10> __VA_ARGS__ : NAME<2, 16> __VA_ARGS__; break; \
+    case 4: rc = (CPV) == 10 ? NAME<4, 10> __VA_ARGS__ : NAME<4, 16> __VA_ARGS__; break; \
+    case 5: rc = (CPV) == 10 ? NAME<5, 10> __VA_ARGS__ : NAME<5, 16> __VA_ARGS__; break; \
+    case 8: rc = (CPV) == 10 ? NAME<8, 10> __VA_ARGS__ : NAME<8, 16> __VA_ARGS__; break; \
+    default: rc = RE2E_E_UNSUPPORTED;                                                   \
+  }
 
 }  // namespace re2e

@@ -879,15 +879,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-inline int loop_check_dims(int S, int B, int Th, int D, int A, int C, int K) {
-  if (S <= 0 || B <= 0 || Th <= 0 || D <= 0 || A <= 0 || C <= 0 || K <= 0) return RE2E_E_ARG;
-  if ((K & 1) == 0) return RE2E_E_ARG;
-  if (A % 64 != 0 || A > 512 || (D & 3) || D > 512 || C > 16) return RE2E_E_UNSUPPORTED;
-  const int apl = A / 64;
-  if (!(apl == 1 || apl == 2 || apl == 4 || apl == 5 || apl == 8)) return RE2E_E_UNSUPPORTED;
-  return RE2E_OK;
-}
-
 inline int pick_cl(int B, int Th) {
   const int sms = num_sms();
   int CL = 1;
@@ -948,48 +939,18 @@ inline bool loop_geom_bwd(int B, int Th, int D, int A, int C, int K, int CP, int
   }
 }
 
-template <typename Kern, typename Params>
-int launch_loop(Kern kern, const Params &prm, int B, int CL, size_t smem, cudaStream_t st) {
-  int rc0 = ensure_smem(reinterpret_cast<const void *>(kern), smem);
-  if (rc0 != RE2E_OK) return rc0;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(B * CL));
-  cfg.blockDim = dim3((unsigned)kLT);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, prm);
-  count_launch();
-  return e == cudaSuccess ? RE2E_OK : (int)e;
-}
-
-#define LOOP_DISPATCH(NAME, APLV, CPV, ...)                                             \
-  switch (APLV) {                                                                       \
-    case 1: rc = (CPV) == 10 ? NAME<1, 10> __VA_ARGS__ : NAME<1, 16> __VA_ARGS__; break; \
-    case 2: rc = (CPV) == 10 ? NAME<2, 10> __VA_ARGS__ : NAME<2, 16> __VA_ARGS__; break; \
-    case 4: rc = (CPV) == 10 ? NAME<4, 10> __VA_ARGS__ : NAME<4, 16> __VA_ARGS__; break; \
-    case 5: rc = (CPV) == 10 ? NAME<5, 10> __VA_ARGS__ : NAME<5, 16> __VA_ARGS__; break; \
-    case 8: rc = (CPV) == 10 ? NAME<8, 10> __VA_ARGS__ : NAME<8, 16> __VA_ARGS__; break; \
-    default: rc = RE2E_E_UNSUPPORTED;                                                   \
-  }
-
+// launched with programmatic dependent launch, like the step kernels
 template <int APL, int CP>
 int run_loop_fwd(const LoopFwdParams &prm, int CL, size_t smem, cudaStream_t st) {
-  if (prm.D == prm.A) return launch_loop(attloc_loop_fwd_kernel<APL, CP, APL>, prm, prm.B, CL, smem, st);
-  return launch_loop(attloc_loop_fwd_kernel<APL, CP, 8>, prm, prm.B, CL, smem, st);
+  const dim3 grid((unsigned)(prm.B * CL));
+  if (prm.D == prm.A) return launch_cluster(attloc_loop_fwd_kernel<APL, CP, APL>, grid, dim3(kLT), smem, st, CL, true, prm);
+  return launch_cluster(attloc_loop_fwd_kernel<APL, CP, 8>, grid, dim3(kLT), smem, st, CL, true, prm);
 }
 template <int APL, int CP>
 int run_loop_bwd(const LoopBwdParams &prm, int CL, size_t smem, cudaStream_t st) {
-  if (prm.D == prm.A) return launch_loop(attloc_loop_bwd_kernel<APL, CP, 2 * APL>, prm, prm.B, CL, smem, st);
-  return launch_loop(attloc_loop_bwd_kernel<APL, CP, 16>, prm, prm.B, CL, smem, st);
+  const dim3 grid((unsigned)(prm.B * CL));
+  if (prm.D == prm.A) return launch_cluster(attloc_loop_bwd_kernel<APL, CP, 2 * APL>, grid, dim3(kLT), smem, st, CL, true, prm);
+  return launch_cluster(attloc_loop_bwd_kernel<APL, CP, 16>, grid, dim3(kLT), smem, st, CL, true, prm);
 }
 
 }  // namespace
@@ -1005,8 +966,7 @@ extern "C" int re2e_loop_debug_read(long long *host_out, int which) {
 #endif
 
 extern "C" int re2e_attloc_loop_supported(int S, int B, int Th, int D, int A, int C, int K) {
-  int rc = loop_check_dims(S, B, Th, D, A, C, K);
-  if (rc != RE2E_OK) return 0;
+  if (S <= 0 || check_dims(B, Th, D, A, C, K) != RE2E_OK) return 0;
   const int CP = C == 10 ? 10 : 16;
   int CLf, CLb;
   size_t smem;
@@ -1017,7 +977,8 @@ extern "C" int re2e_attloc_loop_supported(int S, int B, int Th, int D, int A, in
 }
 
 extern "C" int re2e_attloc_loop_slots(int S, int B, int Th, int D, int A, int C, int K) {
-  int rc = loop_check_dims(S, B, Th, D, A, C, K);
+  RE2E_CHECK_ARG(S > 0);
+  int rc = check_dims(B, Th, D, A, C, K);
   if (rc != RE2E_OK) return rc;
   int CL;
   size_t smem;
@@ -1032,8 +993,8 @@ extern "C" int re2e_attloc_loop_fwd(const float *pre, const float *enc_h, const 
                                     const float *gvec, const float *gvec_b, float scaling, float *c_all,
                                     float *w_all, float *conv_all, int S, int B, int Th, int D, int A, int C,
                                     int K, void *stream) {
-  RE2E_CHECK_ARG(pre && enc_h && dec_proj && att_init && W_att && W_conv && gvec && gvec_b && c_all && w_all);
-  int rc = loop_check_dims(S, B, Th, D, A, C, K);
+  RE2E_CHECK_ARG(pre && enc_h && dec_proj && att_init && W_att && W_conv && gvec && gvec_b && c_all && w_all && S > 0);
+  int rc = check_dims(B, Th, D, A, C, K);
   if (rc != RE2E_OK) return rc;
   RE2E_CHECK_ARG(aligned16(pre) && aligned16(enc_h));
   const int CP = C == 10 ? 10 : 16;
@@ -1045,7 +1006,7 @@ extern "C" int re2e_attloc_loop_fwd(const float *pre, const float *enc_h, const 
   int CL;
   size_t smem;
   if (!loop_geom_fwd(B, Th, D, A, C, K, CP, CL, prm.g, smem)) return RE2E_E_UNSUPPORTED;
-  LOOP_DISPATCH(run_loop_fwd, A / 64, CP, (prm, CL, smem, static_cast<cudaStream_t>(stream)));
+  ATT_DISPATCH(run_loop_fwd, A / 64, CP, (prm, CL, smem, static_cast<cudaStream_t>(stream)));
   return rc;
 }
 
@@ -1056,8 +1017,8 @@ extern "C" int re2e_attloc_loop_bwd(const float *pre, const float *enc_h, const 
                                     float *d_decproj, float *acc_slots, int n_slots, int S, int B, int Th, int D,
                                     int A, int C, int K, void *stream) {
   RE2E_CHECK_ARG(pre && enc_h && dec_proj && att_init && w_all && conv_all && W_att && W_conv && gvec);
-  RE2E_CHECK_ARG(d_pre && d_decproj && acc_slots);
-  int rc = loop_check_dims(S, B, Th, D, A, C, K);
+  RE2E_CHECK_ARG(d_pre && d_decproj && acc_slots && S > 0);
+  int rc = check_dims(B, Th, D, A, C, K);
   if (rc != RE2E_OK) return rc;
   RE2E_CHECK_ARG(aligned16(d_pre));
   const int CP = C == 10 ? 10 : 16;
@@ -1071,6 +1032,6 @@ extern "C" int re2e_attloc_loop_bwd(const float *pre, const float *enc_h, const 
   size_t smem;
   if (!loop_geom_bwd(B, Th, D, A, C, K, CP, D == A ? 2 * (A / 64) : 16, CL, prm.g, smem)) return RE2E_E_UNSUPPORTED;
   if (n_slots < B * CL) return RE2E_E_WORKSPACE;
-  LOOP_DISPATCH(run_loop_bwd, A / 64, CP, (prm, CL, smem, static_cast<cudaStream_t>(stream)));
+  ATT_DISPATCH(run_loop_bwd, A / 64, CP, (prm, CL, smem, static_cast<cudaStream_t>(stream)));
   return rc;
 }

@@ -433,10 +433,9 @@ extern "C" int re2e_log_softmax_topk(const float *logits, long long rows, int V,
                                      int32_t *ids, void *stream) {
   RE2E_CHECK_ARG(logits && vals && ids && rows > 0 && V > 0 && k > 0 && k <= V);
   if (V > kTkThreads * kTkVPT || k > 32) return RE2E_E_UNSUPPORTED;
-  cudaError_t e = launch_pdl(2, log_softmax_topk_kernel, dim3((unsigned)rows), dim3(kTkThreads), 0,
-                             static_cast<cudaStream_t>(stream), logits, full, vals, ids, V, k);
+  log_softmax_topk_kernel<<<(unsigned)rows, kTkThreads, 0, static_cast<cudaStream_t>(stream)>>>(logits, full, vals, ids, V, k);
   count_launch();
-  return e == cudaSuccess ? launch_status() : (int)e;
+  return launch_status();
 }
 
 extern "C" int re2e_beam_joint(const float *att_top, const int32_t *ids, const float *log_psi, const float *psi_prev,
@@ -465,9 +464,9 @@ extern "C" int re2e_beam_advance(const float *att_top, const int32_t *ids, const
     RE2E_CHECK_ARG(src[s] && dst[s] && row_floats[s] > 0 && sub_count[s] >= 0);
     a.g.src[s] = src[s]; a.g.dst[s] = dst[s]; a.g.row_floats[s] = row_floats[s]; a.g.sub_count[s] = sub_count[s];
   }
-  cudaError_t e = launch_pdl(4, beam_advance_kernel, dim3(1), dim3(1024), 0, static_cast<cudaStream_t>(stream), a);
+  beam_advance_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(a);
   count_launch();
-  return e == cudaSuccess ? launch_status() : (int)e;
+  return launch_status();
 }
 
 extern "C" int re2e_beam_init(float *z_in, float *c_in, float *a_in, float *r_in, float *psi_in, const float *lpz,

@@ -4,7 +4,6 @@
 #include <stdint.h>
 
 #include <atomic>
-#include <cstdlib>
 #include <utility>
 
 #include "re2e_b200.h"
@@ -39,37 +38,34 @@ inline int launch_status() {
 
 int num_sms();   // SM count of the CURRENT device (cached per device); defined in api.cu
 
-// RE2E_NO_PDL=1 in the environment restores plain stream order (debugging / A-B timing)
-inline bool pdl_enabled() {
-  static const bool on = [] { const char *e = getenv("RE2E_NO_PDL"); return !(e && e[0] == '1'); }();
-  return on;
-}
-// Launch sites of launch_pdl() are opt-in, one bit each in RE2E_PDL_MASK (default 0 = plain stream order): measured on
-// the beam-search position (six short kernels in a strictly serial chain) programmatic launches made the chain SLOWER
-// (70.2 vs 63.3 us per position: the early-resident successors take SM slots from the running kernel and the graph
-// capture costs 1.5x), so they stay off; the kernels keep the discipline that makes them legal (pdl_wait() first,
-// coherent __ldcg loads for everything an overlapping predecessor may write -- ld.global.nc / __ldg returned stale
-// lines there).
-inline unsigned pdl_mask() {
-  static const unsigned m = [] { const char *e = getenv("RE2E_PDL_MASK"); return e ? (unsigned)strtoul(e, nullptr, 0) : 0u; }();
-  return m;
-}
-// Launch with programmatic stream serialisation: the grid may become resident while its predecessor in the stream is
-// still running.  EVERY kernel launched this way must execute pdl_wait() before it reads or writes anything the
+// Launch of a thread-block-cluster kernel in clusters of cluster_x CTAs along x; counts the launch.
+// pdl = true launches with programmatic stream serialisation: the grid may become resident while its predecessor in
+// the stream is still running, so the kernel must execute pdl_wait() before it reads or writes anything the
 // predecessor (or, transitively, anything earlier in the stream) may still touch.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(int id, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
+inline int launch_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster_x,
+                          bool pdl, Args &&...args) {
+  const void *fn = reinterpret_cast<const void *>(kern);
+  int rc = ensure_smem(fn, smem);
+  if (rc != RE2E_OK) return rc;
+  if (cluster_x > 8) RE2E_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = (unsigned)cluster_x;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl_enabled() && ((pdl_mask() >> id) & 1)) ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+  cfg.numAttrs = pdl ? 2 : 1;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+  count_launch();
+  return e == cudaSuccess ? RE2E_OK : (int)e;
 }
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }

@@ -1040,9 +1040,8 @@ extern "C" int re2e_ctc_prefix_score(const float *lpz, const float *r_prev, cons
   RE2E_CHECK_ARG(lpz && r_prev && cs && last && out_len && log_psi && r_new);
   RE2E_CHECK_ARG(T > 0 && V > 0 && H > 0 && Ccand > 0);
   const int n = H * Ccand;
-  cudaError_t e = launch_pdl(3, ctc_prefix_kernel, dim3((unsigned)((n + kPrefixWarps - 1) / kPrefixWarps)),
-                             dim3(kPrefixWarps * 32), 0, static_cast<cudaStream_t>(stream), lpz, r_prev, cs, last, out_len,
-                             log_psi, r_new, T, V, H, Ccand, blank, eos);
+  ctc_prefix_kernel<<<(n + kPrefixWarps - 1) / kPrefixWarps, kPrefixWarps * 32, 0, static_cast<cudaStream_t>(stream)>>>(
+      lpz, r_prev, cs, last, out_len, log_psi, r_new, T, V, H, Ccand, blank, eos);
   count_launch();
-  return e == cudaSuccess ? launch_status() : (int)e;
+  return launch_status();
 }

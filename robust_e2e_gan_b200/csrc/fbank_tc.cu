@@ -22,7 +22,6 @@
 //   warps 16..19: epilogue -- tcgen05.ld the three column ranges of the finished accumulator (lane <-> frame), sum,
 //                 clamp/log/CMVN, store Y and G
 // Algorithmic HBM bytes: 4*N*(2F + 2M) masked with G, 4*N*(F + M) plain.
-#include <cstdlib>
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -867,8 +866,7 @@ int fbank_tc_fwd(const float *mask, int mask_is_logit, const float *mag, const f
       return rc;                                                                                                        \
     fbank_tc_fwd_kernel<MASKED, DEPTH, FC, PAIR><<<grid, kTcThreads, smem, st>>>(p);                                     \
   } while (0)
-  static const bool pair_enabled = !(getenv("RE2E_FB_PAIR") && atoi(getenv("RE2E_FB_PAIR")) == 0);   // A/B switch: RE2E_FB_PAIR=0
-  const bool pair = pair_enabled && F == 257 && p.nchunks == 8 && ns >= 4 && (reinterpret_cast<uintptr_t>(mag) & 7u) == 0 &&
+  const bool pair = F == 257 && p.nchunks == 8 && ns >= 4 && (reinterpret_cast<uintptr_t>(mag) & 7u) == 0 &&
                     (!mask || (reinterpret_cast<uintptr_t>(mask) & 7u) == 0);
   if (mask) {
     if (pair) RE2E_FB_LAUNCH(true, 2, 257, true);

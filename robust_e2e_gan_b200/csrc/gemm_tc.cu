@@ -18,8 +18,6 @@
 // shape and the UMMA descriptors -- no transposed copies.
 #include <cuda.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -668,11 +666,7 @@ extern "C" int re2e_gemm_tf32x3(const float *A, int lda, int a_mn, const float *
   RE2E_CHECK_ARG(lda >= (a_mn ? M : K) && ldb >= (b_mn ? N : K));
   CUtensorMap ta, tb, tc;
   int rc;
-  int BN = (N % 256 == 0 || N > 1024) ? 256 : 160;
-  {
-    static const int force_bn = [] { const char *e = getenv("RE2E_GEMM_BN"); return e ? atoi(e) : 0; }();   // A/B timing aid
-    if (force_bn == 160 || force_bn == 256) BN = force_bn;
-  }
+  const int BN = (N % 256 == 0 || N > 1024) ? 256 : 160;
   if (!a_mn) rc = make_tmap(&ta, A, K, M, lda, kBM, false);
   else rc = make_tmap(&ta, A, M, K, lda, kBK, true);
   if (rc != RE2E_OK) return rc;
@@ -698,11 +692,10 @@ extern "C" int re2e_gemm_tf32x3(const float *A, int lda, int a_mn, const float *
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   {
-    // persistent tile loop with a double-buffered TMEM accumulator (RE2E_GEMM_PERSIST=0 selects the one-CTA-per-tile
-    // kernel below, kept as the reference implementation and for A/B timing)
-    static const bool persist = [] { const char *e = getenv("RE2E_GEMM_PERSIST"); return !(e && e[0] == '0'); }();
+    // more work items than SMs: persistent tile loop with a double-buffered TMEM accumulator.  A single wave gains
+    // nothing from the tile loop and runs the one-CTA-per-tile kernel below.
     const long long items = (long long)((M + kBM - 1) / kBM) * ((N + BN - 1) / BN) * ((nkb + prm.kb_per - 1) / prm.kb_per);
-    if (persist && items > num_sms()) {   // a single wave gains nothing from the tile loop
+    if (items > num_sms()) {
       prm.tma_c = 0;
       if (BN == 256) return dispatch_major_persist<256, 2>(a_mn, b_mn, ta, tb, prm, st);
       return dispatch_major_persist<160, 3>(a_mn, b_mn, ta, tb, prm, st);

@@ -361,30 +361,12 @@ __global__ void __launch_bounds__(kSThreads) lstm_step_kernel(const LstmStep p) 
   }
 }
 
+// plain stream order (see DESIGN.md on programmatic launches in the beam-search position)
 template <bool FWD>
 int launch_lstm_step(LstmStep prm, int tiles, int cl, cudaStream_t st) {
-  auto kern = lstm_step_kernel<FWD>;
   prm.pitch = lstm_step_pitch(prm.K1, prm.K2, cl);
-  const size_t smem = lstm_step_smem(prm.pitch, cl);
-  int rc = ensure_smem(reinterpret_cast<const void *>(kern), smem);
-  if (rc != RE2E_OK) return rc;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(tiles * cl), (unsigned)((prm.M + kST - 1) / kST));
-  cfg.blockDim = dim3((unsigned)kSThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)cl;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (pdl_enabled() && (pdl_mask() & 1)) ? 2 : 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, prm);
-  count_launch();
-  return e == cudaSuccess ? RE2E_OK : (int)e;
+  const dim3 grid((unsigned)(tiles * cl), (unsigned)((prm.M + kST - 1) / kST));
+  return launch_cluster(lstm_step_kernel<FWD>, grid, dim3(kSThreads), lstm_step_smem(prm.pitch, cl), st, cl, false, prm);
 }
 
 constexpr int kFwdCL = 4, kBwdCL = 8;
@@ -402,10 +384,10 @@ extern "C" int re2e_batch_nt(const float *X, const float *W, const float *bias, 
   const size_t smem = sizeof(float) * (kBM * (kBK + 4) + cols * kBK);
   int rc = ensure_smem(reinterpret_cast<const void *>(batch_nt_kernel), smem);
   if (rc != RE2E_OK) return rc;
-  cudaError_t e = launch_pdl(1, batch_nt_kernel, dim3((unsigned)((N + cols - 1) / cols)), dim3((unsigned)(cols * 32)), smem,
-                             static_cast<cudaStream_t>(stream), X, W, bias, out, M, N, K, accumulate, vec);
+  batch_nt_kernel<<<(N + cols - 1) / cols, cols * 32, smem, static_cast<cudaStream_t>(stream)>>>(X, W, bias, out, M, N, K,
+                                                                                               accumulate, vec);
   count_launch();
-  return e == cudaSuccess ? launch_status() : (int)e;
+  return launch_status();
 }
 
 extern "C" int re2e_sample_tokens_ws_bytes(int M) { return M > 0 ? (int)sizeof(unsigned long long) * (M + 1) : 0; }

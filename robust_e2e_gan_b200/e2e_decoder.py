@@ -177,8 +177,7 @@ class _FusedSearch(object):
         self.pin, self.events = pin
         self.hist_np = self.pin.numpy()
         with torch.cuda.stream(stream):
-            self.position = dec._fused_position(hb, lpz, Cb, self.beam, recog_args.ctc_weight, maxlen, self.pin, tables,
-                                                bool(getattr(recog_args, "fused_tail", True)))
+            self.position = dec._fused_position(hb, lpz, Cb, self.beam, recog_args.ctc_weight, maxlen, self.pin, tables)
         self.use_graph = bool(getattr(recog_args, "cuda_graph", True)) and maxlen >= 6
         self.graph = None
         self.hyps = [(np.float32(0.0), dec.sos, None, 1)]               # hypothesis k lives in device row k
@@ -479,11 +478,11 @@ class Decoder(torch.nn.Module):
         wcat = torch.cat((cell.weight_ih.detach()[:, E:], cell.weight_hh.detach()), 1).float().contiguous()
         return eg, wcat, _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach())
 
-    def _fused_position(self, hb, lpz, Cb, beam, ctc_weight, maxlen, hist, tables, fused_tail=True):
+    def _fused_position(self, hb, lpz, Cb, beam, ctc_weight, maxlen, hist, tables):
         """One output position for all W rows as launches of the library over static buffers (csrc/beam.cu):
         AttLoc step, LSTMCell step (embedding half by token lookup), output layer, log-softmax + top-Cb, CTC prefix
         scores, then joint score + merge + gather of the chosen rows' states for the next position (one launch,
-        ``re2e_beam_advance``; ``fused_tail=False`` runs them as three).  ``hist`` (>= maxlen, 4, beam): page-locked host
+        ``re2e_beam_advance``).  ``hist`` (>= maxlen, 4, beam): page-locked host
         tensor the winners of every position are written to.  ``tables``: ``_beam_tables()`` of this call.  Returns the
         position closure.  The first position needs no special case: the states start as every row's initial state."""
         import ctypes
@@ -498,7 +497,7 @@ class Decoder(torch.nn.Module):
         # every buffer of the search carved out of two allocations (fp32 / int32); `hist` is page-locked HOST memory that
         # the merge kernel writes directly (160 B per position over the bus: no copy, the host just waits for an event)
         use_ctc = lpz is not None
-        sizes = [("sc", W), ("out", 3 * W * beam), ("z_st", W * Z), ("c_st", W * Z), ("z_in", W * Z), ("c_in", W * Z),
+        sizes = [("sc", W), ("z_st", W * Z), ("c_st", W * Z), ("z_in", W * Z), ("c_in", W * Z),
                  ("a_st", W * Th), ("a_in", W * Th), ("att_c", W * D), ("act", W * 4 * Z), ("logits", W * V),
                  ("top_v", W * Cb)]
         if use_ctc:
@@ -510,7 +509,7 @@ class Decoder(torch.nn.Module):
             o += (n_ + 3) // 4 * 4
         ints = torch.empty(4 * W + 4 + W * Cb, device=dev, dtype=torch.int32)
         ctl, state, top_i = ints[:4 * W].view(4, W), ints[4 * W:4 * W + 2], ints[4 * W + 4:]
-        sc, out = bufs["sc"], bufs["out"]
+        sc = bufs["sc"]
         z_st, c_st, z_in, c_in = bufs["z_st"], bufs["c_st"], bufs["z_in"], bufs["c_in"]
         a_st, a_in, att_c, act, logits, top_v = (bufs[k_] for k_ in ("a_st", "a_in", "att_c", "act", "logits", "top_v"))
         segs = [(z_st, z_in, Z, 0), (c_st, c_in, Z, 0), (a_st, a_in, Th, 0)]
@@ -544,17 +543,9 @@ class Decoder(torch.nn.Module):
                 calls.append((lib.re2e_ctc_prefix_score, "re2e_ctc_prefix_score",
                               (P(lpz), P(r_in), P(top_i), P(ctl[2]), P(ctl[3]), P(psi_st), P(r_st), Th, V, W, Cb, 0,
                                self.eos, sp)))
-            if fused_tail:
-                calls.append((lib.re2e_beam_advance, "re2e_beam_advance",
-                              (P(top_v), P(top_i), P(psi_st), P(psi_in), P(sc), w_att, w_ctc, W, Cb, beam, P(state), P(ctl),
-                               P(hist), self.eos, maxlen, n, src, dst, rowf, subc, sp)))
-            else:
-                calls += [
-                    (lib.re2e_beam_joint, "re2e_beam_joint",
-                     (P(top_v), P(top_i), P(psi_st), P(psi_in), P(sc), w_att, w_ctc, W, Cb, beam, P(out), sp)),
-                    (lib.re2e_beam_merge, "re2e_beam_merge",
-                     (P(out), P(state), P(ctl), P(sc), P(hist), W, beam, self.eos, maxlen, sp)),
-                    (lib.re2e_beam_gather, "re2e_beam_gather", (P(ctl[0]), P(ctl[1]), W, n, src, dst, rowf, subc, sp))]
+            calls.append((lib.re2e_beam_advance, "re2e_beam_advance",
+                          (P(top_v), P(top_i), P(psi_st), P(psi_in), P(sc), w_att, w_ctc, W, Cb, beam, P(state), P(ctl),
+                           P(hist), self.eos, maxlen, n, src, dst, rowf, subc, sp)))
             return calls
 
         built = {}
@@ -620,7 +611,7 @@ class Decoder(torch.nn.Module):
             lpz = _lib.f32c(lpz.detach(), dev)
             V = lpz.size(-1)
             Cb = min(V, int(beam * CTC_SCORING_RATIO)) if recog_args.ctc_weight != 1.0 else V
-        if not (bool(getattr(recog_args, "fused_position", True)) and self.dlayers == 1 and beam <= Cb <= 32
+        if not (self.dlayers == 1 and beam <= Cb <= 32
                 and self.output.out_features <= 8192
                 and bool(_lib.lib().re2e_lstm_step_supported(beam, h.size(1), self.dunits))):
             return None
@@ -652,7 +643,7 @@ class Decoder(torch.nn.Module):
                     lp = lpzs[i] if lpzs is not None else None
                     plan = self._fused_plan(hs[i], lp, recog_args)
                     if plan is None:      # shapes the fused position does not take: the per-utterance path
-                        results[i] = self.recognize_beam(hs[i], lp, recog_args, char_list)
+                        results[i] = self._recognize_generic(hs[i], lp, recog_args)
                         continue
                     if tables is None:
                         tables = self._beam_tables()
@@ -688,10 +679,16 @@ class Decoder(torch.nn.Module):
         if rnnlm is not None or fstlm is not None:
             raise NotImplementedError("LM rescoring is outside the hot path (SURVEY.md section 8)")
         _lib.lib()
-        self.att.reset()
         plan = self._fused_plan(h, lpz, recog_args)
-        if plan is not None:
-            return self._recognize_fused(*plan[:2], recog_args, *plan[2:])
+        if plan is None:
+            return self._recognize_generic(h, lpz, recog_args)
+        self.att.reset()
+        return self._recognize_fused(*plan[:2], recog_args, *plan[2:])
+
+    def _recognize_generic(self, h, lpz, recog_args):
+        """``recognize_beam`` on the generic position, for the shapes ``_fused_plan`` does not take; tests compare the
+        fused position against it."""
+        self.att.reset()
         dev = self.embed.weight.device
         h = _lib.f32c(h.detach(), dev)
         Th = h.size(0)

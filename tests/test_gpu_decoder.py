@@ -351,9 +351,9 @@ def test_beam_gather_and_joint():
 @pytest.mark.parametrize("ctc_weight,beam,Th", [(0.3, 10, 60), (0.0, 5, 40), (0.5, 1, 25), (0.3, 4, 2), (0.3, 6, 7),
                                                  (0.7, 3, 11)])
 def test_fused_beam_position_matches_generic_path(ctc_weight, beam, Th):
-    """The fused position (csrc/beam.cu; tail as one launch or as joint / merge / gather) and the generic tensor-op
-    position of recognize_beam give the same n-best list (tokens identical, scores to 1e-4), with and without CUDA-graph
-    replay (fused: 8 positions per replay, history read back in chunks)."""
+    """The fused position (csrc/beam.cu) and the generic tensor-op position of recognize_beam give the same n-best list
+    (tokens identical, scores to 1e-4), with and without CUDA-graph replay (fused: 8 positions per replay, history read
+    back in chunks)."""
     helpers.BEAM_CASES["_tmp"] = dict(helpers.BEAM_CASES["beam_eos"], seed=31, beam=beam, ctc_weight=ctc_weight,
                                       nbest=min(beam, 3), Th=Th)
     try:
@@ -365,18 +365,17 @@ def test_fused_beam_position_matches_generic_path(ctc_weight, beam, Th):
     lpz = ctc.log_softmax(hd.unsqueeze(0))[0] if ctc_weight > 0.0 else None
     res = {}
     # (fused first: a generic search with its graph must also work on a decoder that has run fused searches)
-    for fused, graph, tail in ((True, True, True), (True, False, True), (True, True, False), (True, False, False),
-                               (False, True, True), (False, False, True)):
+    for fused, graph in ((True, True), (True, False), (False, True), (False, False)):
         ra = recog_args(c)
-        ra.fused_position, ra.cuda_graph, ra.fused_tail = fused, graph, tail
+        ra.cuda_graph = graph
         n0 = _lib_count()
         with torch.no_grad():
-            res[fused, graph, tail] = dec.recognize_beam(hd, lpz, ra, None)
+            res[fused, graph] = (dec.recognize_beam if fused else dec._recognize_generic)(hd, lpz, ra)
         if fused and not graph:
-            assert _lib_count() - n0 >= 5 * (len(res[fused, graph, tail][0]["yseq"]) - 2)
-    ref = res[False, False, True]
+            assert _lib_count() - n0 >= 5 * (len(res[fused, graph][0]["yseq"]) - 2)
+    ref = res[False, False]
     for k, got in res.items():
-        assert [x["yseq"] for x in got] == [x["yseq"] for x in ref], "tokens differ for (fused, graph, fused tail) = %s" % (k,)
+        assert [x["yseq"] for x in got] == [x["yseq"] for x in ref], "tokens differ for (fused, graph) = %s" % (k,)
         for a, b in zip(got, ref):
             assert abs(a["score"] - b["score"]) <= 1e-4 * abs(b["score"])
 
@@ -439,10 +438,8 @@ def test_fused_search_sees_weights_written_through_data():
             assert abs(a["score"] - b["score"]) <= 1e-4 * abs(b["score"]), name
 
     same(fused, "fused")
-    ra = recog_args(c)
-    ra.fused_position = False
     with torch.no_grad():
-        generic = dec.recognize_beam(hd, lpz, ra, None)
+        generic = dec._recognize_generic(hd, lpz, recog_args(c))
     same(generic, "generic")
 
 
