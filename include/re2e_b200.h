@@ -218,6 +218,8 @@ int re2e_sample_tokens(const float *X, const float *W, const float *bias, const 
 /* One LSTMCell position in one launch (after the embedding half): gates = egate + ctx @ Wcat[:, :D]^T + h_prev @
  * Wcat[:, D:]^T, then the cell's pointwise arithmetic -> act (B,4Z) gate activations (kept for the backward), c_out, h_out
  * (B,Z).  Wcat (4Z, D+Z) = [W_ih[:, E:] | W_hh].  Clusters of 4 CTAs split the reduction (deterministic order).
+ * An upper layer of a multi-layer decoder (LSTMCell(Z, Z) on the layer below's h) is the same call with ctx = that h
+ * (D = Z), Wcat = [W_ih | W_hh] and egate = the single row b_ih + b_hh, read through an all-zero egate_row.
  * re2e_lstm_step_bwd: d_ctx (B,D) | d_hprev (B,Z) = dgates (B,4Z) @ Wcat, given WcatT (D+Z, 4Z) = Wcat^T (clusters of 8).
  * Supported: D % 4 == Z % 4 == 0, D, Z <= 640, 16 B aligned operands; else RE2E_E_UNSUPPORTED (callers then compose
  * re2e_batch_nt + re2e_lstm_pointwise_*). */
@@ -321,15 +323,18 @@ int re2e_cross_entropy_bwd(const float *logits, long long ld, const long long *t
  * here a position is gather -> re2e_attloc_step_fwd -> re2e_lstm_step_fwd -> re2e_batch_nt (output layer) ->
  * re2e_log_softmax_topk -> re2e_ctc_prefix_score -> re2e_beam_joint over static buffers (graph-replayable).
  *
- * re2e_beam_gather: for each of nseg state tensors, dst[s][m, :] = src[s][parent[m] (, cand[m]), :] (row_floats[s] floats;
- *   sub_count[s] > 0: the source has that many candidate sub-rows per parent row, e.g. the CTC states (W, ctc_beam, T, 2)).
+ * re2e_beam_gather: for each of nseg <= 16 state tensors, dst[s][m, :] = src[s][parent[m] (, cand[m]), :] (row_floats[s]
+ *   floats; sub_count[s] > 0: the source has that many candidate sub-rows per parent row, e.g. the CTC states
+ *   (W, ctc_beam, T, 2)).  A search moves z and c of every decoder layer, the alignment and the two CTC states:
+ *   2 * layers + 3 segments, so decoders of up to 6 layers.
  * re2e_log_softmax_topk: per row log-softmax (optionally written to `full` (rows,V)) and its k largest entries, sorted
  *   descending, ties to the lower index -- what torch.topk(log_softmax(x), k) returns (model/e2e_decoder.py:262,276).
  *   V <= 8192 and k <= 32, else RE2E_E_UNSUPPORTED.
  * re2e_beam_joint: local = w_att * att_top + w_ctc * (log_psi - psi_prev[row]) (log_psi NULL: local = att_top), the `beam`
  *   best of the Cb <= 32 candidates per row; out (3, W, beam) fp32 = {row score + local, token id, candidate index}
  *   (model/e2e_decoder.py:284-292). */
-/* Initial working state of a search (model/e2e_decoder.py:205-231): z_in = c_in = 0 (W,Z), a_in uniform over Th (W,Th),
+/* Initial working state of a search (model/e2e_decoder.py:205-231): z_in = c_in = 0 (W*Z floats each; a decoder of L
+ * layers keeps its layers' states back to back, (L,W,dunits), and passes Z = L * dunits), a_in uniform over Th (W,Th),
  * r_in (W,Th,2) = CTCPrefixScore.initial_state (model/e2e_ctc.py:95-107; r_in / psi_in / lpz NULL without CTC), psi_in = 0,
  * ctl = {parent 0, candidate 0, token sos, position 0}, sc = 0, state = {1 live hypothesis, position 0}. */
 int re2e_beam_init(float *z_in, float *c_in, float *a_in, float *r_in, float *psi_in, const float *lpz, int32_t *ctl,
@@ -349,7 +354,8 @@ int re2e_beam_joint(const float *att_top, const int32_t *ids, const float *log_p
 int re2e_beam_merge(const float *out, int32_t *state, int32_t *ctl, float *sc, float *hist, int W, int beam, int eos,
                     int maxlen, void *stream);
 /* re2e_beam_joint + re2e_beam_merge + re2e_beam_gather (for the NEXT position, with the rows just chosen) in one launch
- * of one CTA: the tail of a position is a strictly serial chain of three tiny kernels, i.e. three launch latencies. */
+ * of one CTA: the tail of a position is a strictly serial chain of three tiny kernels, i.e. three launch latencies.
+ * nseg <= 16 segments, as re2e_beam_gather. */
 int re2e_beam_advance(const float *att_top, const int32_t *ids, const float *log_psi, const float *psi_prev, float *sc,
                       float w_att, float w_ctc, int W, int Cb, int beam, int32_t *state, int32_t *ctl, float *hist,
                       int eos, int maxlen, int nseg, const float *const *src, float *const *dst, const int *row_floats,

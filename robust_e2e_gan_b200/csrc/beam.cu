@@ -24,7 +24,9 @@ __device__ __forceinline__ float ord_val(unsigned k) {
   return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
-constexpr int kMaxSeg = 8;
+// State tensors one gather can move: z and c of every decoder layer (2 per layer), the alignment and the two CTC states,
+// so decoders of up to 6 layers fit with CTC.  The arrays are kernel parameters (400 B of the 4 KB parameter space).
+constexpr int kMaxSeg = 16;
 struct GatherArgs {
   const float *src[kMaxSeg];
   float *dst[kMaxSeg];

@@ -4,31 +4,33 @@ Same constructor, submodule names (``embed``, ``decoder`` = ModuleList of LSTMCe
 state_dict keys as the reference's ``Decoder`` for the configuration the scripts use (no LM fusion,
 ``model_unit='char'``), so reference ``asr_state_dict`` checkpoints load unchanged.
 
-* ``forward(hpad, hlen, ys, scheduled_sampling_rate)`` -- the training loop of model/e2e_decoder.py:79-167:
-  AttLoc step kernel per output position with the alignment fed back un-detached, teacher forcing or scheduled
-  sampling, cross-entropy rescaled by ``mean(len(ys_in)) - 1``.  The output layer of all positions is ONE product on the
-  tcgen05 GEMM after the loop, the first LSTMCell is one cluster kernel per position (lstm.py) and the cross-entropy
-  runs on the library's kernels.  The decoder state fed to step i depends on the context of step i-1 through the
-  LSTMCell, so this loop calls the per-step AttLoc kernels (``AttLoc.forward_loop``, the persistent loop kernels, needs
-  the states of all steps up front).  Scheduled sampling (rate > 0) keeps that shape: the reference's one
-  ``random.random()`` per position is drawn before the loop, the flags reach the device through a page-locked buffer,
-  and a flagged position's token -- the arg-max of the previous position's logits -- is chosen on the device by
-  ``re2e_sample_tokens`` (the logits are never written) into the token buffer the LSTM step looks its embedding half up
-  from.  No host round trip, so the forward + backward can be captured once and replayed with new draws
-  (``draw_sampling``).  ``fused_lstm = False`` or a CPU module runs the reference's own loop.
+* ``forward(hpad, hlen, ys, scheduled_sampling_rate)`` -- the training loop of model/e2e_decoder.py:79-167: AttLoc
+  step kernel per output position with the alignment fed back un-detached, teacher forcing or scheduled sampling,
+  cross-entropy rescaled by ``mean(len(ys_in)) - 1``.  The output layer of all positions is ONE product on the tcgen05
+  GEMM after the loop, every LSTMCell is one cluster kernel per position (lstm.py; the upper layers of a multi-layer
+  decoder through ``LSTMLoop.stacked``) and the cross-entropy runs on the library's kernels.  The decoder state fed to
+  step i depends on the context of step i-1 through the LSTMCell, so this loop calls the per-step AttLoc kernels
+  (``AttLoc.forward_loop``, the persistent loop kernels, needs the states of all steps up front).  Scheduled sampling
+  (rate > 0) keeps that shape: the reference's one ``random.random()`` per position is drawn before the loop, the
+  flags reach the device through a page-locked buffer, and a flagged position's token -- the arg-max of the previous
+  position's logits -- is chosen on the device by ``re2e_sample_tokens`` (the logits are never written) into the token
+  buffer the LSTM step looks its embedding half up from.  No host round trip, so the forward + backward can be
+  captured once and replayed with new draws (``draw_sampling``).  ``fused_lstm = False`` or a CPU module runs the
+  reference's own loop.
 * ``recognize_beam(h, lpz, recog_args, char_list, rnnlm=None, fstlm=None)`` -- hybrid CTC/attention beam search
   (model/e2e_decoder.py:170-369) re-designed for the GPU: ALL live hypotheses advance together (B = beam instead of
   beam x (B = 1) calls) and the whole output position runs on the device as SIX launches of the library over static
-  buffers (csrc/beam.cu): AttLoc step, LSTMCell step (one cluster kernel; the embedding half of its input product is a
-  per-token table looked up inside the kernel), output layer, log-softmax + top-``ctc_beam``, batched CTC prefix
-  scores whose forward variables never leave the device (the reference copies ``lpz`` to the host and loops over T in
-  numpy per hypothesis, model/e2e_ctc.py:143-146), and one kernel for joint score + merge of the beam x beam
-  candidates + gather of the chosen rows' states.  Eight positions are one CUDA-graph replay; the winners of every
-  position land in a history buffer that the host reads back a chunk at a time (two chunks in flight) to run the
-  reference's own bookkeeping -- <eos> handling, length penalty, ``end_detect`` -- so there is no host round trip per
-  position.  Scores accumulate in fp32 exactly as the reference's 0-dim tensors do.  Decoders the fused position does
-  not take (more than one LSTM layer, ctc_weight = 1 i.e. all V candidates, V > 8192, dunits or eprojs not a
-  multiple of 4) use the generic position: library AttLoc / prefix-score kernels + tensor ops, host merge per position.
+  buffers (csrc/beam.cu), one more per extra decoder layer: AttLoc step, LSTMCell step (one cluster kernel; the
+  embedding half of its input product is a per-token table looked up inside the kernel), one LSTMCell step per upper
+  layer, output layer, log-softmax + top-``ctc_beam``, batched CTC prefix scores whose forward variables never leave
+  the device (the reference copies ``lpz`` to the host and loops over T in numpy per hypothesis,
+  model/e2e_ctc.py:143-146), and one kernel for joint score + merge of the beam x beam candidates + gather of the
+  chosen rows' states.  Eight positions are one CUDA-graph replay; the winners of every position land in a history
+  buffer that the host reads back a chunk at a time (two chunks in flight) to run the reference's own bookkeeping --
+  <eos> handling, length penalty, ``end_detect`` -- so there is no host round trip per position.  Scores accumulate in
+  fp32 exactly as the reference's 0-dim tensors do.  Decoders the fused position does not take (more than
+  FUSED_MAX_LAYERS = 6 LSTM layers, ctc_weight = 1 i.e. all V candidates, V > 8192, dunits or eprojs not a multiple of
+  4) use the generic position: library AttLoc / prefix-score kernels + tensor ops, host merge per position.
 """
 import random
 import time
@@ -44,6 +46,9 @@ from .linear import linear
 from .lstm import LSTMLoop
 
 CTC_SCORING_RATIO = 1.5   # model/e2e_decoder.py:20
+# deepest decoder the fused beam-search position takes: re2e_beam_advance gathers at most 16 state tensors, z and c of
+# every layer + the alignment + the two CTC states (include/re2e_b200.h)
+FUSED_MAX_LAYERS = 6
 
 
 def end_detect(ended_hyps, i, M=3, D_end=np.log(1 * np.exp(-10))):
@@ -318,7 +323,7 @@ class Decoder(torch.nn.Module):
         self.labeldist = labeldist
         self.vlabeldist = None
         self.lsm_weight = lsm_weight
-        self.fused_lstm = True     # training loop: first LSTMCell on the library's kernels (lstm.py); False = torch.nn.LSTMCell
+        self.fused_lstm = True     # training loop: every LSTMCell on the library's kernels (lstm.py); False = torch.nn.LSTMCell
 
     def zero_state(self, hpad):
         return hpad.new_zeros(hpad.size(0), self.dunits)
@@ -375,6 +380,8 @@ class Decoder(torch.nn.Module):
             # ... and the embedding half of the first LSTMCell's input product is one dense product before the loop; per
             # position only the context / state products (batch-sized) and one fused pointwise kernel remain (lstm.py)
             lstm0 = LSTMLoop(self.decoder[0], eys) if (fused and not sampling) else None
+        # layers 1 .. dlayers-1 (input: the layer below's state) on the same step kernel, one launch per layer and position
+        upper = [LSTMLoop.stacked(self.decoder[l]) for l in range(1, self.dlayers)] if fused else None
         z_top = []
         for i in range(olength):
             att_c, att_w = self.att(hpad, hlen, z_list[0], att_w)
@@ -397,7 +404,10 @@ class Decoder(torch.nn.Module):
                     ey = torch.cat((eys[:, i, :], att_c), dim=1)
                 z_list[0], c_list[0] = self.decoder[0](ey, (z_list[0], c_list[0]))
             for l in range(1, self.dlayers):
-                z_list[l], c_list[l] = self.decoder[l](z_list[l - 1], (z_list[l], c_list[l]))
+                if upper is not None:
+                    z_list[l], c_list[l] = upper[l - 1].step(i, z_list[l - 1], z_list[l], c_list[l])
+                else:
+                    z_list[l], c_list[l] = self.decoder[l](z_list[l - 1], (z_list[l], c_list[l]))
             if batched_output:
                 z_top.append(z_list[-1])
             else:
@@ -467,7 +477,8 @@ class Decoder(torch.nn.Module):
     def _beam_tables(self):
         """Per-model constants of the fused beam-search position: the embedding half of the LSTMCell input product for
         EVERY token (V, 4Z) = embed.weight @ W_ih[:, :E]^T + b_ih + b_hh (looked up by token in the step kernel), the
-        recurrent matrices side by side (4Z, D+Z), and the output layer.  Built once per recognize_beam /
+        recurrent matrices side by side (4Z, D+Z), the output layer, and per upper layer (decoder[1:]) its matrices side
+        by side [W_ih | W_hh] (4Z, 2Z) with its gate row b_ih + b_hh (1, 4Z).  Built once per recognize_beam /
         recognize_beam_batch call, never cached across calls: a write through ``.data`` (checkpoint averaging, a
         training step between decodes) changes a parameter without bumping its version counter, so no cache key can see
         it, and stale tables would make the fused search silently decode with the old weights."""
@@ -476,28 +487,33 @@ class Decoder(torch.nn.Module):
         eg = linear(_lib.f32c(self.embed.weight.detach()), cell.weight_ih.detach()[:, :E].contiguous(),
                     (cell.bias_ih + cell.bias_hh).detach()).contiguous()
         wcat = torch.cat((cell.weight_ih.detach()[:, E:], cell.weight_hh.detach()), 1).float().contiguous()
-        return eg, wcat, _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach())
+        upper = [(torch.cat((c.weight_ih.detach(), c.weight_hh.detach()), 1).float().contiguous(),
+                  _lib.f32c((c.bias_ih + c.bias_hh).detach()).view(1, -1)) for c in self.decoder[1:]]
+        return eg, wcat, _lib.f32c(self.output.weight.detach()), _lib.f32c(self.output.bias.detach()), upper
 
     def _fused_position(self, hb, lpz, Cb, beam, ctc_weight, maxlen, hist, tables):
         """One output position for all W rows as launches of the library over static buffers (csrc/beam.cu):
-        AttLoc step, LSTMCell step (embedding half by token lookup), output layer, log-softmax + top-Cb, CTC prefix
-        scores, then joint score + merge + gather of the chosen rows' states for the next position (one launch,
-        ``re2e_beam_advance``).  ``hist`` (>= maxlen, 4, beam): page-locked host
-        tensor the winners of every position are written to.  ``tables``: ``_beam_tables()`` of this call.  Returns the
+        AttLoc step, LSTMCell step (embedding half by token lookup), one LSTMCell step per upper layer (context = the
+        new state of the layer below, gate row b_ih + b_hh through the all-zero row index ``zrow``), output layer on the
+        top layer, log-softmax + top-Cb, CTC prefix scores, then joint score + merge + gather of the chosen rows' states
+        (z and c of every layer, alignment, CTC) for the next position (one launch, ``re2e_beam_advance``).
+        ``hist`` (>= maxlen, 4, beam): page-locked host tensor the winners of every position are written to.  ``tables``: ``_beam_tables()`` of this call.  Returns the
         position closure.  The first position needs no special case: the states start as every row's initial state."""
         import ctypes
         lib = _lib.lib()
         dev = hb.device
         W, Th, D = hb.shape
         Z, V = self.dunits, self.output.out_features
-        eg, wcat, w_out, b_out = tables
+        NL = self.dlayers
+        eg, wcat, w_out, b_out, upper = tables
         st = self.att.precompute(hb)
         _, _, _, A, _, C, K = st.dims
         W_dec, W_att, W_conv, gvec, gvec_b = st.weights
         # every buffer of the search carved out of two allocations (fp32 / int32); `hist` is page-locked HOST memory that
         # the merge kernel writes directly (160 B per position over the bus: no copy, the host just waits for an event)
         use_ctc = lpz is not None
-        sizes = [("sc", W), ("z_st", W * Z), ("c_st", W * Z), ("z_in", W * Z), ("c_in", W * Z),
+        # z / c of the layers back to back, (NL, W, Z) per buffer: re2e_beam_init zeroes all layers' inputs at once
+        sizes = [("sc", W), ("z_st", NL * W * Z), ("c_st", NL * W * Z), ("z_in", NL * W * Z), ("c_in", NL * W * Z),
                  ("a_st", W * Th), ("a_in", W * Th), ("att_c", W * D), ("act", W * 4 * Z), ("logits", W * V),
                  ("top_v", W * Cb)]
         if use_ctc:
@@ -507,12 +523,15 @@ class Decoder(torch.nn.Module):
         for name, n_ in sizes:
             bufs[name] = flat[o:o + n_]
             o += (n_ + 3) // 4 * 4
-        ints = torch.empty(4 * W + 4 + W * Cb, device=dev, dtype=torch.int32)
-        ctl, state, top_i = ints[:4 * W].view(4, W), ints[4 * W:4 * W + 2], ints[4 * W + 4:]
+        ints = torch.empty(4 * W + 4 + W * Cb + (W if NL > 1 else 0), device=dev, dtype=torch.int32)
+        ctl, state, top_i = ints[:4 * W].view(4, W), ints[4 * W:4 * W + 2], ints[4 * W + 4:4 * W + 4 + W * Cb]
+        zrow = ints[4 * W + 4 + W * Cb:].zero_() if NL > 1 else None
         sc = bufs["sc"]
-        z_st, c_st, z_in, c_in = bufs["z_st"], bufs["c_st"], bufs["z_in"], bufs["c_in"]
+        z_st, c_st, z_in, c_in = (bufs[k_].view(NL, W * Z) for k_ in ("z_st", "c_st", "z_in", "c_in"))
         a_st, a_in, att_c, act, logits, top_v = (bufs[k_] for k_ in ("a_st", "a_in", "att_c", "act", "logits", "top_v"))
-        segs = [(z_st, z_in, Z, 0), (c_st, c_in, Z, 0), (a_st, a_in, Th, 0)]
+        segs = [(z_st[0], z_in[0], Z, 0), (c_st[0], c_in[0], Z, 0), (a_st, a_in, Th, 0)]
+        for l in range(1, NL):
+            segs += [(z_st[l], z_in[l], Z, 0), (c_st[l], c_in[l], Z, 0)]
         r_st = r_in = psi_st = psi_in = None
         if use_ctc:
             r_st, r_in, psi_st, psi_in = bufs["r_st"], bufs["r_in"], bufs["psi_st"], bufs["psi_in"]
@@ -525,8 +544,8 @@ class Decoder(torch.nn.Module):
         w_att, w_ctc = float(1.0 - ctc_weight), float(ctc_weight)
         P = _lib.ptr
         with _lib.on(dev):
-            _lib.check(lib.re2e_beam_init(P(z_in), P(c_in), P(a_in), P(r_in), P(psi_in), P(lpz), P(ctl), P(sc), P(state), W, Z,
-                                          Th, V, 0, self.sos, _lib.stream_ptr()), "re2e_beam_init")
+            _lib.check(lib.re2e_beam_init(P(z_in), P(c_in), P(a_in), P(r_in), P(psi_in), P(lpz), P(ctl), P(sc), P(state), W,
+                                          NL * Z, Th, V, 0, self.sos, _lib.stream_ptr()), "re2e_beam_init")
 
         def build(sp):
             """The position's launches with their argument tuples, for one stream (everything else is constant)."""
@@ -535,8 +554,13 @@ class Decoder(torch.nn.Module):
                  (P(st.pre), P(st.enc), P(z_in), P(a_in), P(W_dec), P(W_att), P(W_conv), P(gvec), P(gvec_b), 2.0, P(att_c),
                   P(a_st), None, None, None, W, Th, D, A, Z, C, K, sp)),
                 (lib.re2e_lstm_step_fwd, "re2e_lstm_step_fwd",
-                 (P(att_c), P(z_in), P(c_in), P(wcat), P(eg), P(ctl[2]), P(act), P(c_st), P(z_st), W, D, Z, sp)),
-                (lib.re2e_batch_nt, "re2e_batch_nt", (P(z_st), P(w_out), P(b_out), P(logits), W, V, Z, 0, sp)),
+                 (P(att_c), P(z_in[0]), P(c_in[0]), P(wcat), P(eg), P(ctl[2]), P(act), P(c_st[0]), P(z_st[0]), W, D, Z, sp)),
+            ] + [
+                (lib.re2e_lstm_step_fwd, "re2e_lstm_step_fwd",
+                 (P(z_st[l - 1]), P(z_in[l]), P(c_in[l]), P(upper[l - 1][0]), P(upper[l - 1][1]), P(zrow), P(act),
+                  P(c_st[l]), P(z_st[l]), W, Z, Z, sp)) for l in range(1, NL)
+            ] + [
+                (lib.re2e_batch_nt, "re2e_batch_nt", (P(z_st[NL - 1]), P(w_out), P(b_out), P(logits), W, V, Z, 0, sp)),
                 (lib.re2e_log_softmax_topk, "re2e_log_softmax_topk", (P(logits), W, V, Cb, None, P(top_v), P(top_i), sp)),
             ]
             if lpz is not None:
@@ -561,7 +585,7 @@ class Decoder(torch.nn.Module):
                     if rc != 0:
                         _lib.check(rc, name)
 
-        position.keep = (flat, ints, eg, wcat, w_out, b_out, lpz, st)   # buffers a captured graph points into
+        position.keep = (flat, ints, eg, wcat, w_out, b_out, upper, lpz, st)   # buffers a captured graph points into
         return position
 
     def _host_merge(self, hyps, ended_hyps, entries, i, maxlen, minlen, penalty):
@@ -611,9 +635,11 @@ class Decoder(torch.nn.Module):
             lpz = _lib.f32c(lpz.detach(), dev)
             V = lpz.size(-1)
             Cb = min(V, int(beam * CTC_SCORING_RATIO)) if recog_args.ctc_weight != 1.0 else V
-        if not (self.dlayers == 1 and beam <= Cb <= 32
+        lib = _lib.lib()
+        if not (self.dlayers <= FUSED_MAX_LAYERS and beam <= Cb <= 32
                 and self.output.out_features <= 8192
-                and bool(_lib.lib().re2e_lstm_step_supported(beam, h.size(1), self.dunits))):
+                and bool(lib.re2e_lstm_step_supported(beam, h.size(1), self.dunits))
+                and (self.dlayers == 1 or bool(lib.re2e_lstm_step_supported(beam, self.dunits, self.dunits)))):
             return None
         hb = h.unsqueeze(0).expand(beam, Th, h.size(1)).contiguous()
         return hb, lpz, Cb, maxlen, minlen

@@ -15,6 +15,10 @@ Same arithmetic as ``torch.nn.LSTMCell`` (gate order i, f, g, o) split the way t
 ``LSTMLoop.by_token`` is the same loop with the embedding half looked up by token inside the step kernel from a per-token
 table (V, 4Z), for inputs that are chosen while the loop runs (scheduled sampling): the tokens live in a device buffer
 the caller may overwrite before each step, and the anchor forms the embedding-half gradients from the final buffer.
+
+``LSTMLoop.stacked`` is the loop of an upper layer of a multi-layer decoder (``LSTMCell(dunits, dunits)`` on the layer
+below's state): the context is that state, the recurrent matrices are ``[W_ih | W_hh]``, and the "embedding half" is
+the constant row b_ih + b_hh, which every batch row reads through an all-zero row index.  Same kernels, same anchor.
 """
 import torch
 
@@ -34,6 +38,7 @@ class _State(object):
     def __init__(self):
         self.W_c = self.W_hh = self.W_cT = self.W_hhT = self.Wcat = self.WcatT = self.egates = None
         self.tok = None                  # token-lookup mode: (L, B) int32 rows of `egates` (the per-token table)
+        self.rows0 = None                # stacked mode: (B,) int32 zeros, every row reads `egates` (1, 4Z) = the bias row
         self.dg, self.ctx, self.hprev = {}, {}, {}
 
 
@@ -63,22 +68,28 @@ class _Anchor(torch.autograd.Function):
 
 
 def _recurrent_grads(st):
-    """(d_eg (L,B,4Z), dW_c, dW_hh) from the gate gradients the steps left in ``st``, or Nones when no step had one."""
+    """(d_eg (L,B,4Z), dW_c, dW_hh) from the gate gradients the steps left in ``st``, or Nones when no step had one.
+    Stacked mode: d_eg is the (n*B, 4Z) stack of the n positions that had a gradient (the bias gradient is its column
+    sums; positions without one would only add zero rows)."""
     dW_c = dW_hh = d_eg = None
     if st.dg:
-        L_, B = st.tok.shape if st.tok is not None else st.egates.shape[:2]
         G4 = st.egates.shape[-1]
-        zero = None
-        rows = []
-        for i in range(L_):
-            if i in st.dg:
-                rows.append(st.dg[i])
-            else:
-                zero = zero if zero is not None else torch.zeros(B, G4, device=st.egates.device)
-                rows.append(zero)
-        d_eg = torch.stack(rows, 0)                                           # (L, B, 4Z)
         idx = sorted(st.dg)
+        if st.rows0 is not None:
+            B = st.rows0.numel()
+        else:
+            L_, B = st.tok.shape if st.tok is not None else st.egates.shape[:2]
+            zero = None
+            rows = []
+            for i in range(L_):
+                if i in st.dg:
+                    rows.append(st.dg[i])
+                else:
+                    zero = zero if zero is not None else torch.zeros(B, G4, device=st.egates.device)
+                    rows.append(zero)
+            d_eg = torch.stack(rows, 0)                                       # (L, B, 4Z)
         DG = torch.stack([st.dg[i] for i in idx], 0).view(len(idx) * B, G4)
+        d_eg = DG if st.rows0 is not None else d_eg
         XC = torch.stack([st.ctx[i] for i in idx], 0).view(len(idx) * B, -1)
         HP = torch.stack([st.hprev[i] for i in idx], 0).view(len(idx) * B, -1)
         dW_c = torch.empty_like(st.W_c)
@@ -124,6 +135,25 @@ class _TokenAnchor(torch.autograd.Function):
         return dW_c, dW_hh, dW_e, db, db.clone(), d_emb.to(ctx.emb.dtype), None, None, None
 
 
+class _StackedAnchor(torch.autograd.Function):
+    """``_Anchor`` of an upper layer: Wcat = [W_ih | W_hh], the gate row b_ih + b_hh shared by every batch row.  The
+    backward forms dW_ih = sum_s dgates_s^T h_below_s and dW_hh (the two GEMMs of ``_recurrent_grads``) and
+    d b_ih = d b_hh = column sums of all positions' gate gradients; there is no embedding gradient."""
+
+    @staticmethod
+    def forward(ctx, W_ih, W_hh, b_ih, b_hh, state):
+        _Anchor.forward(ctx, W_ih, W_hh, (b_ih.detach() + b_hh.detach()).view(1, -1), state)
+        return torch.zeros(1, device=W_ih.device, dtype=torch.float32)
+
+    @staticmethod
+    def backward(ctx, _g):
+        DG, dW_ih, dW_hh = _recurrent_grads(ctx.state)
+        if DG is None:
+            return (None,) * 5
+        db = colsum(DG)
+        return dW_ih, dW_hh, db, db.clone(), None
+
+
 class _Step(torch.autograd.Function):
     @staticmethod
     def forward(ctx, anchor, att_c, h_prev, c_prev, state, i):
@@ -132,6 +162,10 @@ class _Step(torch.autograd.Function):
         xc, hp, cp = _lib.f32c(att_c.detach()), _lib.f32c(h_prev.detach()), _lib.f32c(c_prev.detach())
         B, Z = hp.shape
         row = state.tok[i] if state.tok is not None else None          # token lookup: egates is the (V, 4Z) table
+        if state.rows0 is not None:                                    # stacked: egates is the bias row (1, 4Z)
+            if state.rows0.numel() != B:
+                state.rows0 = torch.zeros(B, device=dev, dtype=torch.int32)
+            row = state.rows0
         eg = state.egates[i] if row is None else state.egates
         D = xc.shape[1]
         gates = torch.empty(B, 4 * Z, device=dev, dtype=torch.float32)
@@ -217,6 +251,16 @@ class LSTMLoop(object):
         self.state = _State()
         self.anchor = _TokenAnchor.apply(W_ih[:, E:].contiguous(), cell.weight_hh, W_ih[:, :E], cell.bias_ih,
                                          cell.bias_hh, embed_weight, table, tok, self.state)
+        return self
+
+    @classmethod
+    def stacked(cls, cell):
+        """The loop of an upper decoder layer, ``cell`` = LSTMCell(Z, Z) whose whole input is the layer below's state:
+        ``step(i, h_below, h_prev, c_prev)``."""
+        self = cls.__new__(cls)
+        self.state = _State()
+        self.state.rows0 = torch.zeros(0, device=cell.weight_ih.device, dtype=torch.int32)   # sized at the first step
+        self.anchor = _StackedAnchor.apply(cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, self.state)
         return self
 
     def step(self, i, att_c, h_prev, c_prev):
