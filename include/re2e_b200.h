@@ -113,7 +113,16 @@ int re2e_attloc_init_att(const int32_t *hlens, float *att_prev, int B, int Th, v
  * through distributed shared memory).  Optional outputs (NULL when not needed):
  *   dec_proj (B,A) = dec_z @ W_dec^T
  *   conv (B,Th,C)  = loc_conv(att_prev)                               (saved for the backward)
- *   xsave (B,Th,A) = tanh(mlp_att(conv) + pre + dec_proj)             (saved for the backward) */
+ *   xsave (B,Th,A) = tanh(mlp_att(conv) + pre + dec_proj)             (saved for the backward)
+ * Shapes: one cluster of up to 16 CTAs per utterance, each CTA holding its frame range on chip; the grid runs in waves
+ * when it has more CTAs than the GPU has SMs.  Supported, in both directions: B <= 128 with Th <= 1000 at the default
+ * dims (D = A = 320, Z = 300, C = 10, K = 201), and B <= 128 with Th <= 512 at D = A = 512.  Other shapes:
+ * RE2E_E_UNSUPPORTED, returned before anything is launched.
+ * re2e_attloc_step_supported: 1 when both directions take the shape, else 0; *cl_fwd_host / *cl_bwd_host (either may
+ * be NULL) receive the cluster size of each direction, 0 where it is unsupported.  Needs no device (the SM count is
+ * then taken as the B200's 148). */
+int re2e_attloc_step_supported(int B, int Th, int D, int A, int Z, int C, int K, int *cl_fwd_host,
+                               int *cl_bwd_host);
 int re2e_attloc_step_fwd(const float *pre, const float *enc_h, const float *dec_z,
                          const float *att_prev, const float *W_dec, const float *W_att,
                          const float *W_conv, const float *gvec, const float *gvec_b,
@@ -135,7 +144,9 @@ int re2e_attloc_step_fwd(const float *pre, const float *enc_h, const float *dec_
  *                         dgvec_b 1]; zero them once per decoder loop, every step ADDS into them without atomics
  *                         (one slot per CTA), re2e_attloc_acc_reduce sums the slots after the loop.
  * d enc_h is NOT produced here: sum_i w_i (x) dc_i is a rank-(#steps) update applied once by
- * re2e_attloc_enc_grad after the loop (no per-step read-modify-write of (B,Th,D)). */
+ * re2e_attloc_enc_grad after the loop (no per-step read-modify-write of (B,Th,D)).
+ * re2e_attloc_acc_slots: B * (the backward's cluster size) for the shapes re2e_attloc_step_fwd lists as supported,
+ * RE2E_E_UNSUPPORTED otherwise; re2e_attloc_step_bwd returns RE2E_E_WORKSPACE for fewer slots. */
 size_t re2e_attloc_acc_floats(int A, int C, int K);
 int re2e_attloc_acc_slots(int B, int Th, int D, int A, int Z, int C, int K);
 int re2e_attloc_step_bwd(const float *dc, const float *dw, const float *xsave, const float *enc_h,
@@ -148,7 +159,7 @@ int re2e_attloc_step_bwd(const float *dc, const float *dw, const float *xsave, c
 int re2e_attloc_acc_reduce(const float *acc_slots, int n_slots, float *out, int A, int C, int K,
                            void *stream);
 
-/* d_enc_h[b,t,:] (+)= sum_i w_all[i,b,t] * dc_all[i,b,:]   (i < steps); accumulate != 0 adds. */
+/* d_enc_h[b,t,:] (+)= sum_i w_all[i,b,t] * dc_all[i,b,:]   (i < steps, any number of steps); accumulate != 0 adds. */
 int re2e_attloc_enc_grad(const float *w_all, const float *dc_all, float *d_enc_h, int steps,
                          int B, int Th, int D, int accumulate, void *stream);
 

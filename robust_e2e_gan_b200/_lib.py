@@ -38,6 +38,7 @@ SIGNATURES = {
     "re2e_mask_apply_bwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "re2e_cmvn_stats": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "re2e_attloc_init_att": (_I, [_P, _P, _I, _I, _P]),
+    "re2e_attloc_step_supported": (_I, [_I] * 7 + [_P, _P]),
     "re2e_attloc_step_fwd": (_I, [_P] * 9 + [_F] + [_P] * 5 + [_I] * 7 + [_P]),
     "re2e_attloc_acc_floats": (_SZ, [_I, _I, _I]),
     "re2e_attloc_acc_slots": (_I, [_I] * 7),

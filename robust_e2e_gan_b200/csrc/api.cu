@@ -43,6 +43,41 @@ int num_sms() {
   cache[dev] = sms;
   return sms;
 }
+
+bool cluster_fits(const void *func, int cluster_x, int threads, size_t smem) {
+  static std::mutex mu;
+  static std::map<std::pair<std::pair<int, const void *>, std::pair<int, size_t>>, bool> cache;
+  int ndev = 0, dev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || cudaGetDevice(&dev) != cudaSuccess) {
+    cudaGetLastError();
+    return true;   // no device: host-only shape queries
+  }
+  std::lock_guard<std::mutex> lk(mu);
+  auto key = std::make_pair(std::make_pair(dev, func), std::make_pair(cluster_x, smem));
+  auto it = cache.find(key);
+  if (it != cache.end()) return it->second;
+  int n = 0;
+  cudaError_t e = ensure_smem(func, smem) == RE2E_OK ? cudaSuccess : cudaErrorInvalidValue;
+  if (e == cudaSuccess && cluster_x > 8) e = cudaFuncSetAttribute(func, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+  if (e == cudaSuccess) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)cluster_x);
+    cfg.blockDim = dim3((unsigned)threads);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = (unsigned)cluster_x;
+    attr.val.clusterDim.y = 1;
+    attr.val.clusterDim.z = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = 1;
+    e = cudaOccupancyMaxActiveClusters(&n, func, &cfg);
+  }
+  if (e != cudaSuccess) cudaGetLastError();   // a refused query must not surface as the status of a later launch
+  const bool ok = e == cudaSuccess && n > 0;
+  cache[key] = ok;
+  return ok;
+}
 }  // namespace re2e
 
 namespace re2e {
@@ -96,7 +131,7 @@ extern "C" int re2e_colsum(const float *X, long long ld, int rows, int cols, flo
   return launch_status();
 }
 
-extern "C" int re2e_abi_version(void) { return 8; }
+extern "C" int re2e_abi_version(void) { return 9; }
 
 extern "C" const char *re2e_build_info(void) {
   return "re2e_b200 sm_100a nvcc " __DATE__ " " __TIME__

@@ -108,6 +108,9 @@ constexpr int kFP = 8;                  // warp pairs = frames per chunk
 constexpr int kFW = 2 * kFP;            // compute warps
 constexpr int kFT = kFW * 32;
 constexpr int kDpl = 8;                 // D <= 512: encoder channels per lane per half
+static_assert(8 * (kMaxStages + 2) <= 256, "forward: the mbarriers must leave bytes 256..383 of the header to the exchange");
+// rows of the partial-context buffer: 8 up to clusters of 8
+inline int fwd_rank_rows(int CL) { return CL > 8 ? CL : 8; }
 
 template <int APL, int CP, int DPL>
 __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p) {
@@ -139,8 +142,8 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
   float *e_s = conv_s + g.tloc_max * CPP;                  // round4(tloc_max)  scaled energies
   float *epart = e_s + round4(g.tloc_max);                 // 2*tloc_max  per-frame partial energies of the two halves
   float *wstat = epart + round4(2 * g.tloc_max);           // kFW*2
-  float *cbuf = wstat + 2 * kFW;                           // 8*Dp   partial contexts (used on rank 0)
-  float *xch = cbuf + 8 * Dp;                              // 8*2    (max, sum) of every rank
+  float *cbuf = wstat + 2 * kFW;                           // max(CL,8)*Dp  partial contexts (used on rank 0)
+  float *xch = reinterpret_cast<float *>(smraw + 256);     // 2*16   (max, sum) of every rank, behind the mbarriers
   float *cred = stages;                                    // kFP*Dp, aliases the ring once it is drained
 
   ATT_MARK(0, 0);
@@ -1205,6 +1208,9 @@ enc_grad_kernel(const float *__restrict__ w_all, const float *__restrict__ dc_al
 }
 
 // forward (v3) geometry: stage = kFP frames of (pre | enc); the ring holds the whole frame range when it fits
+// Clusters of 16 are non-portable: the pickers ask the device whether one fits at the chosen shared-memory size.  Every
+// instantiation of a direction runs the same block (__launch_bounds__(threads, 1), dynamic shared memory only), so the
+// default-dims instantiation stands for all of them.
 inline bool pick_geom_fwd(int B, int Th, int D, int A, int Z, int C, int K, int CP, int &CL, AttGeom &g,
                           size_t &smem) {
   const int sms = num_sms();
@@ -1216,22 +1222,31 @@ inline bool pick_geom_fwd(int B, int Th, int D, int A, int Z, int C, int K, int 
   g.Thp = round4(Th);
   g.CKp = round4(C * K);
   g.App = round4(Th + 2 * filts + 8);
-  g.tloc_max = (Th + CL - 1) / CL;
-  g.nch = (g.tloc_max + kFP - 1) / kFP;
-  const size_t fixed = 512 + sizeof(float) * ((size_t)g.App + g.CKp + (size_t)A * (CP + 1) + round4(Z) + A +
-                                              (size_t)round4(kKQ * g.tloc_max * CP) + (size_t)g.tloc_max * round4(CP) +
-                                              round4(g.tloc_max) + round4(2 * g.tloc_max) +
-                                              2 * kFW + 8 * (size_t)round4(D) + 16);
   const size_t budget = 224 * 1024;
   const size_t stage_bytes = sizeof(float) * (size_t)g.stage_floats;
-  if (fixed + 2 * stage_bytes > budget) return false;
+  size_t fixed;
+  for (;;) {
+    g.tloc_max = (Th + CL - 1) / CL;
+    g.nch = (g.tloc_max + kFP - 1) / kFP;
+    // the last 16 floats once held the (max, sum) exchange, now in the header: kept so that no size changes
+    fixed = 512 + sizeof(float) * ((size_t)g.App + g.CKp + (size_t)A * (CP + 1) + round4(Z) + A +
+                                   (size_t)round4(kKQ * g.tloc_max * CP) + (size_t)g.tloc_max * round4(CP) +
+                                   round4(g.tloc_max) + round4(2 * g.tloc_max) +
+                                   2 * kFW + (size_t)fwd_rank_rows(CL) * round4(D) + 16);
+    if (fixed + 2 * stage_bytes <= budget) break;
+    // long utterances: the per-frame part of the fixed area shrinks with the CTA's frame range -- split further, up to
+    // the non-portable cluster size of 16 (the grid runs in waves when B*CL CTAs exceed the SMs: clusters do not wait
+    // for each other)
+    if (CL >= 16) return false;
+    CL *= 2;
+  }
   int ns = (int)((budget - fixed) / stage_bytes);
   if (ns > g.nch) ns = g.nch;
   if (ns > kMaxStages) ns = kMaxStages;
   if (ns < 1) ns = 1;
   g.ns = ns;
   smem = fixed + ns * stage_bytes;
-  return true;
+  return CL <= 8 || cluster_fits(reinterpret_cast<const void *>(attloc_fwd_kernel<5, 10, 5>), CL, kFT, smem);
 }
 
 // backward (v3) geometry: all activations of the CTA resident, enc_h through a ring of kBW-frame stages
@@ -1269,10 +1284,12 @@ inline bool pick_geom_bwd(int B, int Th, int D, int A, int Z, int C, int K, int 
       if (ring < alias_bytes) ring = alias_bytes;
       g.ring_floats = (int)(ring / sizeof(float));
       smem = fixed + ring;
-      return true;
+      return CL <= 8 || cluster_fits(reinterpret_cast<const void *>(attloc_bwd_kernel<5, 10, 10>), CL, kBT, smem);
     }
-    // long utterances: split further, up to the non-portable cluster size of 16 (B*16 CTAs must be co-resident)
-    if (CL >= 16 || B * CL * 2 > sms) return false;
+    // long utterances: split further, up to the non-portable cluster size of 16.  Only the CTAs of one cluster need to
+    // be co-resident (they synchronise through DSMEM and the cluster barrier; nothing is shared across clusters), so
+    // the grid may run in waves when B*CL exceeds the SMs.
+    if (CL >= 16) return false;
     CL *= 2;
   }
 }
@@ -1354,6 +1371,22 @@ extern "C" int re2e_attloc_step_fwd(const float *pre, const float *enc_h, const 
   return rc;
 }
 
+extern "C" int re2e_attloc_step_supported(int B, int Th, int D, int A, int Z, int C, int K, int *cl_fwd_host,
+                                          int *cl_bwd_host) {
+  int clf = 0, clb = 0;
+  if (check_dims(B, Th, D, A, C, K) == RE2E_OK && Z > 0) {
+    const int CP = C == 10 ? 10 : 16;
+    AttGeom g;
+    size_t smem;
+    int CL;
+    if (pick_geom_fwd(B, Th, D, A, Z, C, K, CP, CL, g, smem)) clf = CL;
+    if (pick_geom_bwd(B, Th, D, A, Z, C, K, CP, CL, g, smem)) clb = CL;
+  }
+  if (cl_fwd_host) *cl_fwd_host = clf;
+  if (cl_bwd_host) *cl_bwd_host = clb;
+  return clf > 0 && clb > 0;
+}
+
 extern "C" size_t re2e_attloc_acc_floats(int A, int C, int K) {
   return (size_t)round4(A * C + C * K + A + 1);
 }
@@ -1413,17 +1446,29 @@ extern "C" int re2e_attloc_enc_grad(const float *w_all, const float *dc_all, flo
                                     int B, int Th, int D, int accumulate, void *stream) {
   RE2E_CHECK_ARG(w_all && dc_all && d_enc_h && steps > 0 && B > 0 && Th > 0 && D > 0);
   const int tt = 32;   // frames per CTA: the utterance's dc block (steps x D) is re-read Th/tt times from L2
-  const size_t smem = sizeof(float) * ((size_t)round4(steps * D) + (size_t)steps * tt);
-  if (smem > 200 * 1024) return RE2E_E_UNSUPPORTED;
+  // The dc rows of the launch's steps are staged in shared memory (<= 200 KB).  A longer decoder loop runs as several
+  // launches over equal runs of steps, the first with the caller's `accumulate`, the others adding to it: every
+  // element still sums its steps in order, so the result does not depend on the split.
+  const int max_steps = (200 * 1024 / (int)sizeof(float) - 3) / (D + tt);
+  if (max_steps < 1) return RE2E_E_UNSUPPORTED;
+  const int launches = (steps + max_steps - 1) / max_steps;
+  const int per = (steps + launches - 1) / launches;
   {
+    const size_t smem = sizeof(float) * ((size_t)round4(per * D) + (size_t)per * tt);
     int rc0 = ensure_smem(reinterpret_cast<const void *>(enc_grad_kernel), smem);
     if (rc0 != RE2E_OK) return rc0;
   }
   const int tiles = (Th + tt - 1) / tt;
-  enc_grad_kernel<<<B * tiles, kEGThreads, smem, static_cast<cudaStream_t>(stream)>>>(w_all, dc_all, d_enc_h, steps, B,
-                                                                              Th, D, tt, accumulate);
-  count_launch();
-  return launch_status();
+  for (int s0 = 0; s0 < steps; s0 += per) {
+    const int n = min(per, steps - s0);
+    const size_t smem = sizeof(float) * ((size_t)round4(n * D) + (size_t)n * tt);
+    enc_grad_kernel<<<B * tiles, kEGThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+        w_all + (size_t)s0 * B * Th, dc_all + (size_t)s0 * B * D, d_enc_h, n, B, Th, D, tt, s0 == 0 ? accumulate : 1);
+    count_launch();
+    const int rc = launch_status();
+    if (rc != RE2E_OK) return rc;
+  }
+  return RE2E_OK;
 }
 
 // out[M,N] (+)= X[M,K] @ W[N,K]^T   /   X[M,K] @ W[K,N]     (M = batch-sized)

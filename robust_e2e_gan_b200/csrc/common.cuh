@@ -37,6 +37,9 @@ inline int launch_status() {
 }
 
 int num_sms();   // SM count of the CURRENT device (cached per device); defined in api.cu
+// true when at least one cluster of cluster_x CTAs of `threads` threads and `smem` dynamic shared memory bytes can be
+// resident on the current device (cudaOccupancyMaxActiveClusters, cached); true without a device.  Defined in api.cu.
+bool cluster_fits(const void *func, int cluster_x, int threads, size_t smem);
 
 // Launch of a thread-block-cluster kernel in clusters of cluster_x CTAs along x; counts the launch.
 // pdl = true launches with programmatic stream serialisation: the grid may become resident while its predecessor in
