@@ -195,22 +195,14 @@ int re2e_attloc_loop_bwd(const float *pre, const float *enc_h, const float *dec_
                          float *d_decproj, float *acc_slots, int n_slots, int S, int B, int Th, int D, int A,
                          int C, int K, void *stream);
 
-/* Batch-sized ("skinny", M <= a few hundred rows) fp32 products on the per-step path:
- *   out[M,N] (+)= X[M,K] @ W[N,K]^T   (re2e_skinny_nt)   dec_proj = dec_z @ W_dec^T  (mlp_dec, :278)
- *   out[M,N] (+)= X[M,K] @ W[K,N]     (re2e_skinny_nn)   d_dec_z  = d_decproj @ W_dec */
-int re2e_skinny_nt(const float *X, const float *W, float *out, int M, int N, int K, int accumulate,
-                   void *stream);
-int re2e_skinny_nn(const float *X, const float *W, float *out, int M, int N, int K, int accumulate,
-                   void *stream);
-
 /* LSTMCell step of the attention decoder (model/e2e_decoder.py:128, torch.nn.LSTMCell, gate order i,f,g,o), fused
- * pointwise part (csrc/lstm.cu).  The caller forms the recurrent products with re2e_skinny_nt into `gates` (B,4Z):
+ * pointwise part (csrc/lstm.cu).  The caller forms the recurrent products with re2e_batch_nt into `gates` (B,4Z):
  *   gates = context @ W_ih[:, Z:]^T + h_prev @ W_hh^T ;  egate (B,4Z, optional) = embed(y) @ W_ih[:, :Z]^T + b_ih + b_hh
  * (the embedding half of every position comes from ONE dense product before the loop).
  *   fwd: gates <- gate activations (i,f,g,o) in place (saved for the backward); c_out, h_out (B,Z).  c_prev NULL = zeros.
  *   bwd: dh / dc = gradients arriving at (h_out, c_out), NULL = zero; dgates (B,4Z) w.r.t. the pre-activation gates
- *        (d context = dgates @ W_ih[:, Z:], d h_prev = dgates @ W_hh via re2e_skinny_nn; weight gradients of all steps are
- *        two dense products after the loop); dc_prev (B,Z). */
+ *        (d context = dgates @ W_ih[:, Z:], d h_prev = dgates @ W_hh via re2e_batch_nt on transposed weight copies;
+ *        weight gradients of all steps are two dense products after the loop); dc_prev (B,Z). */
 /* out[M,N] (+)= X[M,K] @ W[N,K]^T for a batch-sized M and long N / K (the decoder's per-position recurrent products,
  * N or K = 4Z): one CTA per 8 output columns so that all SMs stream the weight matrix once, reduction staged in chunks
  * (128-bit staging when K % 4 == 0 and X, W are 16 B aligned, scalar staging otherwise).  The backward uses it on transposed weight copies made once per loop. */

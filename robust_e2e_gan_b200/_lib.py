@@ -49,8 +49,6 @@ SIGNATURES = {
     "re2e_attloc_loop_slots": (_I, [_I] * 7),
     "re2e_attloc_loop_fwd": (_I, [_P] * 8 + [_F] + [_P] * 3 + [_I] * 7 + [_P]),
     "re2e_attloc_loop_bwd": (_I, [_P] * 11 + [_F] + [_P] * 3 + [_I] * 8 + [_P]),
-    "re2e_skinny_nt": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
-    "re2e_skinny_nn": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "re2e_batch_nt": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "re2e_sample_tokens_ws_bytes": (_I, [_I]),
     "re2e_sample_tokens": (_I, [_P] * 6 + [_I, _I, _I, _P]),

@@ -131,7 +131,7 @@ extern "C" int re2e_colsum(const float *X, long long ld, int rows, int cols, flo
   return launch_status();
 }
 
-extern "C" int re2e_abi_version(void) { return 9; }
+extern "C" int re2e_abi_version(void) { return 10; }
 
 extern "C" const char *re2e_build_info(void) {
   return "re2e_b200 sm_100a nvcc " __DATE__ " " __TIME__

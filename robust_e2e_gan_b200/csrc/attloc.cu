@@ -26,27 +26,6 @@
 namespace re2e {
 namespace {
 
-#ifdef RE2E_ATT_DEBUG
-// per-CTA phase timestamps (thread 0), 16 slots per CTA, read back with re2e_att_debug_read
-__device__ long long g_att_dbg[2][16 * 512];
-__device__ __forceinline__ long long att_gtime() {
-  long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define ATT_MARK(which, slot)                                                          \
-  do {                                                                                 \
-    if (threadIdx.x == 0) g_att_dbg[which][blockIdx.x * 16 + (slot)] = att_gtime();    \
-  } while (0)
-#define ATT_MARK_T(which, slot, t)                                                       \
-  do {                                                                                 \
-    if (threadIdx.x == (t)) g_att_dbg[which][blockIdx.x * 16 + (slot)] = att_gtime();  \
-  } while (0)
-#else
-#define ATT_MARK(which, slot)
-#define ATT_MARK_T(which, slot, t)
-#endif
-
 constexpr int kMaxStages = 30;
 
 struct AttGeom {
@@ -146,7 +125,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
   float *xch = reinterpret_cast<float *>(smraw + 256);     // 2*16   (max, sum) of every rank, behind the mbarriers
   float *cred = stages;                                    // kFP*Dp, aliases the ring once it is drained
 
-  ATT_MARK(0, 0);
   auto issue = [&](int q) {
     const int st = q % g.ns;
     const int r0 = t0 + kFP * q;
@@ -259,7 +237,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
     for (int i = tid + NT; i < Z; i += NT) dz_s[i] = p.dec_z ? __ldcg(p.dec_z + (size_t)b * Z + i) : 0.0f;
   }
   __syncthreads();  // #1
-  ATT_MARK(0, 1);
 
   // ---- mlp_dec slice of this CTA: channels [rank*A/CL, (rank+1)*A/CL), one warp per channel, lane <-> z
   for (int base = 0; base < apc; base += kFW * kCPW) {
@@ -316,7 +293,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
     }
   }
 
-  ATT_MARK(0, 2);
   // ---- location convolution: conv[t,c] = sum_k Wc[c,k] * att_prev[t + k - filts]  (zero padded).
   //      item = (k quarter, channel, group of 5 frames): 2 shared loads per 5 FMAs
   {
@@ -358,7 +334,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
       WattP[jp][c] = make_float2(c < C ? watt_s[a0 * WP + c] : 0.0f, (c < C && 2 * jp + 1 < APL) ? watt_s[a1 * WP + c] : 0.0f);
   }
   __syncthreads();  // #2
-  ATT_MARK(0, 3);
   for (int i = tid; i < tloc * CPP; i += NT) {
     const int tl = i / CPP, c = i - tl * CPP;
     float v = 0.0f;
@@ -371,7 +346,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
   }
   if (p.dec_z) mbar_wait(dpbar, 0);   // dp_s holds the full dec_proj row (A floats pushed by the CTAs of the cluster)
   __syncthreads();  // #3: conv_s visible
-  ATT_MARK(0, 4);
 
   float m_run = -CUDART_INF_F, s_run = 0.0f;
   float acc[DPL];
@@ -395,7 +369,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
       const uint32_t ph = (uint32_t)((qg / g.ns) & 1);
       if (whole) { if (tloc > 0) mbar_wait(&full[0], 0); }
       else for (int i = 0; i < gsz; ++i) mbar_wait(&full[i], ph);
-      ATT_MARK(0, 8);
       // (1) partial energies of this warp's half of the channels
 #pragma unroll 2
       for (int i = 0; i < gsz; ++i) {
@@ -430,9 +403,7 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
           if (lane == 0) epart[2 * tl + half] = part;
         }
       }
-      ATT_MARK(0, 9);
       pair_bar(1 + pair, 64);
-      ATT_MARK(0, 10);
       if (gsz <= 8) {
         // common case (<= 8 frames per pair and group): everything of steps (2) and (3) for the group's frames is
         // issued up front -- 16 broadcast LDS, 8 exponentials, 8*DPL independent LDS -- instead of one frame at a
@@ -507,7 +478,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
         }
       }
       }
-      ATT_MARK(0, 11);
       if (qg + g.ns < nch) {   // ring shorter than the frame range (long utterances): refill behind a CTA barrier
         __syncthreads();
         if (tid == 0) {
@@ -519,7 +489,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
     if (lane == 0) { wstat[2 * warp] = m_run; wstat[2 * warp + 1] = s_run; }
   }
   __syncthreads();  // #4: ring drained, per-warp statistics published
-  ATT_MARK(0, 5);
 
   // ---- CTA combine (deterministic order), then push to the cluster
   float Mc = -CUDART_INF_F;
@@ -548,7 +517,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
     st_async_f32(dsmem_addr(xch + 2 * rank, (uint32_t)tid), Mc, dsmem_addr(xbar, (uint32_t)tid));
     st_async_f32(dsmem_addr(xch + 2 * rank + 1, (uint32_t)tid), sc, dsmem_addr(xbar, (uint32_t)tid));
   }
-  ATT_MARK(0, 6);
   mbar_wait(xbar, 0);   // every rank's (max, sum) -- and on rank 0 every partial context -- has landed here
   float M = -CUDART_INF_F;
   for (int r = 0; r < CL; ++r) M = fmaxf(M, xch[2 * r]);
@@ -565,7 +533,6 @@ __global__ void __launch_bounds__(kFT, 1) attloc_fwd_kernel(const AttFwdParams p
       p.c[(size_t)b * D + d] = sum * inv;
     }
   }
-  ATT_MARK(0, 7);
   // no trailing cluster barrier: a CTA leaves only after everything addressed to it has landed (xbar), and it
   // never reads remote shared memory
 }
@@ -633,7 +600,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
   float *xch = ddp_t + A;                                   // 16      sum_t w dwt partials of every rank
   float *slot = p.acc_slots + (size_t)blockIdx.x * p.slot_stride;   // [dW_att A*C | dW_conv C*K | dgvec A | dgvec_b 1]
 
-  ATT_MARK(1, 0);
   const bool whole_e = g.ns >= nche;   // the enc_h ring holds the CTA's whole frame range
   auto issue_e = [&](int q) {
     const int st = q % g.ns;
@@ -744,7 +710,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
   for (int j = 0; j < DPL2; ++j) dcr[j] = (p.dc && lane + 32 * j < D) ? __ldcg(p.dc + (size_t)b * D + lane + 32 * j) : 0.0f;
   for (int i = tid; i < tloc; i += NT) dwt_s[i] = p.dw ? __ldcg(p.dw + (size_t)b * Th + t0 + i) : 0.0f;
   __syncthreads();  // #1
-  ATT_MARK(1, 1);
 
   // ---- pass 1: dwt[t] = dw[t] + enc_h[t,:] . dc   (warp per frame, lane <-> d)
   {
@@ -781,7 +746,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
       WattC[j][c2] = make_float2(2 * c2 < C ? watt_s[a * WP + 2 * c2] : 0.0f, 2 * c2 + 1 < C ? watt_s[a * WP + 2 * c2 + 1] : 0.0f);
   }
   __syncthreads();  // #2: dwt complete; the enc ring is free
-  ATT_MARK(1, 2);
   cluster_wait();   // peers are resident: remote stores may start
   if (warp == 0) {
     float s1 = 0.0f;
@@ -794,7 +758,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
   for (int r = 0; r < CL; ++r) Stot += xch[r];
   for (int tl = tid; tl < tloc; tl += NT) de_s[tl] = p.scaling * w_s[tl] * (dwt_s[tl] - Stot);
   __syncthreads();  // #3
-  ATT_MARK(1, 3);
 
   // ---- pass 2: through tanh.  pair <-> frame, lane <-> channel
   float dgv[APL], ddp[APL];
@@ -855,7 +818,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
     }
   }
   __syncthreads();  // #4: all d pre tiles written, per-warp partials published
-  ATT_MARK(1, 4);
 
   // ---- d dec_z[z] = sum_a d dec_proj[a] W_dec[a,z] for this rank's slice of z, from the TRANSPOSED weight
   //      W_decT (Z x A, built once per decoder loop): row z is one contiguous, 16 B aligned run of A floats, so the
@@ -880,7 +842,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
     }
   };
   if (p.d_dec_z) load_wz(0);
-  ATT_MARK(1, 10);
 
   // ---- post pass A (needs nothing from the other CTAs)
   // d conv of this CTA's frames -> every CTA of the cluster (channel-major, padded)
@@ -904,14 +865,12 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
       st_async_f32(dsmem_addr(ddp_x + rank * A + a, (uint32_t)r), sd, dsmem_addr(xbar2, (uint32_t)r));
     slot[A * C + C * K + a] = sg0 + sg;
   }
-  ATT_MARK(1, 11);
   if (warp == kBW - 1) {   // d gvec.bias = sum_t de[t]  (analytically zero over the utterance; kept for fidelity)
     float s2 = 0.0f;
     for (int tl = lane; tl < tloc; tl += 32) s2 += de_s[tl];
     s2 = warp_sum(s2);
     if (lane == 0 && tloc > 0) slot[A * C + C * K + A] += s2;
   }
-  ATT_MARK_T(1, 12, NT - 1);
   // The two parameter gradients that only need THIS CTA's frames run side by side on disjoint sets of warps:
   //   threads [0, A)       : dW_att[a,c] += sum_t d pre[t,a] conv[t,c]   straight from the resident tile (thread <-> a)
   //   threads [A, NT)      : dW_conv[c,k] += sum_{t in mine} dconv[t,c] att_prev[t + k - filts]  (6 taps per item)
@@ -966,10 +925,7 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
       }
     }
   }
-  ATT_MARK(1, 5);
-  ATT_MARK_T(1, 13, NT - 1);
   mbar_wait(xbar2, 0);
-  ATT_MARK(1, 14);   // d conv of all Th frames and every rank's d dec_proj partial have landed here
   for (int a = tid; a < A; a += NT) {
     float sd = 0.0f;
     for (int r = 0; r < CL; ++r) sd += ddp_x[r * A + a];
@@ -977,7 +933,6 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
     if (rank == 0) p.d_decproj[(size_t)b * A + a] = sd;
   }
   __syncthreads();  // #5 (also: scr aliases the per-warp partials read above)
-  ATT_MARK(1, 6);
 
   // ---- post pass B
   // d dec_z from the prefetched W_decT rows: one dot product of length A per z row, reduced inside the warp
@@ -1030,16 +985,13 @@ __global__ void __launch_bounds__(kBT, 1) attloc_bwd_kernel(const AttBwdParams p
       if (nv > 4) o[4] = a4;
     }
     __syncthreads();  // #6
-    ATT_MARK(1, 7);
     for (int tl = tid; tl < tloc; tl += NT) {
       float sum = 0.0f;
       for (int i = 0; i < kKQ * C; ++i) sum += scr[(size_t)i * g.tloc_max + tl];
       p.d_att_prev[(size_t)b * Th + t0 + tl] = sum;
     }
   }
-  ATT_MARK(1, 8);
   if (tid == 0) bulk_wait<0>();  // all d_pre traffic of this CTA has left shared memory / landed
-  ATT_MARK(1, 9);
 }
 
 // out[i] = sum_s slots[s*stride + i]   -- once per decoder loop, fixed summation order.
@@ -1071,78 +1023,6 @@ acc_reduce_kernel(const float *__restrict__ slots, int n_slots, int stride, int 
 // ------------------------------------------------------------------------------------------------
 // small helpers
 // ------------------------------------------------------------------------------------------------
-// out[m,n] (+)= sum_k X[m,k] * W[n,k] (NT) or W[k,n] (NN);  M small (batch).  One warp per output column,
-// lane <-> row m; X and the CTA's slab of W are staged with 128-bit loads issued back to back.
-constexpr int kSkWarps = 16;
-template <bool NN>
-__global__ void __launch_bounds__(kSkWarps * 32) skinny_gemm_kernel(const float *__restrict__ X,
-                                                                   const float *__restrict__ W,
-                                                                   float *__restrict__ out, int M, int N, int Kd,
-                                                                   int accumulate, int vec_ok) {
-  extern __shared__ __align__(16) float smem[];
-  constexpr int NT = kSkWarps * 32;
-  const int Kp = Kd | 1;                   // odd pitch: lane <-> row reads are conflict free
-  float *x_s = smem;                       // [M][Kp]
-  float *w_s = smem + round4(M * Kp);      // [kSkWarps][Kd], 16 B aligned for the float4 stores
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int n0 = blockIdx.x * kSkWarps;
-  if (vec_ok) {
-    const int k4n = Kd >> 2;
-    for (int i = tid; i < M * k4n; i += NT) {
-      const int m = i / k4n, k4 = i - m * k4n;
-      const float4 v = __ldg(reinterpret_cast<const float4 *>(X + (size_t)m * Kd) + k4);
-      float *d = x_s + m * Kp + 4 * k4;
-      d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
-    }
-  } else {
-    for (int i = tid; i < M * Kd; i += NT) {
-      const int m = i / Kd, k = i - m * Kd;
-      x_s[m * Kp + k] = __ldg(X + i);
-    }
-  }
-  if (NN) {
-    for (int i = tid; i < kSkWarps * Kd; i += NT) {
-      const int k = i / kSkWarps, w4 = i - k * kSkWarps;
-      const int n = n0 + w4;
-      w_s[w4 * Kd + k] = n < N ? __ldg(W + (size_t)k * N + n) : 0.0f;
-    }
-  } else if (vec_ok) {
-    const int k4n = Kd >> 2;
-    for (int i = tid; i < kSkWarps * k4n; i += NT) {
-      const int w4 = i / k4n, k4 = i - w4 * k4n;
-      const int n = n0 + w4;
-      float4 v = make_float4(0, 0, 0, 0);
-      if (n < N) v = __ldg(reinterpret_cast<const float4 *>(W + (size_t)n * Kd) + k4);
-      *reinterpret_cast<float4 *>(w_s + w4 * Kd + 4 * k4) = v;
-    }
-  } else {
-    for (int i = tid; i < kSkWarps * Kd; i += NT) {
-      const int w4 = i / Kd, k = i - w4 * Kd;
-      const int n = n0 + w4;
-      w_s[w4 * Kd + k] = n < N ? __ldg(W + (size_t)n * Kd + k) : 0.0f;
-    }
-  }
-  __syncthreads();
-  const int n = n0 + warp;
-  if (n >= N) return;
-  const float *wr = w_s + warp * Kd;
-  for (int m = lane; m < M; m += 32) {
-    const float *xr = x_s + m * Kp;
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-    int k = 0;
-    for (; k + 3 < Kd; k += 4) {
-      a0 = fmaf(xr[k], wr[k], a0);
-      a1 = fmaf(xr[k + 1], wr[k + 1], a1);
-      a2 = fmaf(xr[k + 2], wr[k + 2], a2);
-      a3 = fmaf(xr[k + 3], wr[k + 3], a3);
-    }
-    for (; k < Kd; ++k) a0 = fmaf(xr[k], wr[k], a0);
-    const float v = (a0 + a1) + (a2 + a3);
-    float *o = out + (size_t)m * N + n;
-    *o = accumulate ? *o + v : v;
-  }
-}
-
 __global__ void init_att_kernel(const int32_t *__restrict__ hlens, float *__restrict__ att, int B, int Th) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * Th) return;
@@ -1310,35 +1190,10 @@ int run_bwd(const AttBwdParams &prm, int CL, size_t smem, cudaStream_t st) {
   return launch_cluster(attloc_bwd_kernel<APL, CP, 2 * kDpl>, grid, dim3(kBT), smem, st, CL, true, prm);
 }
 
-int skinny(bool nn, const float *X, const float *W, float *out, int M, int N, int Kd, int accumulate,
-           cudaStream_t st) {
-  const size_t smem = sizeof(float) * ((size_t)round4(M * (Kd | 1)) + (size_t)kSkWarps * Kd);
-  if (smem > 200 * 1024) return RE2E_E_UNSUPPORTED;
-  const int vec_ok = ((Kd & 3) == 0) && aligned16(X) && aligned16(W);
-  int rc0;
-  const int grid = (N + kSkWarps - 1) / kSkWarps;
-  if (nn) {
-    if ((rc0 = ensure_smem(reinterpret_cast<const void *>(skinny_gemm_kernel<true>), smem)) != RE2E_OK) return rc0;
-    skinny_gemm_kernel<true><<<grid, kSkWarps * 32, smem, st>>>(X, W, out, M, N, Kd, accumulate, vec_ok);
-  } else {
-    if ((rc0 = ensure_smem(reinterpret_cast<const void *>(skinny_gemm_kernel<false>), smem)) != RE2E_OK) return rc0;
-    skinny_gemm_kernel<false><<<grid, kSkWarps * 32, smem, st>>>(X, W, out, M, N, Kd, accumulate, vec_ok);
-  }
-  count_launch();
-  return launch_status();
-}
-
 }  // namespace
 }  // namespace re2e
 
 using namespace re2e;
-
-#ifdef RE2E_ATT_DEBUG
-extern "C" int re2e_att_debug_read(long long *host_out, int which) {
-  cudaDeviceSynchronize();
-  return (int)cudaMemcpyFromSymbol(host_out, g_att_dbg, sizeof(long long) * 16 * 512, sizeof(long long) * 16 * 512 * which);
-}
-#endif
 
 extern "C" int re2e_attloc_init_att(const int32_t *hlens, float *att_prev, int B, int Th, void *stream) {
   RE2E_CHECK_ARG(hlens && att_prev && B > 0 && Th > 0);
@@ -1469,16 +1324,4 @@ extern "C" int re2e_attloc_enc_grad(const float *w_all, const float *dc_all, flo
     if (rc != RE2E_OK) return rc;
   }
   return RE2E_OK;
-}
-
-// out[M,N] (+)= X[M,K] @ W[N,K]^T   /   X[M,K] @ W[K,N]     (M = batch-sized)
-extern "C" int re2e_skinny_nt(const float *X, const float *W, float *out, int M, int N, int K,
-                              int accumulate, void *stream) {
-  RE2E_CHECK_ARG(X && W && out && M > 0 && N > 0 && K > 0);
-  return skinny(false, X, W, out, M, N, K, accumulate, static_cast<cudaStream_t>(stream));
-}
-extern "C" int re2e_skinny_nn(const float *X, const float *W, float *out, int M, int N, int K,
-                              int accumulate, void *stream) {
-  RE2E_CHECK_ARG(X && W && out && M > 0 && N > 0 && K > 0);
-  return skinny(true, X, W, out, M, N, K, accumulate, static_cast<cudaStream_t>(stream));
 }

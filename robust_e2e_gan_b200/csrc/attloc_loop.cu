@@ -29,34 +29,6 @@
 namespace re2e {
 namespace {
 
-#ifdef RE2E_ATT_DEBUG
-// per-CTA phase clocks (thread 0): cycles spent between consecutive marks, summed over all steps of the loop;
-// 16 slots per CTA and direction, read back with re2e_loop_debug_read (tools/loop_debug.py)
-__device__ long long g_loop_dbg[2][16 * 512];
-#define LOOP_DBG_DECL                                                  \
-  __shared__ long long dbg_acc[16];                                    \
-  if (threadIdx.x == 0)                                                \
-    for (int i_ = 0; i_ < 16; ++i_) dbg_acc[i_] = 0;                   \
-  long long dbg_last = clock64()
-#define LOOP_MARK(slot)                                              \
-  do {                                                               \
-    if (threadIdx.x == 0) {                                          \
-      const long long t_ = clock64();                                \
-      dbg_acc[slot] += t_ - dbg_last;                                \
-      dbg_last = t_;                                                 \
-    }                                                                \
-  } while (0)
-#define LOOP_DBG_FLUSH(which)                                                                   \
-  do {                                                                                          \
-    if (threadIdx.x == 0)                                                                       \
-      for (int i_ = 0; i_ < 16; ++i_) g_loop_dbg[which][blockIdx.x * 16 + i_] = dbg_acc[i_];    \
-  } while (0)
-#else
-#define LOOP_DBG_DECL
-#define LOOP_MARK(slot)
-#define LOOP_DBG_FLUSH(which)
-#endif
-
 __device__ __forceinline__ void cp_async4(void *dst_smem, const void *src_gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
 }
@@ -207,8 +179,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
   const int aoff = half * (A / 2) + lane;
   cluster_wait();                            // every peer CTA is resident, its mbarriers initialised
   if (tloc > 0) mbar_wait(full, 0);
-  LOOP_DBG_DECL;
-  LOOP_MARK(0);   // prologue
 
   for (int s = 0; s < S; ++s) {
     const uint32_t par = (uint32_t)s & 1u, ph = ((uint32_t)s >> 1) & 1u;
@@ -248,7 +218,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
       }
     }
     __syncthreads();  // #1
-    LOOP_MARK(1);   // conv partials
     for (int i = tid; i < tloc * CPP; i += NT) {
       const int tl = i / CPP, c = i - tl * CPP;
       float v = 0.0f;
@@ -260,7 +229,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
       conv_s[i] = v;
     }
     __syncthreads();  // #2: conv_s visible
-    LOOP_MARK(2);   // conv reduce
 
     // ---- energies of step s and, in the same sweep over the resident frames, the context of step s-1 from the
     //      normalised alignment that is still in `app` (the context does not feed the recurrence: it is taken off
@@ -302,9 +270,7 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
 #pragma unroll
     for (int j = 0; j < DPL; ++j)
       if (dmask & (1u << j)) cred[pair * Dp + half * Dh + lane + 32 * j] = acc[j];
-    LOOP_MARK(3);   // energies + context sweep
     __syncthreads();  // #3: partial energies and per-pair partial contexts published
-    LOOP_MARK(4);   // barrier #3
 
     // ---- ONE push per step: context partial of step s-1 -> rank 0, my frames' scaled energies -> every CTA
     for (int d = tid; d < D; d += NT) {
@@ -318,9 +284,7 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
       const float e = p.scaling * ((epart[2 * tl] + epart[2 * tl + 1]) + gb);
       st_async_f32(dsmem_addr(e_cur + t0 + tl, (uint32_t)r), e, dsmem_addr(&xbar[par], (uint32_t)r));
     }
-    LOOP_MARK(5);   // pushes
     mbar_wait(&xbar[par], ph);   // the scaled energies of ALL frames (on rank 0 also the partial contexts) are here
-    LOOP_MARK(6);   // exchange wait
     // softmax statistics of the whole row, redundantly per warp (same order everywhere: bit-identical), no barrier
     float M = -CUDART_INF_F;
     for (int t = lane; t < Th; t += 32) M = fmaxf(M, e_cur[t]);
@@ -344,7 +308,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
     }
     if (tid == 0) mbar_expect_tx(&xbar[par], xbytes);   // re-arm this parity's barrier for step s+2
     __syncthreads();  // #5: alignment row complete; receive buffers of this parity consumed
-    LOOP_MARK(7);   // softmax + outputs
   }
   // ---- tail: the context of the last step
   {
@@ -381,7 +344,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_fwd_kernel(const LoopFwdPa
       }
     }
   }
-  LOOP_DBG_FLUSH(0);
   // no trailing cluster barrier: a CTA leaves only after everything addressed to it has landed (its last wait)
   // and it never reads remote shared memory
 }
@@ -588,8 +550,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
   const int nkg = (K + kKG - 1) / kKG;
   const bool conv_thread = tid >= A && tid - A < C * nkg;
   const int cw_c = conv_thread ? (tid - A) / nkg : 0, cw_kb = conv_thread ? ((tid - A) % nkg) * kKG : 0;
-  LOOP_DBG_DECL;
-  LOOP_MARK(0);   // prologue
 
   for (int it = 0; it < S; ++it) {
     const int s = S - 1 - it;
@@ -621,7 +581,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
       }
     }
     __syncthreads();  // #1
-    LOOP_MARK(1);   // per-step loads
 
     // ---- pass 1: dwt[t] += enc_h[t,:] . dc   (warp per frame, lane <-> d, enc_h from TMEM)
     for (int q = 0; q < nche; ++q) {
@@ -636,7 +595,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
       if (lane == 0 && tl < tloc) dwt_s[tl] += dot;
     }
     __syncthreads();  // #2: dwt complete
-    LOOP_MARK(2);   // pass 1
     if (warp == 0) {
       float s1 = 0.0f;
       for (int tl = lane; tl < tloc; tl += 32) s1 = fmaf(w_s[tl], dwt_s[tl], s1);
@@ -652,7 +610,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
       if (it > 0) bulk_wait<0>();   // the previous step's d pre tile has left shared memory (and landed)
     }
     __syncthreads();  // #3
-    LOOP_MARK(3);   // softmax exchange
 
     // ---- pass 2: recompute x = tanh(W_att conv + pre + dec_proj), through tanh.  pair <-> frame, lane <-> channel
     float ddp[APL];
@@ -723,7 +680,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
         }
       }
     }
-    LOOP_MARK(4);   // pass 2
     fence_proxy_async_smem();   // this thread's tile writes -> visible to the bulk (async proxy) reads
     __syncwarp();
     if (lane == 0) mbar_arrive1(done_x);
@@ -741,7 +697,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
 #pragma unroll
     for (int j = 0; j < APL; ++j) ddp_w[warp * (A / 2) + lane + 32 * j] = ddp[j];
     __syncthreads();  // #4: d pre tile complete, per-warp partials published
-    LOOP_MARK(5);   // TMA hand-off + barrier #4
 
     // ---- post pass A: pushes first (their latency overlaps the parameter-gradient work below)
     for (int item = tid; item < tloc * C; item += NT) {   // d conv of my frames -> every CTA (channel-major, padded)
@@ -762,7 +717,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
       for (int tl = lane; tl < tloc; tl += 32) s2 += de_s[tl];
       dgb += warp_sum(s2);
     }
-    LOOP_MARK(6);   // pushes
     // parameter gradients that only need THIS CTA's frames, side by side on disjoint threads, into registers:
     //   threads [0, A)          : dW_att[a,c]  += sum_t d pre[t,a] conv[t,c]            (thread <-> a, from the tile)
     //   threads [A, A + C*nkg)  : dW_conv[c,k] += sum_t dconv[t,c] att_prev[t+k-filts]  (12 taps per thread)
@@ -794,9 +748,7 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
         for (int i = 0; i < kKG - 1; ++i) x[i] = x[i + 1];
       }
     }
-    LOOP_MARK(7);   // parameter gradients (thread 0: dW_att)
     mbar_wait(&xbar2[par], ph);   // d conv of all Th frames (and on rank 0 every rank's d dec_proj partial) are here
-    LOOP_MARK(8);   // d conv exchange wait
     if (rank == 0) {
       for (int a = tid; a < A; a += NT) {
         float sd = 0.0f;
@@ -835,7 +787,6 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
     }
     if (tid == 0) mbar_expect_tx(&xbar2[par], x2bytes);
     __syncthreads();  // #5
-    LOOP_MARK(9);   // d att_prev partials
     if (s > 0) {
       for (int tl = tid; tl < tloc; tl += NT) {
         float sum = 0.0f;
@@ -843,11 +794,9 @@ __global__ void __launch_bounds__(kLT, 1) attloc_loop_bwd_kernel(const LoopBwdPa
         dwn_s[tl] = sum;
       }
     }
-    LOOP_MARK(10);  // d att_prev reduce
     // the next iteration's barrier #1 orders dwn_s / scr / conv_s / app reuse
   }
 
-  LOOP_DBG_FLUSH(1);
   // ---- epilogue: running parameter gradients -> this CTA's private slot (plain stores; summed by acc_reduce)
   if (tid < A) {
 #pragma unroll
@@ -957,13 +906,6 @@ int run_loop_bwd(const LoopBwdParams &prm, int CL, size_t smem, cudaStream_t st)
 }  // namespace re2e
 
 using namespace re2e;
-
-#ifdef RE2E_ATT_DEBUG
-extern "C" int re2e_loop_debug_read(long long *host_out, int which) {
-  cudaDeviceSynchronize();
-  return (int)cudaMemcpyFromSymbol(host_out, g_loop_dbg, sizeof(long long) * 16 * 512, sizeof(long long) * 16 * 512 * which);
-}
-#endif
 
 extern "C" int re2e_attloc_loop_supported(int S, int B, int Th, int D, int A, int C, int K) {
   if (S <= 0 || check_dims(B, Th, D, A, C, K) != RE2E_OK) return 0;

@@ -51,30 +51,7 @@ struct FbTcParams {
   int ntail;         // trailing bins (<= 4, e.g. the Nyquist bin of F = 257) added by the epilogue as plain FMAs
   int rows_per_cta;
   int nstages;
-  long long *dbg;    // optional per-CTA timing record (RE2E_FB_DEBUG builds only)
 };
-
-#ifdef RE2E_FB_DEBUG
-__device__ __forceinline__ long long gtime() {
-  long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define DBG_T(var) const long long var = gtime()
-#define DBG_ACC(acc, t0) acc += gtime() - (t0)
-#define DBG_C(var) const long long var = clock64()
-#define DBG_CACC(acc, t0) acc += clock64() - (t0)
-#define DBG_PUT(slot, val)                                        \
-  do {                                                            \
-    if (p.dbg) p.dbg[(size_t)blockIdx.x * 16 + (slot)] = (val);   \
-  } while (0)
-#else
-#define DBG_T(var)
-#define DBG_ACC(acc, t0)
-#define DBG_C(var)
-#define DBG_CACC(acc, t0)
-#define DBG_PUT(slot, val)
-#endif
 
 __device__ __forceinline__ float tf32_trunc_lo(float x) {
   // the tensor core reads the top 19 bits of an fp32 operand; what it drops is re-fed as a second operand
@@ -107,11 +84,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
   float *fct_s = c1_s + NB;          // [ntail][NB] filter-bank rows of the trailing bins
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  DBG_T(t_start);
-#ifdef RE2E_FB_DEBUG
-  long long w_acc = 0;
-  long long c_wait = 0, c_conv = 0, c_fence = 0, c_arrive = 0, c_load = 0;   // converter phases, SM clocks
-#endif
   const int row_begin = min(p.N, (int)blockIdx.x * p.rows_per_cta);
   const int row_end = min(p.N, row_begin + p.rows_per_cta);
   const int ntiles = (row_end - row_begin + kRows - 1) / kRows;
@@ -151,8 +123,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const int nitems = ntiles * p.nchunks;
-  DBG_T(t_setup);
-  if (tid == 0) { DBG_PUT(0, t_start); DBG_PUT(1, t_setup - t_start); }
 
   if (PAIR && FC == 257 && warp < kCW) {
     // ================= converters, F = 257 (8 B per lane) =================
@@ -229,16 +199,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
           const int s1 = st;
           const uint32_t ph1 = ph;
           if (++st == NS) { st = 0; ph ^= 1u; }
-          {
-            DBG_T(tw);
-            DBG_C(cw);
-            if (nchunk >= NS) mbar_wait(&empty[s0], ph0 ^ 1u);
-            if (nchunk + 1 >= NS) mbar_wait(&empty[s1], ph1 ^ 1u);
-            DBG_ACC(w_acc, tw);
-            DBG_CACC(c_wait, cw);
-          }
+          if (nchunk >= NS) mbar_wait(&empty[s0], ph0 ^ 1u);
+          if (nchunk + 1 >= NS) mbar_wait(&empty[s1], ph1 ^ 1u);
           nchunk += 2;
-          DBG_C(cc0);
           unsigned char *sa = stage0 + (size_t)(hsel ? s1 : s0) * 2 * kATile + offp;
           const int kcol = 64 * c_g + 2 * lane;
           auto masked_x = [&](float g, float k, bool v) {
@@ -299,18 +262,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
               *reinterpret_cast<float *>(p0 + kATile) = tf32_trunc_lo(x02);
             }
           }
-          DBG_CACC(c_conv, cc0);
-          DBG_C(cc1);
           fence_proxy_async_smem();
-          DBG_CACC(c_fence, cc1);
-          DBG_C(cc2);
           __syncwarp();
           if (lane == 0) { mbar_arrive(&full[s0]); mbar_arrive(&full[s1]); }
-          DBG_CACC(c_arrive, cc2);
           if (++c_g == 4) { c_g = 0; c_row0 += kRows; }
-          DBG_C(cc3);
           if (l_item < npi) load(mg[d], mk[MASKED ? d : 0], eg[d], ek[MASKED ? d : 0]);
-          DBG_CACC(c_load, cc3);
         }
       }
     }
@@ -367,14 +323,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
               }
             }
           }
-          {
-            DBG_T(tw);
-            DBG_C(cw);
-            if (q >= NS) mbar_wait(&empty[st], ph ^ 1u);
-            DBG_ACC(w_acc, tw);
-            DBG_CACC(c_wait, cw);
-          }
-          DBG_C(cc0);
+          if (q >= NS) mbar_wait(&empty[st], ph ^ 1u);
           unsigned char *sa = stage0 + (size_t)st * 2 * kATile + off0;
           const int kcol = c_c * kKC + lane;
 #pragma unroll
@@ -390,19 +339,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
             *reinterpret_cast<float *>(sa + j * 2048) = x2;
             *reinterpret_cast<float *>(sa + kATile + j * 2048) = tf32_trunc_lo(x2);
           }
-          DBG_CACC(c_conv, cc0);
-          DBG_C(cc1);
           fence_proxy_async_smem();
-          DBG_CACC(c_fence, cc1);
-          DBG_C(cc2);
           __syncwarp();
           if (lane == 0) mbar_arrive(&full[st]);
-          DBG_CACC(c_arrive, cc2);
           if (++st == NS) { st = 0; ph ^= 1u; }
           if (++c_c == p.nchunks) { c_c = 0; c_row0 += kRows; }
-          DBG_C(cc3);
           if (l_item < nitems) load(mg[d], mk[MASKED ? d : 0]);
-          DBG_CACC(c_load, cc3);
         }
       }
     }
@@ -419,11 +361,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(buf * WD);
         for (int c = 0; c < p.nchunks; ++c) {
-          {
-            DBG_T(tw);
-            mbar_wait(&full[st], ph);
-            DBG_ACC(w_acc, tw);
-          }
+          mbar_wait(&full[st], ph);
           tc_fence_after();
           const uint32_t a_hi = smem_u32(stage0 + (size_t)st * 2 * kATile);
           const uint32_t a_lo = a_hi + kATile;
@@ -469,11 +407,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
             xt2[kt] = x * x;
           }
       }
-      {
-        DBG_T(tw);
-        mbar_wait(&tfull[buf], (uint32_t)((t >> 1) & 1));
-        DBG_ACC(w_acc, tw);
-      }
+      mbar_wait(&tfull[buf], (uint32_t)((t >> 1) & 1));
       tc_fence_after();
       for (int c16 = 0; c16 < NB; c16 += 16) {
         if (c16 >= M) continue;
@@ -527,19 +461,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) fbank_tc_fwd_kernel(const FbTcP
       if (lane == 0) mbar_arrive(&tempty[buf]);
     }
   }
-#ifdef RE2E_FB_DEBUG
-  if (lane == 0 && (warp == 0 || warp == kCW || warp == kCW + kEW)) {
-    const int base = warp == 0 ? 2 : warp == kCW ? 4 : 6;   // converter / epilogue / mma: (end time, wait time)
-    DBG_PUT(base, gtime() - t_start);
-    DBG_PUT(base + 1, w_acc);
-  }
-#endif
   tc_fence_before();
   __syncthreads();
-  if (tid == 0) DBG_PUT(8, gtime() - t_start);
-#ifdef RE2E_FB_DEBUG
-  if (tid == 0) { DBG_PUT(9, c_wait); DBG_PUT(10, c_conv); DBG_PUT(11, c_fence); DBG_PUT(12, c_arrive); DBG_PUT(13, c_load); }
-#endif
   if (warp == kCW + kEW) {
     tc_fence_after();
     tmem_dealloc(tmem_base, tmem_cols);
@@ -809,15 +732,6 @@ inline size_t fwd_smem_bytes(int nchunks, int MB, int NB, int ns) {
 
 }  // namespace
 
-#ifdef RE2E_FB_DEBUG
-long long *g_fb_dbg = nullptr;
-extern "C" int re2e_fb_debug_read(long long *host_out) {   // 16 x 256 values of the last launch
-  if (!g_fb_dbg) return -1;
-  cudaDeviceSynchronize();
-  return (int)cudaMemcpy(host_out, g_fb_dbg, sizeof(long long) * 16 * 256, cudaMemcpyDeviceToHost);
-}
-#endif
-
 // Whether fbank_tc_fwd has a configuration for (F, M): two accumulator buffers of [hi.hi | hi.lo | lo.hi] columns fit
 // tensor memory and one stage fits shared memory.  Pointer alignment is checked at launch.
 bool fbank_tc_fwd_fits(int F, int M) {
@@ -834,16 +748,6 @@ int fbank_tc_fwd(const float *mask, int mask_is_logit, const float *mag, const f
   FbTcParams p;
   p.mask = mask; p.mag = mag; p.fc = fc; p.cmvn = cmvn; p.lens = lens; p.Y = Y; p.G = G; p.enh = enh_out;
   p.mask_is_logit = mask_is_logit; p.N = B * T; p.T = T; p.F = F; p.M = M;
-  p.dbg = nullptr;
-#ifdef RE2E_FB_DEBUG
-  {
-    static long long *dbg_buf = nullptr;
-    if (!dbg_buf) cudaMalloc(&dbg_buf, sizeof(long long) * 16 * 256);
-    p.dbg = dbg_buf;
-    extern long long *g_fb_dbg;
-    g_fb_dbg = dbg_buf;
-  }
-#endif
   p.NB = (M + 15) / 16 * 16;
   p.MB = (M + 7) / 8 * 8;
   p.ntail = (F >= kKC && (F % kKC) >= 1 && (F % kKC) <= 4) ? F % kKC : 0;

@@ -24,22 +24,6 @@
 namespace re2e {
 namespace {
 
-#ifdef RE2E_GEMM_DEBUG
-__device__ long long g_gemm_dbg[8 * 2048];   // per CTA (first 2048): start, setup done, first stage landed, mma done, epilogue done
-__device__ __forceinline__ long long gemm_gtime() {
-  long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define GEMM_MARK(slot)                                                                                          \
-  do {                                                                                                           \
-    const int cta_ = blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z);                             \
-    if (cta_ < 2048) g_gemm_dbg[cta_ * 8 + (slot)] = gemm_gtime();                                               \
-  } while (0)
-#else
-#define GEMM_MARK(slot)
-#endif
-
 constexpr int kBM = 128;
 constexpr int kBK = 32;                 // fp32 elements per k-block = one 128 B swizzle row
 constexpr int kConvWarps = 8;              // converter warps; the first four double as the epilogue warps
@@ -150,7 +134,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   const int nkb = min((p.K + kBK - 1) / kBK - kb_begin, p.kb_per);
   const bool split = gridDim.z > 1;
 
-  if (threadIdx.x == 0) GEMM_MARK(0);
   if (threadIdx.x == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
@@ -178,7 +161,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) GEMM_MARK(1);
 
   if (warp == 0) {
     // ===== TMA producer =====
@@ -209,7 +191,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       for (int kb = 0; kb < nkb; ++kb) {
         const int s = kb % STAGES;
         mbar_wait(&conv[s], (uint32_t)((kb / STAGES) & 1));
-        if (kb == 0) GEMM_MARK(2);
         tc_fence_after();
         const uint32_t a_hi = smem_u32(stage0 + (size_t)s * STAGE_BYTES);
         const uint32_t b_hi = a_hi + A_BYTES;
@@ -255,7 +236,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     // epilogue (warps 2..5): warp w may touch TMEM lanes [32*(w%4), +32)
     if (warp < 6) {
     mbar_wait(tmem_full, 0);
-    if (threadIdx.x == 64) GEMM_MARK(3);
     tc_fence_after();
     const int q = warp & 3;
     const int row = m0 + 32 * q + lane;
@@ -352,7 +332,6 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   }
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) GEMM_MARK(4);
   if (warp == 1) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
@@ -645,17 +624,6 @@ int dispatch_major(int a_mn, int b_mn, const CUtensorMap &ta, const CUtensorMap 
 }  // namespace re2e
 
 using namespace re2e;
-
-#ifdef RE2E_GEMM_DEBUG
-extern "C" int re2e_gemm_debug_read(long long *host_out) {   // returns the records and clears them
-  cudaDeviceSynchronize();
-  cudaError_t e = cudaMemcpyFromSymbol(host_out, g_gemm_dbg, sizeof(long long) * 8 * 2048);
-  void *p = nullptr;
-  if (e == cudaSuccess) e = cudaGetSymbolAddress(&p, g_gemm_dbg);
-  if (e == cudaSuccess) e = cudaMemset(p, 0, sizeof(long long) * 8 * 2048);
-  return (int)e;
-}
-#endif
 
 // C[M,N] (+)= Aop[M,K] * Bop[N,K]^T (+ bias[N]);  a_mn = 0: A is [M][lda>=K] (K contiguous), a_mn = 1: A is
 // stored [K][lda>=M] (M contiguous).  Same for B with N.  lda, ldb multiples of 4; A, B 16 B aligned.

@@ -32,7 +32,7 @@ from test_gpu_frontend_paths import _template_args
 
 gpu = pytest.mark.gpu
 DEV = "cuda:0"
-E_ARG, E_UNSUPPORTED = -1, -2
+E_ARG = -1
 B200_SMS = 148
 TILE, PERSIST = "gemm_tf32x3_kernel", "gemm_tf32x3_persist_kernel"
 TAU = 1e-5
@@ -529,58 +529,6 @@ def test_linear_skips_the_unneeded_gradient_product(needs):
         assert w.grad is None and rel_err(x.grad, gy.double() @ w.detach().double()) < 1e-5
     else:
         assert x.grad is None and rel_err(w.grad, gy.double().t() @ x.detach().double()) < 1e-5
-
-
-# ---- re2e_skinny_nt / re2e_skinny_nn --------------------------------------------------------------------------------------
-@gpu
-@pytest.mark.parametrize("nn", [0, 1], ids=["nt", "nn"])
-@pytest.mark.parametrize("M,N,K,x_off,acc", [
-    (1, 37, 45, 0, 0),        # odd K: scalar staging
-    (31, 37, 64, 1, 0),       # K % 4 == 0 but X one float past 16 B: scalar staging
-    (32, 1200, 300, 0, 0),    # vector staging
-    (33, 50, 45, 0, 1),
-    (70, 33, 320, 1, 1),      # three rows per lane
-    (70, 1200, 300, 0, 1),
-])
-def test_skinny_matches_fp64(nn, M, N, K, x_off, acc):
-    g = torch.Generator().manual_seed(M * N + K + nn)
-    X = torch.randn(M, K, generator=g)
-    W = torch.randn(K, N, generator=g) if nn else torch.randn(N, K, generator=g)
-    out0 = torch.randn(M, N, generator=g) if acc else None
-    xb = torch.full((M * K + 8,), float("nan"), device=DEV)
-    xb[x_off:x_off + M * K] = X.flatten().to(DEV)
-    ob = torch.full((M * N + 64,), float("nan"), device=DEV)
-    out = ob[32:32 + M * N].view(M, N)
-    if acc:
-        out.copy_(out0)
-    Wd = W.to(DEV)
-    fn = _lib.lib().re2e_skinny_nn if nn else _lib.lib().re2e_skinny_nt
-    n0 = _lib.launch_count()
-    assert fn(xb.data_ptr() + 4 * x_off, Wd.data_ptr(), out.data_ptr(), M, N, K, acc, _lib.stream_ptr()) == 0
-    torch.cuda.synchronize()
-    assert _lib.launch_count() == n0 + 1
-    assert torch.isnan(ob[:32]).all() and torch.isnan(ob[32 + M * N:]).all()
-    Wt = W.double() if nn else W.double().t()
-    ref = X.double() @ Wt + (out0.double() if acc else 0.0)
-    scale = X.double().abs() @ Wt.abs() + (out0.double().abs() if acc else 0.0)
-    # fp32 FMA chains of <= K terms plus the accumulate add: |error| <= (K + 2) u (sum |x||w| + |out0|), u = 2^-24
-    ratio = float(((out.cpu().double() - ref).abs() / scale).max())
-    assert ratio <= (K + 2) * 2.0 ** -24, ratio
-    assert rel_err(out, ref) < 1e-5
-
-
-@gpu
-@pytest.mark.parametrize("nn", [0, 1], ids=["nt", "nn"])
-def test_skinny_rejects_shapes_over_its_shared_memory(nn):
-    M, N, K = 64, 32, 800      # 4 (64 * 801 + 16 * 800) B = 256 KB > 200 KB
-    X = torch.randn(M, K, device=DEV)
-    W = torch.randn(N, K, device=DEV)
-    out = torch.full((M, N), 7.0, device=DEV)
-    fn = _lib.lib().re2e_skinny_nn if nn else _lib.lib().re2e_skinny_nt
-    n0 = _lib.launch_count()
-    assert fn(X.data_ptr(), W.data_ptr(), out.data_ptr(), M, N, K, 0, _lib.stream_ptr()) == E_UNSUPPORTED
-    torch.cuda.synchronize()
-    assert _lib.launch_count() == n0 and bool((out == 7.0).all())
 
 
 # ---- column sums --------------------------------------------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-"""Device time of the decoder's per-position products: re2e_batch_nt against the generic batch-sized kernels / GEMM."""
+"""Device time of the decoder's per-position products: re2e_batch_nt against the dense GEMM."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -59,8 +59,6 @@ for M, N, K in [(32, 1200, 320), (32, 1200, 300), (32, 320, 1200), (32, 300, 120
     row = {"shape": (M, N, K),
            "batch_nt": graph_time(lambda: L.re2e_batch_nt(_lib.ptr(X), _lib.ptr(W), None, _lib.ptr(O), M, N, K, 0, sp())),
            "gemm": graph_time(lambda: gemm_tf32x3(X, False, WT, True, O, M, N, K))}
-    if K <= 320:
-        row["skinny"] = graph_time(lambda: L.re2e_skinny_nt(_lib.ptr(X), _lib.ptr(W), _lib.ptr(O), M, N, K, 0, sp()))
     print({k: (round(v, 2) if isinstance(v, float) else v) for k, v in row.items()}, flush=True)
 
 B, D, Z = 32, 320, 300
